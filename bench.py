@@ -2,7 +2,7 @@
 """bench.py -- BASELINE.json's metric on B200: training sequences/s (BERT4Rec, SASRec) and full-catalogue top-10
 evaluation users/s, one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload bert|sasrec|eval] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload bert|sasrec|eval] [--impl reference] [--dump-outputs DIR]
 
 Workloads (SURVEY.md 8d):
   bert    (default, the headline line) BASELINE configs[1]: BERT4Rec nb=2 d=64 h=2 L=200 mask_prob=0.15, ML-1M-shaped
@@ -23,6 +23,9 @@ evaluation batch (transformer body, fused scoring + top-10, HR/NDCG).  One JSON 
                THIS world size: sharded 10M-item evaluation, SASRec cfg3 strong scaling (global B=4096), BERT4Rec
                configs[3] (d=256, 1M items) with row-sharded tables -- each with a single-GPU-equivalence check.
 `--impl reference` times only the CPU arm (rank 0) and prints the same line with "impl": "reference".
+`--dump-outputs DIR` writes what the top-level workload's last timed step returned, as DIR/<name>.npy (rank 0): for training
+the loss plus every parameter and gradient after that step, for evaluation the top-10 values / ids and the metric means.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -89,6 +92,24 @@ def host_threads():
         n = max(1, os.cpu_count() or 1)
     torch.set_num_threads(n)
     return torch.get_num_threads()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+    """Save {name: tensor} as out_dir/<name>.npy: floating tensors as float32, integer ones (ids) as float64, which holds
+    every id below 2^53 exactly."""
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        host[name] = (t.double() if not t.is_floating_point() else t.float()).numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def load_peaks():
@@ -377,9 +398,11 @@ class Ctx:
 
 
 # ------------------------------------------------------------------------------------- training workloads (bert / sasrec)
-def train_workload(ctx, key, steps, warmup, batch=None, with_cpu=True, with_roofline=True, global_batch=None, check_equivalence=False):
+def train_workload(ctx, key, steps, warmup, batch=None, with_cpu=True, with_roofline=True, global_batch=None, check_equivalence=False,
+                   dump=None):
     """One training line.  Data parallel over ctx.world ranks: weak scaling with `batch` sequences per GPU, or strong
-    scaling when `global_batch` is given (each rank takes global_batch / world sequences)."""
+    scaling when `global_batch` is given (each rank takes global_batch / world sequences).  `dump`: directory that gets
+    the loss, parameters and gradients of the last timed step (rank 0)."""
     import rbm_b200
     from rbm_b200 import lib as L
     from rbm_b200.dist import GradSync, decorrelate_dropout
@@ -402,7 +425,12 @@ def train_workload(ctx, key, steps, warmup, batch=None, with_cpu=True, with_roof
     host = [tuple(torch.from_numpy(x).pin_memory() for x in b) for b in raw]
     devb = [tuple(x.to(dev) for x in b) for b in host]
 
-    step_dev = lambda i: trainer.train_step(devb[i % N_ROT])
+    last = {}
+
+    def step_dev(i):
+        # detached: a loss that kept its autograd graph alive into capture_train_step would invalidate the capture
+        last["loss"] = trainer.train_step(devb[i % N_ROT]).detach()
+
     step_mode = args.step_mode
     if step_mode == "graph":
         for i in range(2):
@@ -420,6 +448,13 @@ def train_workload(ctx, key, steps, warmup, batch=None, with_cpu=True, with_roof
     ms_dev = ctx.timed(step_dev, steps)
     launches = L.launch_count
     clocks = sampler.stop() if sampler else None
+    if dump and rank == 0:
+        outs = {"loss": last["loss"]}
+        for k, p in model.named_parameters():
+            outs["param." + k] = p
+            if p.grad is not None:
+                outs["grad." + k] = p.grad
+        write_outputs(dump, outs)
 
     # ---- end-to-end leg: host pinned buffers -> trainer API -> loss value back on the host, every step
     losses = []
@@ -514,7 +549,7 @@ def dp_equivalence(ctx, spec, Bsz):
 
 
 # ------------------------------------------------------------------------------------------- evaluation workload
-def eval_workload(ctx, steps, warmup, with_cpu=True, V=None):
+def eval_workload(ctx, steps, warmup, with_cpu=True, V=None, dump=None):
     """Full-catalogue top-10 HR/NDCG users/s.  world == 1: the whole item table on one GPU.  world > 1: the table is
     row-sharded (shard_sas_model), every rank brings users_per_step / world users per step; last hidden rows all-gathered,
     shard-local fused scoring + top-10 with global ids, all-to-all of the lists by user range, merge, HR/NDCG partial sums
@@ -557,10 +592,12 @@ def eval_workload(ctx, steps, warmup, with_cpu=True, V=None):
             means = means / world
         return means
 
+    last_dev = {}
+
     def step_dev(i):
         with torch.no_grad():
-            _, ids = model.full_catalogue_topk(seqs[i % 2], 10)
-            return metrics_dev(ids, poss[i % 2])
+            vals, ids = model.full_catalogue_topk(seqs[i % 2], 10)
+            last_dev.update(top10_values=vals, top10_ids=ids, metric_means=metrics_dev(ids, poss[i % 2]))
 
     if world > 1:
         with torch.no_grad():
@@ -575,6 +612,8 @@ def eval_workload(ctx, steps, warmup, with_cpu=True, V=None):
     ms_dev = ctx.timed(step_dev, steps)
     launches = L.launch_count
     clocks = sampler.stop() if sampler else None
+    if dump and rank == 0:
+        write_outputs(dump, last_dev)
     last = {}
 
     def step_e2e(i):
@@ -832,6 +871,8 @@ def main():
                     help="graph: trainer.capture_train_step (CUDA-graph replay of the whole optimisation step); eager: launch by launch")
     ap.add_argument("--dp-collective", default=os.environ.get("RBM_BENCH_DP_COLLECTIVE", "split"), choices=["split", "graph"],
                     help="N>1 with --step-mode graph: eager NCCL all-reduce between two graphs (split) or captured inside one graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the top-level workload to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
@@ -842,9 +883,9 @@ def main():
     world = ctx.world
 
     if args.workload == "eval":
-        line = eval_workload(ctx, steps=min(args.steps, 10), warmup=min(args.warmup, 3))
+        line = eval_workload(ctx, steps=args.steps, warmup=min(args.warmup, 3), dump=args.dump_outputs)
     else:
-        line = train_workload(ctx, args.workload, args.steps, args.warmup, batch=args.batch)
+        line = train_workload(ctx, args.workload, args.steps, args.warmup, batch=args.batch, dump=args.dump_outputs)
 
     extras = None
     if not args.no_extras and args.workload == "bert":
