@@ -17,16 +17,23 @@ W0, W1 = 0x9E3779B9, 0xBB67AE85
 MASK32 = 0xFFFFFFFF
 
 
-def philox4x32_10(counter: Sequence[int], key: Sequence[int]) -> Tuple[int, int, int, int]:
-    """One Philox4x32-10 block: counter (c0..c3), key (k0, k1) -> four 32-bit words."""
-    c0, c1, c2, c3 = [int(c) & MASK32 for c in counter]
+def philox4x32(counter: Sequence, key: Sequence[int], rounds: int) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+    """Philox4x32 with ``rounds`` rounds over numpy arrays: counter words (c0..c3, each an int or an array; they broadcast
+    against each other), key (k0, k1) -> four uint64 arrays holding the 32-bit output words."""
+    c0, c1, c2, c3 = [np.asarray(c, dtype=np.uint64) & np.uint64(MASK32) for c in counter]
     k0, k1 = [int(k) & MASK32 for k in key]
-    for _ in range(10):
-        p0, p1 = M0 * c0, M1 * c2
-        hi0, lo0, hi1, lo1 = p0 >> 32, p0 & MASK32, p1 >> 32, p1 & MASK32
-        c0, c1, c2, c3 = (hi1 ^ c1 ^ k0) & MASK32, lo1, (hi0 ^ c3 ^ k1) & MASK32, lo0
+    m0, m1, lo32 = np.uint64(M0), np.uint64(M1), np.uint64(MASK32)
+    for _ in range(rounds):
+        p0, p1 = m0 * c0, m1 * c2  # 32 x 32 -> 64 bits: exact in uint64
+        hi0, lo0, hi1, lo1 = p0 >> np.uint64(32), p0 & lo32, p1 >> np.uint64(32), p1 & lo32
+        c0, c1, c2, c3 = hi1 ^ c1 ^ np.uint64(k0), lo1, hi0 ^ c3 ^ np.uint64(k1), lo0
         k0, k1 = (k0 + W0) & MASK32, (k1 + W1) & MASK32
     return c0, c1, c2, c3
+
+
+def philox4x32_10(counter: Sequence[int], key: Sequence[int]) -> Tuple[int, int, int, int]:
+    """One Philox4x32-10 block: counter (c0..c3), key (k0, k1) -> four 32-bit words."""
+    return tuple(int(w) for w in philox4x32(counter, key, 10))
 
 
 def rbm_philox(seed: int, site: int, idx4: int) -> Tuple[int, int, int, int]:

@@ -40,6 +40,42 @@ class DropoutPlan:
 NO_DROPOUT = DropoutPlan(training=False)
 
 
+def _philox7(seed: int, site: int, call: np.ndarray):
+    """Philox4x32-7 of the dropout sites: key = seed, counter = (call lo, call hi, site lo, site hi)."""
+    from .batches import philox4x32
+    call = np.asarray(call, dtype=np.uint64)
+    return philox4x32((call, call >> np.uint64(32), site & 0xFFFFFFFF, site >> 32), (seed & 0xFFFFFFFF, seed >> 32), 7)
+
+
+def keep_mask(n: int, p: float, seed: int, site: int) -> np.ndarray:
+    """Keep mask (bool [n]) of an element-wise dropout site (include/rbm.h): element e takes word e % 4 of the Philox4x32-7 call
+    e // 4 and is kept iff that word >= floor(p * 2^32), with p rounded to fp32 first as the C ABI passes it."""
+    t = float(np.float32(p)) * 4294967296.0
+    thr = 0 if t <= 0.0 else (0xFFFFFFFF if t >= 4294967295.0 else int(t))
+    words = _philox7(seed, site, np.arange((n + 3) // 4, dtype=np.uint64))
+    return (np.stack(words, axis=1).reshape(-1)[:n] >= thr)
+
+
+def attn_keep_mask(BH: int, L: int, p: float, seed: int, site: int) -> np.ndarray:
+    """Keep mask (bool [BH * L, L], row = bh * L + i, column = key j) of an attention dropout site (csrc/common.cuh): element
+    (bh, i, j) is the 16-bit field  f = ((i >> 3) & 1) * 4 + (j & 1) * 2 + ((j >> 3) & 1)  (word f >> 1, high half when f is odd)
+    of Philox4x32-7 call  ((((bh * 16 + (i >> 4)) * 8 + (i & 7)) * 4 + ((j & 7) >> 1)) * 16 + (j >> 4)),  kept iff the field
+    >= round(p * 65536)."""
+    t = float(np.float32(p)) * 65536.0 + 0.5
+    thr16 = 0 if t <= 0.5 else (65535 if t >= 65535.0 else int(t))
+    i = np.arange(L, dtype=np.int64)[:, None]
+    j = np.arange(L, dtype=np.int64)[None, :]
+    local = ((((i >> 4) * 8 + (i & 7)) * 4 + ((j & 7) >> 1)) * 16 + (j >> 4))  # the call index without bh: < 8192
+    field = ((i >> 3) & 1) * 4 + (j & 1) * 2 + ((j >> 3) & 1)
+    calls, inv = np.unique(local, return_inverse=True)
+    inv = inv.reshape(L, L)
+    bh = np.arange(BH, dtype=np.uint64)[:, None]
+    words = np.stack(_philox7(seed, site, bh * np.uint64(8192) + calls.astype(np.uint64)[None, :]), axis=-1)  # [BH, calls, 4]
+    w = words[:, inv, field >> 1]  # [BH, L, L]
+    f16 = np.where((field & 1).astype(bool), w >> np.uint64(16), w & np.uint64(0xFFFF))
+    return (f16 >= thr16).reshape(BH * L, L)
+
+
 def torch_layernorm(x: torch.Tensor, w: torch.Tensor, b: torch.Tensor, eps: float) -> torch.Tensor:
     """``torch.nn.LayerNorm`` as used at NN/models/sas_model/sas.py:39,42,50 (eps=1e-8):
     biased variance, eps inside the sqrt."""

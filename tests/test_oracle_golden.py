@@ -207,6 +207,35 @@ def test_philox_known_answers():
     assert philox4x32_10((0xffffffff,) * 4, (0xffffffff, 0xffffffff)) == (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)
     assert philox4x32_10((0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344), (0xa4093822, 0x299f31d0)) == (
         0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1)
+    from oracle.batches import philox4x32  # the same vectors as one array call
+    cs = np.array([[0, 0xffffffff, 0x243f6a88], [0, 0xffffffff, 0x85a308d3], [0, 0xffffffff, 0x13198a2e], [0, 0xffffffff, 0x03707344]])
+    got = philox4x32(list(cs), (0xa4093822, 0x299f31d0), 10)
+    assert [int(w[2]) for w in got] == [0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1]
+
+
+@pytest.mark.parametrize("L", [1, 7, 16, 17, 40])
+def test_dropout_masks_restate_the_per_element_rule(L):
+    """The vectorised masks of oracle/common.py against a per-element transcription of the scalar rules of csrc/common.cuh
+    (rbm_drop4, rbm_attn_keep): seed and site with their high 32 bits set."""
+    from oracle.batches import philox4x32
+    seed, site, p = (0xA5A5 << 32) | 77, (3 << 32) | 9, 0.3
+
+    def r7(call):
+        return [int(w) for w in philox4x32((call & 0xFFFFFFFF, call >> 32, site & 0xFFFFFFFF, site >> 32), (seed & 0xFFFFFFFF, seed >> 32), 7)]
+
+    thr = int(float(np.float32(p)) * 2 ** 32)
+    n = 4 * L + 3
+    assert oc.keep_mask(n, p, seed, site).tolist() == [r7(e // 4)[e % 4] >= thr for e in range(n)]
+    thr16 = int(float(np.float32(p)) * 65536 + 0.5)
+    BH = 3
+    got = oc.attn_keep_mask(BH, L, p, seed, site)
+    for bh in range(BH):
+        for i in range(L):
+            for j in range(L):
+                r = r7((((bh * 16 + (i >> 4)) * 8 + (i & 7)) * 4 + ((j & 7) >> 1)) * 16 + (j >> 4))
+                f = ((i >> 3) & 1) * 4 + (j & 1) * 2 + ((j >> 3) & 1)
+                w = r[f >> 1]
+                assert bool(got[bh * L + i, j]) == (((w >> 16) if f & 1 else (w & 0xFFFF)) >= thr16), (bh, i, j)
 
 
 def _histories(z):
