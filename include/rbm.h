@@ -116,7 +116,7 @@ int rbm_layernorm_bwd_fanout(const float* x, const float* gamma, const float* dy
  * pre = x[M,K] . w[N,K]^T + bias        (optionally stored to `pre` when act needs it in backward)
  * y   = rowkeep * dropB( residual + dropA( act(pre) ) )      rowkeep(r) = row_tok ? row_tok[r]!=0 : 1
  * Blackwell path: tcgen05.mma kind::tf32 (fp32 operands read as TF32, fp32 accumulation in TMEM), TMA-fed, whenever
- * K % 32 == 0 and N % 16 == 0; other shapes use the fp32 SIMT kernel.  RBM_LINEAR_IMPL=simt forces the latter.
+ * K % 32 == 0 and N % 16 == 0; other shapes use the fp32 SIMT kernel.
  * replaces nn.Linear / Conv1d(k=1) + Dropout + activation + residual chains:
  *   NN/models/bert_modules/attention/multi_head.py:29-30,40; utils/feed_forward.py:16; utils/sublayer.py:18;
  *   transformer.py:32; NN/models/sas_model/sas.py:16-19,75,79,84 (in/out-proj of nn.MultiheadAttention). */

@@ -18,12 +18,11 @@
 // elected thread of warp 0 issues the MMAs.  Dropout follows the library's Philox
 // contract (common.cuh, rbm_attn_keep), atomics-free and bit-deterministic.
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E
 #include "tc_ptx.cuh"
 #include "attention_pair.cuh"
+#include "attention_tc.cuh"  // rbm_attn_tc_enabled
 
 namespace {
 
@@ -610,29 +609,16 @@ __global__ void __launch_bounds__(THREADS, 1) attn_pair_bwd_kernel(const PairArg
   }
 }
 
-bool pair_enabled() {
-  const char* e = getenv("RBM_ATTN_IMPL");
-  return !(e && strcmp(e, "mma") == 0);
-}
 float pscale_for(float inv_keep) {
   int e = 0;
   frexpf(inv_keep, &e);           // inv_keep <= 2^e
   return ldexpf(1.f, 14 - e);     // P~ * pscale <= 2^14
 }
-template <typename K>
-bool set_smem(K kern, size_t bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
-    return false;
-  }
-  return true;
-}
 
 }  // namespace
 
 bool rbm_attn_pair_supported(int L, int dk, int mask_mode) {
-  return pair_enabled() && dk == DK && L >= 1 && L <= 64 && (mask_mode == RBM_MASK_NONE || mask_mode == RBM_MASK_CAUSAL);
+  return rbm_attn_tc_enabled() && dk == DK && L >= 1 && L <= 64 && (mask_mode == RBM_MASK_NONE || mask_mode == RBM_MASK_CAUSAL);
 }
 
 int rbm_attn_pair_fwd(const float* q, int64_t ldq, const float* k, int64_t ldk, const float* v, int64_t ldv, float* out, int64_t ldo,

@@ -16,12 +16,11 @@
 // Reference semantics kept: padded keys score -1e9 (masked_fill: a fully padded row gets the uniform softmax) and pass no
 // score gradient; causal / beyond-L keys are excluded; dropout per the library's Philox contract (common.cuh).
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E, RBM_PADFILL
 #include "tc_ptx.cuh"
 #include "attention_seq.cuh"
+#include "attention_tc.cuh"  // rbm_attn_tc_enabled
 
 namespace {
 
@@ -663,19 +662,6 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_dkv_kernel(const SeqArgs 
   SEQ_EPILOGUE(512);
 }
 
-bool seq_enabled() {
-  const char* e = getenv("RBM_ATTN_IMPL");
-  return !(e && strcmp(e, "mma") == 0);
-}
-template <typename K>
-bool set_smem(K kern, size_t bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
-    return false;
-  }
-  return true;
-}
 void fill_common(SeqArgs& a, int B, int L, int h, int mask_mode, float scale, float p, uint64_t seed, uint64_t site, const int64_t* tok) {
   a.L = L; a.h = h; a.n_items = B * h; a.mask_mode = mask_mode; a.scale = scale; a.tok = tok;
   a.thr16 = rbm_drop_threshold16(p);
@@ -689,7 +675,7 @@ void fill_common(SeqArgs& a, int B, int L, int h, int mask_mode, float scale, fl
 
 }  // namespace
 
-bool rbm_attn_seq_supported(int L, int dk, int mask_mode) { return seq_enabled() && dk == DK && L > 64 && L <= 256 && mask_mode >= 0 && mask_mode <= 2; }
+bool rbm_attn_seq_supported(int L, int dk, int mask_mode) { return rbm_attn_tc_enabled() && dk == DK && L > 64 && L <= 256 && mask_mode >= 0 && mask_mode <= 2; }
 
 int rbm_attn_seq_fwd(const float* q, int64_t ldq, const float* k, int64_t ldk, const float* v, int64_t ldv, const int64_t* tok, float* out,
                      int64_t ldo, float* stats, int B, int L, int h, int mask_mode, float scale, float p, uint64_t seed, uint64_t site,

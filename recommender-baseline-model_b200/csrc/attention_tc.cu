@@ -1339,26 +1339,9 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
 // [B, L, width] fp32 view of a token-major buffer with row stride ld; box = [1, box_rows, 32], 128-byte swizzle
 bool encode_map3(CUtensorMap* map, const float* base, int B, int L, int width, int64_t ld, int box_rows, bool mn_major) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[3] = {(cuuint64_t)width, (cuuint64_t)L, (cuuint64_t)B};
   cuuint64_t gstride[2] = {(cuuint64_t)ld * sizeof(float), (cuuint64_t)L * ld * sizeof(float)};
@@ -1374,20 +1357,22 @@ bool encode_map3(CUtensorMap* map, const float* base, int B, int L, int width, i
   return r == CUDA_SUCCESS;
 }
 
-bool tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("RBM_ATTN_IMPL");
-    v = (e && strcmp(e, "mma") == 0) ? 0 : 1;
-  }
-  return v == 1;
-}
-
 }  // namespace
+
+// RBM_ATTN_IMPL=mma sends every dense attention call to the SIMT kernels of attention.cu: tests/test_attention_gpu.py and
+// tools/run_env_matrix.sh use it to run those kernels at d_k = 32 and 64, where the shape rules pick the tensor-core ones.  Read
+// once per process: the tests set it before the library is loaded.
+bool rbm_attn_tc_enabled() {
+  static const bool v = [] {
+    const char* e = getenv("RBM_ATTN_IMPL");
+    return !(e && strcmp(e, "mma") == 0);
+  }();
+  return v;
+}
 
 bool rbm_attn_fwd_tc_supported(int L, int dk, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo, const void* q, const void* k,
                                const void* v, const void* out) {
-  if (!tc_enabled() || dk != DK || L < 1 || L > 256) return false;  // the score tile is one TMEM region of Lp <= 256 columns
+  if (!rbm_attn_tc_enabled() || dk != DK || L < 1 || L > 256) return false;  // the score tile is one TMEM region of Lp <= 256 columns
   if (ldq % 4 || ldk % 4 || ldv % 4 || ldo % 4) return false;
   if (((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)out) & 15) return false;
   return get_encode() != nullptr;
@@ -1433,7 +1418,7 @@ int rbm_attn_fwd_tc_launch(const float* q, int64_t ldq, const float* k, int64_t 
 
 bool rbm_attn_bwd_dq_tc_supported(int L, int dk, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo, int64_t lddo, int64_t lddq,
                                   const void* q, const void* k, const void* v, const void* o, const void* dout, const void* dq) {
-  if (!tc_enabled() || dk != DK || L < 1 || L > 256) return false;
+  if (!rbm_attn_tc_enabled() || dk != DK || L < 1 || L > 256) return false;
   if (ldq % 4 || ldk % 4 || ldv % 4 || ldo % 4 || lddo % 4 || lddq % 4) return false;
   if (((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)o | (uintptr_t)dout | (uintptr_t)dq) & 15) return false;
   return get_encode() != nullptr;
@@ -1483,7 +1468,7 @@ int rbm_attn_bwd_dq_tc_launch(const float* q, int64_t ldq, const float* k, int64
 
 bool rbm_attn_bwd_dkv_tc_supported(int L, int dk, int64_t ldq, int64_t ldk, int64_t ldv, int64_t lddo, int64_t lddk, int64_t lddv,
                                    const void* q, const void* k, const void* v, const void* dout, const void* dk_, const void* dv) {
-  if (!tc_enabled() || dk != DK || L < 1 || L > 256) return false;
+  if (!rbm_attn_tc_enabled() || dk != DK || L < 1 || L > 256) return false;
   if (ldq % 4 || ldk % 4 || ldv % 4 || lddo % 4 || lddk % 4 || lddv % 4) return false;
   if (((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)dout | (uintptr_t)dk_ | (uintptr_t)dv) & 15) return false;
   return get_encode() != nullptr;

@@ -4,6 +4,9 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+// false under RBM_ATTN_IMPL=mma; gates the tcgen05 kernels of attention_tc.cu, attention_pair.cu and attention_seq.cu
+bool rbm_attn_tc_enabled();
+
 bool rbm_attn_fwd_tc_supported(int L, int dk, int64_t ldq, int64_t ldk, int64_t ldv, int64_t ldo, const void* q, const void* k,
                                const void* v, const void* out);
 int rbm_attn_fwd_tc_launch(const float* q, int64_t ldq, const float* k, int64_t ldk, const float* v, int64_t ldv, const int64_t* tok,

@@ -9,8 +9,6 @@
 //   ce_bwd_dw_tc  rows = 128 vocab entries (W rows in TMEM); compacted hidden rows stream in 64-row chunks (K-major for
 //                 S^T = W.H^T, MN-major for dW += G^T.H); db = row sums of G^T; row chunks split over blockIdx.y with
 //                 a fixed-order reduction.
-#include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E, RBM_LN2
 #include "tc_ptx.cuh"
@@ -615,26 +613,9 @@ __global__ void __launch_bounds__(256) gather_split_kernel(const float* __restri
   st4(hcl + i * 4, make_float4(lo_of(v.x), lo_of(v.y), lo_of(v.z), lo_of(v.w)));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
 // [rows, d] fp32, box [64 rows x 32 cols]; K-major consumers: 128B swizzle, MN-major consumers: 32-byte-atom variant
 bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int d, bool mn) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)d, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)d * sizeof(float)};
@@ -644,32 +625,10 @@ bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int d, bool m
              mn ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-bool tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("RBM_CE_IMPL");
-    v = (e && strcmp(e, "mma") == 0) ? 0 : 1;
-  }
-  return v == 1;
-}
-template <typename K>
-bool set_smem(K kern, size_t bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
-    return false;
-  }
-  return true;
-}
-
 }  // namespace
 
 bool rbm_ce_tc_supported(int V1, int d, const void* h, const void* w) {
-  if (!tc_enabled() || (d != 32 && d != 64) || V1 < CW) return false;  // backward: 4d + 256 TMEM columns
-  if (d == 64) {  // experiment switch: hand d = 64 to the split-fp16 kernels of ce_wide.cu
-    const char* e = getenv("RBM_CE_WIDE_D64");
-    if (e && atoi(e) != 0) return false;
-  }
+  if ((d != 32 && d != 64) || V1 < CW) return false;  // backward: 4d + 256 TMEM columns
   if (((uintptr_t)h | (uintptr_t)w) & 15) return false;
   return get_encode() != nullptr;
 }

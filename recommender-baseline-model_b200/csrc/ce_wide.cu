@@ -12,12 +12,14 @@
 // would be L2-bound.  16-bit operands also need no second (MN-major) copy of the streamed tile: the 128-byte-swizzled
 // K-major tile TMA writes is, read with an MN-major descriptor, exactly the B operand of the update product.
 //
-// One kernel template, three modes; a CTA owns 128 "resident" rows (TMEM lanes, one epilogue thread per row) and streams
-// the other side in NV-row chunks (NV = 48 at d = 256, 64 at d = 128):
-//   FWD  resident = 128 compacted hidden rows, stream = vocabulary range of the unit: S = R.W^T into TMEM, two groups of
-//        four warps alternate chunks keeping an online (max, sum-exp) in the log2 domain + the target logit.
-//   DH   same streaming; G = (softmax - onehot) as split fp16 pairs overwrites TMEM columns and feeds
-//        D[128 x d] += G . W[chunk]   (A from TMEM, B = the same streamed tile read MN-major).
+// A CTA owns 128 "resident" rows (TMEM lanes, one epilogue thread per row) and streams the other side in chunks:
+//   FWD  (ce_wide_fwd128_kernel) resident = 128 compacted hidden rows, stream = vocabulary range of the unit in 128-row tiles:
+//        S = R.W^T into TMEM, two groups of four warps alternate chunks keeping an online (max, sum-exp) in the log2 domain +
+//        the target logit.
+//   The backward is one kernel template with two modes, streaming NV-row chunks (NV = 48 at d = 256, 64 at d = 128):
+//   DH   resident = 128 compacted hidden rows, stream = vocabulary range of the unit: S = R.W^T, then G = (softmax - onehot) as
+//        split fp16 pairs overwrites TMEM columns and feeds D[128 x d] += G . W[chunk]   (A from TMEM, B = the same streamed
+//        tile read MN-major).
 //   DW   resident = 128 vocabulary rows, stream = compacted hidden rows: S^T, G^T, D[128 x d] += G^T . H[chunk],
 //        db = row sums of G^T; hidden-row chunks split over blockIdx.y.
 // Units: FWD / DH = (row tile, vocabulary split); the split count is derived ON THE DEVICE from the live row count (the
@@ -25,7 +27,6 @@
 // statistics / dH blocks per unit are combined in fixed order by small kernels (no atomics: bit-deterministic).
 #include <cuda_fp16.h>
 #include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E, RBM_LN2
 #include "tc_ptx.cuh"
@@ -41,7 +42,7 @@ constexpr int RBLK = 128 * 128;          // one resident K-block: 128 rows x 64 
 constexpr int UMAX = 8 * RBM_NUM_SMS;    // most (row tile, vocabulary split) units the device-side decomposition creates
 constexpr float GSCALE = 16384.f;        // softmax - onehot in [-1, 1] -> fp16 range with 2^-14 * 2^-24 absolute resolution
 
-enum { MODE_FWD = 0, MODE_DH = 1, MODE_DW = 2 };
+enum { MODE_DH = 1, MODE_DW = 2 };
 
 struct WideArgs {
   const int32_t* rows;
@@ -56,7 +57,7 @@ struct WideArgs {
   float* part_b;              // DW: [S][V1]
   const __half *r_hi, *r_lo;  // pre-split resident matrix ([r_rows, d] fp16): hidden rows (FWD / DH) or the weight (DW)
   int64_t r_rows;
-  int V1, d, KB, NV, nstage, npass, S, bias_vec, pair;
+  int V1, d, KB, NV, nstage, npass, S, bias_vec;
 };
 
 // vocabulary splits per row tile: the split count that fills whole waves of 148 SMs best with at most UMAX units
@@ -126,15 +127,15 @@ __device__ __forceinline__ void split_pack16(const float (&g)[16], uint32_t (&hi
   }
 }
 
-// --------------------------------------------------------------------------------------------------- the kernel
+// --------------------------------------------------------------------------------------------- the backward kernel
 // The resident operand's hi half lives in TENSOR MEMORY (16-bit A operand: two K elements per 32-bit column), written once
 // per unit by the epilogue threads from the pre-split global copy, so the score products read only the streamed tile from
 // shared memory: with both operands in shared memory a 128 x NV x 16 instruction fetches 4 KB of A + 32 NV bytes of B and
 // measured ~70 cycles whatever NV (~80 B/cycle of operand fetch), three times the tensor floor of NV/2 cycles.  The lo
-// half follows into TMEM where columns are left (FWD: no accumulator; d = 128); at d = 256 in DH / DW it stays in shared
-// memory (64 KB, K-major) and only the third pass pays the shared-memory fetch.
+// half follows into TMEM where columns are left (d = 128); at d = 256 it stays in shared memory (64 KB, K-major) and only the
+// third pass pays the shared-memory fetch.
 //   TMEM columns: R hi [0, d/2) | group g at 128 + 64 g: S [+0, +NV) fp32, overwritten by G hi [+0, +NV/2) | G lo
-//                 [+NV/2, +NV) | D [256, 256 + d)   (FWD, no D: R lo [256, 256 + d/2);  d = 128: R lo [384, 448))
+//                 [+NV/2, +NV) | D [256, 256 + d)   (d = 128: R lo [384, 448))
 //   SMEM: { resident lo: KB blocks of 16 KB, unless it is in TMEM } | nstage x { streamed hi (KB blocks of NV x 128 B) | lo }
 template <int MODE>
 __global__ void __launch_bounds__(64 + 32 * NSW, 1)
@@ -147,7 +148,7 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int count = *a.count;
   const int d = a.d, KB = a.KB, NV = a.NV, ns = a.nstage, V1 = a.V1;
-  const bool lo_tmem = (MODE == MODE_FWD) || d <= 128;
+  const bool lo_tmem = d <= 128;
   // ---- unit: resident tile + chunk range [c_begin, c_end) step c_step of the streamed side
   int r_tile, c_begin, c_end, c_step, unit;
   if (MODE == MODE_DW) {
@@ -193,7 +194,7 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = tmem_base_slot;
-  const uint32_t tRh = tmem, tG0 = tmem + 128, tD = tmem + 256, tRl = tmem + ((MODE == MODE_FWD) ? 256 : 384);
+  const uint32_t tRh = tmem, tG0 = tmem + 128, tD = tmem + 256, tRl = tmem + 384;
 
   if (warp == 0) {
     // ------------------------------------------------------------------------------------------ TMA producer
@@ -250,60 +251,23 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
         const int n = pend[grp], s = n % ns;
         mbar_wait(smem_u32(&g_full[grp]), (n >> 1) & 1);
         tc_fence_after();
-        if (MODE != MODE_FWD) {
-          const uint32_t sa = sSt + s * stage_bytes, tGh = tG0 + (uint32_t)grp * 64, tGl = tGh + (uint32_t)(NV / 2);
-          for (int pass = 0; pass < a.npass; ++pass) {
-            const uint32_t ga = pass == 2 ? tGl : tGh, cb = pass == 1 ? sa + KB * sblk : sa;
-            for (int ks = 0; ks < NV / 16; ++ks) {
-              umma_f16_ts(tD, ga + (uint32_t)(ks * 8), make_sw128_desc_mn16(cb + ks * 2048, sblk), idU, d_started ? 1u : 0u);
-              d_started = true;
-            }
+        const uint32_t sa = sSt + s * stage_bytes, tGh = tG0 + (uint32_t)grp * 64, tGl = tGh + (uint32_t)(NV / 2);
+        for (int pass = 0; pass < a.npass; ++pass) {
+          const uint32_t ga = pass == 2 ? tGl : tGh, cb = pass == 1 ? sa + KB * sblk : sa;
+          for (int ks = 0; ks < NV / 16; ++ks) {
+            umma_f16_ts(tD, ga + (uint32_t)(ks * 8), make_sw128_desc_mn16(cb + ks * 2048, sblk), idU, d_started ? 1u : 0u);
+            d_started = true;
           }
-          umma_commit(smem_u32(&empty_bar[s]));
         }
+        umma_commit(smem_u32(&empty_bar[s]));
         pend[grp] = -1;
       };
-      if (MODE == MODE_FWD && a.pair) {
-        // two chunks at a time, their k-steps interleaved: consecutive instructions accumulate into DIFFERENT score blocks
-        for (int n = 0; n < NL; n += 2) {
-          const bool two = n + 1 < NL;
-          if (n >= 2) {
-            mbar_wait(smem_u32(&g_full[0]), ((n >> 1) - 1) & 1);
-            if (two) mbar_wait(smem_u32(&g_full[1]), ((n >> 1) - 1) & 1);
-          }
-          mbar_wait(smem_u32(&full_bar[n % ns]), (n / ns) & 1);
-          if (two) mbar_wait(smem_u32(&full_bar[(n + 1) % ns]), ((n + 1) / ns) & 1);
-          tc_fence_after();
-          const uint32_t sa0 = sSt + (n % ns) * stage_bytes, sa1 = sSt + ((n + 1) % ns) * stage_bytes;
-          uint32_t acc = 0;
-          for (int pass = 0; pass < a.npass; ++pass) {
-            const uint32_t off = pass == 1 ? KB * sblk : 0u;
-            for (int kb = 0; kb < KB; ++kb) {
-              const uint64_t b0 = make_sw128_desc(sa0 + off + kb * sblk), b1 = make_sw128_desc(sa1 + off + kb * sblk);
-              const uint32_t ta = (pass == 2 ? tRl : tRh) + (uint32_t)(kb * 32);
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                umma_f16_ts(tG0, ta + (uint32_t)(k * 8), b0 + (uint64_t)(k * 2), idS, acc);
-                if (two) umma_f16_ts(tG0 + 64, ta + (uint32_t)(k * 8), b1 + (uint64_t)(k * 2), idS, acc);
-                acc = 1;
-              }
-            }
-          }
-          umma_commit(smem_u32(&empty_bar[n % ns]));
-          umma_commit(smem_u32(&s_full[0]));
-          if (two) {
-            umma_commit(smem_u32(&empty_bar[(n + 1) % ns]));
-            umma_commit(smem_u32(&s_full[1]));
-          }
-        }
-      } else
       for (int n = 0; n < NL; ++n) {
         const int s = n % ns, grp = n & 1;
         if (pend[grp] >= 0) accum(grp);  // frees the group's column block (the tensor pipe runs in order)
         mbar_wait(smem_u32(&full_bar[s]), (n / ns) & 1);
         tc_fence_after();
         scores(n);
-        if (MODE == MODE_FWD) umma_commit(smem_u32(&empty_bar[s]));
         umma_commit(smem_u32(&s_full[grp]));
         pend[grp] = n;
       }
@@ -346,28 +310,25 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&rt_bar));
     }
-    if (MODE != MODE_DW) {
+    if (MODE == MODE_DH) {
       const int r = r_tile * 128 + rl;
       const bool valid = r < count;
       int64_t tg = valid ? a.tgt[r] : -1;
       if (tg < 0 || tg >= V1) tg = -1;  // a target outside this (shard of the) vocabulary matches no column
-      const float lse2 = (MODE == MODE_DH) ? (valid ? a.lse_in[r] * RBM_LOG2E : INFINITY) : 0.f;  // rows beyond the count: p = 0
-      float m = -INFINITY, l = 0.f, tl = 0.f;
+      const float lse2 = valid ? a.lse_in[r] * RBM_LOG2E : INFINITY;  // rows beyond the count: p = 0
       for (int n = grp; n < NL; n += 2) {
         const int c = c_begin + n;
         mbar_wait(smem_u32(&s_full[grp]), (n >> 1) & 1);
         tc_fence_after();
-        float sv[64];  // the chunk's scores of this row (DH: all of them are read before G overwrites the columns)
-        if (MODE == MODE_DH) {
+        float sv[64];  // the chunk's scores of this row (all of them are read before G overwrites the columns)
 #pragma unroll
-          for (int part = 0; part < 4; ++part)
-            if (part * 16 < NV) tmem_ld16(tS + (uint32_t)(part * 16), *reinterpret_cast<float(*)[16]>(&sv[part * 16]));
-        }
+        for (int part = 0; part < 4; ++part)
+          if (part * 16 < NV) tmem_ld16(tS + (uint32_t)(part * 16), *reinterpret_cast<float(*)[16]>(&sv[part * 16]));
 #pragma unroll
         for (int part = 0; part < 4; ++part) {
           if (part * 16 < NV) {
             const int v0 = c * NV + part * 16;
-            float bb[16];  // bias in the log2 domain (minus the row's log-sum-exp in DH); -inf beyond the vocabulary
+            float bb[16];  // bias in the log2 domain minus the row's log-sum-exp; -inf beyond the vocabulary
             if (v0 + 16 <= V1 && (a.bias == nullptr || a.bias_vec)) {
 #pragma unroll
               for (int j = 0; j < 16; j += 4) {
@@ -380,87 +341,40 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
               for (int j = 0; j < 16; ++j) bb[j] = v0 + j < V1 ? fmaf(a.bias ? a.bias[v0 + j] : 0.f, RBM_LOG2E, -lse2) : -INFINITY;
             }
             float(&v)[16] = *reinterpret_cast<float(*)[16]>(&sv[part * 16]);
-            if (MODE == MODE_FWD) tmem_ld16(tS + (uint32_t)(part * 16), v);
             const uint32_t ts = (uint32_t)(tg - (int64_t)v0);  // this row's target column inside the slice, if < 16
             const bool hit = __any_sync(0xffffffffu, ts < 16u);
-            if (MODE == MODE_FWD) {
-              if ((part + 1) * 16 >= NV) {  // last read of this chunk's score block
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(smem_u32(&g_full[grp]));
-              }
-              float cm = -INFINITY;
+            uint32_t hi[8], lo[8];
 #pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                v[j] = fmaf(v[j], c1, bb[j]);
-                cm = fmaxf(cm, v[j]);
-              }
-              if (hit) {
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                  if (ts == (uint32_t)j) tl = v[j];
-              }
-              const float mn = fmaxf(m, cm);
-              if (mn > -INFINITY) {
-                float ps = 0.f;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) ps += ex2(v[j] - mn);
-                l = l * (m == -INFINITY ? 0.f : ex2(m - mn)) + ps;
-                m = mn;
-              }
-            } else {
-              uint32_t hi[8], lo[8];
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                float p = ex2(fmaf(v[j], c1, bb[j]));
-                if (hit && ts == (uint32_t)j) p -= 1.f;
-                v[j] = p * GSCALE;
-              }
-              split_pack16(v, hi, lo);
-              tmem_st8(tS + (uint32_t)(part * 8), hi);
-              tmem_st8(tGl + (uint32_t)(part * 8), lo);
+            for (int j = 0; j < 16; ++j) {
+              float p = ex2(fmaf(v[j], c1, bb[j]));
+              if (hit && ts == (uint32_t)j) p -= 1.f;
+              v[j] = p * GSCALE;
             }
+            split_pack16(v, hi, lo);
+            tmem_st8(tS + (uint32_t)(part * 8), hi);
+            tmem_st8(tGl + (uint32_t)(part * 8), lo);
           }
         }
-        if (MODE == MODE_DH) {
-          tmem_st_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(smem_u32(&g_full[grp]));
-        }
+        tmem_st_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(smem_u32(&g_full[grp]));
       }
-      if (MODE == MODE_FWD) {
-        // every chunk's scores have been read, hence every MMA has completed and every stage is free
-        named_bar_sync(7, NSW * 32);
-        xch[(grp * 3 + 0) * 128 + rl] = m;
-        xch[(grp * 3 + 1) * 128 + rl] = l;
-        xch[(grp * 3 + 2) * 128 + rl] = tl;
-        named_bar_sync(7, NSW * 32);
-        if (grp == 0) {
-          const float m0 = xch[rl], m1 = xch[3 * 128 + rl];
-          const float mm = fmaxf(m0, m1);
-          const float ll = xch[128 + rl] * (m0 == -INFINITY ? 0.f : ex2(m0 - mm)) + xch[4 * 128 + rl] * (m1 == -INFINITY ? 0.f : ex2(m1 - mm));
-          a.st_m[(int64_t)unit * 128 + rl] = mm;
-          a.st_l[(int64_t)unit * 128 + rl] = ll;
-          a.st_t[(int64_t)unit * 128 + rl] = xch[2 * 128 + rl] + xch[5 * 128 + rl];
-        }
-      } else {
-        mbar_wait(smem_u32(&done_bar), 0);
-        tc_fence_after();
-        // unscaled partial dH block of this unit; the two groups split the d columns
-        float* dst = a.dpart + ((int64_t)unit * 128 + rl) * d;
-        const int dc = d / 2;
-        for (int c0 = grp * dc; c0 < (grp + 1) * dc; c0 += 16) {
-          float o[16];
-          if (NL > 0) {
-            tmem_ld16(tD + lane_sel + (uint32_t)c0, o);
-          } else {
+      mbar_wait(smem_u32(&done_bar), 0);
+      tc_fence_after();
+      // unscaled partial dH block of this unit; the two groups split the d columns
+      float* dst = a.dpart + ((int64_t)unit * 128 + rl) * d;
+      const int dc = d / 2;
+      for (int c0 = grp * dc; c0 < (grp + 1) * dc; c0 += 16) {
+        float o[16];
+        if (NL > 0) {
+          tmem_ld16(tD + lane_sel + (uint32_t)c0, o);
+        } else {
 #pragma unroll
-            for (int j = 0; j < 16; ++j) o[j] = 0.f;
-          }
-#pragma unroll
-          for (int j = 0; j < 16; j += 4) st4(dst + c0 + j, make_float4(o[j], o[j + 1], o[j + 2], o[j + 3]));
+          for (int j = 0; j < 16; ++j) o[j] = 0.f;
         }
+#pragma unroll
+        for (int j = 0; j < 16; j += 4) st4(dst + c0 + j, make_float4(o[j], o[j + 1], o[j + 2], o[j + 3]));
       }
     } else {
       // ------------------------------------------------------------------------------------------ DW: rows = vocabulary
@@ -854,26 +768,9 @@ __global__ void __launch_bounds__(256) dh_reduce_kernel(const float* __restrict_
   st4(dh_full + ((int64_t)rows[r] * d4 + c4) * 4, make_float4(s.x * mul, s.y * mul, s.z * mul, s.w * mul));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
 // [rows, d] fp16, box [box_rows x 64 columns], 128-byte swizzle; rows beyond the tensor read as zeros
 bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int d, int box_rows) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)d, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)d * sizeof(__half)};
@@ -882,43 +779,31 @@ bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int d, int box
   return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-bool wide_enabled() {
-  const char* e = getenv("RBM_CE_IMPL");
-  return !(e && strcmp(e, "mma") == 0);
-}
-int env_int(const char* name, int dflt) {
-  const char* e = getenv(name);
-  return e ? atoi(e) : dflt;
+// fp16 passes per product: 3 (hi.hi + hi.lo + lo.hi), or 1 (hi.hi) under RBM_CE_WIDE_PASSES=1, the reduced-precision line.
+// Read on every call, never cached: bench.py's labelled reduced-precision line and test_score_ce_wide_million_items set and
+// unset the variable inside one process, and a cached value would time or test the three-pass kernels under the wrong label.
+int wide_passes() {
+  const char* e = getenv("RBM_CE_WIDE_PASSES");
+  return e && atoi(e) == 1 ? 1 : 3;
 }
 struct Shape {
   int NV, ns, npass;
   size_t smem;
 };
-// streamed rows per chunk, ring depth, shared memory: FWD (and every mode at d = 128) keeps both resident halves in tensor
-// memory -> all shared memory is ring; DH / DW at d = 256 keep the resident lo half (64 KB) in shared memory
-Shape pick_shape(int d, int mode) {
+// streamed rows per chunk, ring depth, shared memory of the backward kernels: at d = 128 both resident halves are in tensor
+// memory -> all shared memory is ring; at d = 256 the resident lo half (64 KB) stays in shared memory
+Shape pick_shape(int d) {
   Shape s;
-  const bool lo_tmem = mode == MODE_FWD || d <= 128;
-  s.NV = env_int(mode == MODE_FWD ? "RBM_CE_WIDE_NV_FWD" : "RBM_CE_WIDE_NV", lo_tmem ? 64 : 48);
-  if (s.NV != 32 && s.NV != 48 && s.NV != 64) s.NV = lo_tmem ? 64 : 48;
+  const bool lo_tmem = d <= 128;
+  s.NV = lo_tmem ? 64 : 48;
   const size_t res = lo_tmem ? 0 : (size_t)(d / 64) * RBLK, stage = (size_t)2 * (d / 64) * s.NV * 128;
   int ns = (int)(((size_t)231000 - 1024 - res) / stage);
   s.ns = ns > 4 ? 4 : ns;
-  s.npass = env_int("RBM_CE_WIDE_PASSES", 3) == 1 ? 1 : 3;
+  s.npass = wide_passes();
   s.smem = res + (size_t)s.ns * stage + 1024;
   return s;
 }
 int64_t grid_units(int64_t cap128) { return cap128 / 128 > UMAX ? cap128 / 128 : UMAX; }
-
-template <typename K>
-bool set_smem(K kern, size_t bytes, const char* name) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
-    return false;
-  }
-  return true;
-}
 
 // workspace carve-up (floats): scales + bits (16) | W hi | W lo | Hc hi | Hc lo | fwd stats 3 x UG x 128 | dH partial UG x 128 x d
 struct WideWs {
@@ -966,18 +851,10 @@ int prepare(const float* h, const int32_t* rows, const int32_t* count, const flo
 
 }  // namespace
 
-// d = 64 is an experiment switch (RBM_CE_WIDE_D64=1): the 3xTF32 kernels of ce_tc.cu serve it by default
-static bool wide_d64() {
-  static const bool v = [] {
-    const char* e = getenv("RBM_CE_WIDE_D64");
-    return e && atoi(e) != 0;
-  }();
-  return v;
-}
-static bool wide_dim(int d) { return d == 128 || d == 256 || (d == 64 && wide_d64()); }
+static bool wide_dim(int d) { return d == 128 || d == 256; }
 
 bool rbm_ce_wide_supported(int V1, int d, const void* h, const void* w) {
-  if (!wide_enabled() || !wide_dim(d) || V1 < 64) return false;
+  if (!wide_dim(d) || V1 < 64) return false;
   if (((uintptr_t)h | (uintptr_t)w) & 15) return false;
   return get_encode() != nullptr;
 }
@@ -1001,32 +878,20 @@ int rbm_ce_wide_fwd(const float* h, const int32_t* rows, const int64_t* tgt, con
   const int64_t cap128 = (cap + 127) / 128 * 128;
   const WideWs ws = carve(extra_ws, cap, V1, d);
   if (int rc = prepare(h, rows, count, w, cap, V1, d, ws, st)) return rc;
-  const Shape sh = pick_shape(d, MODE_FWD);
-  CUtensorMap mRl, mSh, mSl;
-  if (!encode_map(&mRl, ws.h_lo, cap128, d, 128) || !encode_map(&mSh, ws.w_hi, V1, d, sh.NV) || !encode_map(&mSl, ws.w_lo, V1, d, sh.NV)) {
+  // 128-row vocabulary tiles through a ring of K-block pieces (N = 128 instructions)
+  CUtensorMap mSh, mSl;
+  if (!encode_map(&mSh, ws.w_hi, V1, d, 128) || !encode_map(&mSl, ws.w_lo, V1, d, 128)) {
     rbm_set_error("rbm_ce_fwd(wide): cuTensorMapEncodeTiled failed");
     return -1;
   }
   WideArgs a{};
   a.rows = rows; a.tgt = tgt; a.count = count; a.bias = bias; a.scales = ws.scales; a.st_m = ws.st_m; a.st_l = ws.st_l; a.st_t = ws.st_t;
   a.r_hi = (const __half*)ws.h_hi; a.r_lo = (const __half*)ws.h_lo; a.r_rows = cap128;
-  a.V1 = V1; a.d = d; a.KB = d / 64; a.NV = sh.NV; a.nstage = sh.ns; a.npass = sh.npass;
+  a.V1 = V1; a.d = d; a.KB = d / 64; a.npass = wide_passes();
   a.bias_vec = bias != nullptr && ((uintptr_t)bias & 15) == 0;
-  a.pair = env_int("RBM_CE_WIDE_PAIR", 0);  // interleaving two chunks' k-steps was measured slower (32 vs 24 ms)
-  if (env_int("RBM_CE_WIDE_FWD128", 1)) {  // 128-row vocabulary tiles through a ring of K-block pieces (N = 128 instructions)
-    CUtensorMap m128h, m128l;
-    if (!encode_map(&m128h, ws.w_hi, V1, d, 128) || !encode_map(&m128l, ws.w_lo, V1, d, 128)) {
-      rbm_set_error("rbm_ce_fwd(wide): cuTensorMapEncodeTiled failed");
-      return -1;
-    }
-    const size_t smem128 = (size_t)NPIECE * RBLK + 1024;
-    if (!set_smem(ce_wide_fwd128_kernel, smem128, "rbm_ce_fwd(wide 128)")) return -1;
-    a.NV = 128;
-    ce_wide_fwd128_kernel<<<(unsigned)grid_units(cap128), 64 + 32 * NSW, smem128, st>>>(m128h, m128l, a);
-  } else {
-    if (!set_smem(ce_wide_kernel<MODE_FWD>, sh.smem, "rbm_ce_fwd(wide)")) return -1;
-    ce_wide_kernel<MODE_FWD><<<(unsigned)grid_units(cap128), 64 + 32 * NSW, sh.smem, st>>>(mRl, mSh, mSl, a);
-  }
+  const size_t smem = (size_t)NPIECE * RBLK + 1024;
+  if (!set_smem(ce_wide_fwd128_kernel, smem, "rbm_ce_fwd(wide 128)")) return -1;
+  ce_wide_fwd128_kernel<<<(unsigned)grid_units(cap128), 64 + 32 * NSW, smem, st>>>(mSh, mSl, a);
   RBM_LAUNCH_CHECK("rbm_ce_fwd(wide)");
   const int nblk = (int)(cap128 / 128);
   fwd_combine_kernel<<<nblk, 128, 0, st>>>(ws.st_m, ws.st_l, ws.st_t, count, lse, partial);
@@ -1041,7 +906,7 @@ int rbm_ce_wide_bwd(const float* h, const int32_t* rows, const int64_t* tgt, con
   const int64_t cap128 = (cap + 127) / 128 * 128;
   const WideWs ws = carve(extra_ws, cap, V1, d);
   if (int rc = prepare(h, rows, count, w, cap, V1, d, ws, st)) return rc;
-  const Shape sh = pick_shape(d, MODE_DH);
+  const Shape sh = pick_shape(d);
   CUtensorMap mHlr, mWs, mWls, mWlr, mHs, mHls;
   if (!encode_map(&mHlr, ws.h_lo, cap128, d, 128) || !encode_map(&mWs, ws.w_hi, V1, d, sh.NV) || !encode_map(&mWls, ws.w_lo, V1, d, sh.NV) ||
       !encode_map(&mWlr, ws.w_lo, V1, d, 128) || !encode_map(&mHs, ws.h_hi, cap128, d, sh.NV) || !encode_map(&mHls, ws.h_lo, cap128, d, sh.NV)) {

@@ -136,6 +136,17 @@ inline void rbm_bind_context() {
   }
 }
 
+// raises a kernel's dynamic shared-memory limit; false, with the error recorded under `name`, when the runtime refuses
+template <typename K>
+inline bool set_smem(K kern, size_t bytes, const char* name) {
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e != cudaSuccess) {
+    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
+    return false;
+  }
+  return true;
+}
+
 // ---------------------------------------------------------------------------------------------
 // warp helpers
 // ---------------------------------------------------------------------------------------------

@@ -5,8 +5,6 @@
 //
 // Round-1 implementation: register-tiled SIMT fp32 GEMM (exact fp32 parity with the reference).  The tcgen05 /
 // TMEM path for these shapes is tracked in DESIGN.md ("next").
-#include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "tc_gemm.cuh"
 #include "tc_dw16.cuh"
@@ -294,16 +292,6 @@ __global__ void __launch_bounds__(256) epilogue_bwd_kernel(const float* __restri
   st4(dpre + i * 4, g);
 }
 
-// RBM_LINEAR_IMPL=simt forces the fp32 SIMT kernels (A/B testing); default: tcgen05 wherever the shape allows
-bool use_tc() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("RBM_LINEAR_IMPL");
-    v = (e && strcmp(e, "simt") == 0) ? 0 : 1;
-  }
-  return v == 1;
-}
-
 __global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict__ src, float* __restrict__ dst, int rows, int cols) {
   __shared__ float tile[32][33];
   int c = blockIdx.x * 32 + threadIdx.x, r0 = blockIdx.y * 32;
@@ -352,7 +340,7 @@ int tn_splits(int64_t M, int N, int K) {
 }  // namespace
 
 // wide layers with enough rows to fill the machine go to the split-fp16 tiled kernel (tc_gemm16.cu); N = output columns, K = contraction
-// length.  Measured at M = 102400 / 204800 (tools/dbg_gemm16.py): 1.5x .. 2.5x the 3xTF32 kernel from K = 256 up, slower at K = 128
+// length.  Measured at M = 102400 / 204800: 1.5x .. 2.5x the 3xTF32 kernel from K = 256 up, slower at K = 128
 // (two MMA k-blocks per unit cannot cover the epilogue)
 static bool gemm16_wanted(int64_t M, int N, int K) { return M >= 512 && N >= 128 && K >= 256; }
 
@@ -381,13 +369,13 @@ extern "C" int rbm_linear_fwd_ws(const float* x, int64_t ldx, const float* w, co
   RBM_REQUIRE(rbm_aligned16(x) && rbm_aligned16(w) && rbm_aligned16(y) && rbm_aligned16(bias) && rbm_aligned16(pre) && rbm_aligned16(residual),
               "rbm_linear_fwd: pointers must be 16B aligned");
   if (M == 0) return 0;
-  if (use_tc() && gemm16_wanted(M, N, K) && ws && rbm_aligned16(ws) && ws_bytes >= rbm_gemm16_ws_bytes(N, K) &&
+  if (gemm16_wanted(M, N, K) && ws && rbm_aligned16(ws) && ws_bytes >= rbm_gemm16_ws_bytes(N, K) &&
       rbm_gemm16_supported(M, N, K, ldx, x, w)) {
     RbmTcEpilogue te{y, ldy, pre, bias, residual, ldres, row_tok, act, rbm_drop_threshold(pA), rbm_drop_threshold(pB),
                      1.f / (1.f - pA), 1.f / (1.f - pB), siteA, siteB, seed};
     return rbm_gemm16_launch(x, ldx, w, M, N, K, te, ws, (cudaStream_t)stream);
   }
-  if (use_tc() && ldy % 4 == 0 && rbm_tc_linear_supported(M, N, K, ldx, x, w)) {
+  if (ldy % 4 == 0 && rbm_tc_linear_supported(M, N, K, ldx, x, w)) {
     RbmTcEpilogue te{y, ldy, pre, bias, residual, ldres, row_tok, act, rbm_drop_threshold(pA), rbm_drop_threshold(pB),
                      1.f / (1.f - pA), 1.f / (1.f - pB), siteA, siteB, seed};
     return rbm_tc_linear_launch(x, ldx, w, M, N, K, te, (cudaStream_t)stream);
@@ -429,7 +417,7 @@ extern "C" int rbm_linear_bwd_data(const float* dpre, int64_t lddpre, const floa
   if (M == 0) return 0;
   // dx = dpre . w  ==  dpre[M,N] . (w^T)[K,N]^T : the tcgen05 kernel wants both operands contraction-major, so the
   // (small) weight is transposed into the workspace first
-  if (use_tc() && ws && ws_bytes >= rbm_linear_bwd_data_ws_bytes(N, K) && rbm_aligned16(ws) &&
+  if (ws && ws_bytes >= rbm_linear_bwd_data_ws_bytes(N, K) && rbm_aligned16(ws) &&
       rbm_tc_linear_supported(M, K, N, lddpre, dpre, ws)) {
     float* wt = (float*)ws;
     dim3 tg((unsigned)rbm_cdiv(K, 32), (unsigned)rbm_cdiv(N, 32)), tb(32, 8);
@@ -469,7 +457,7 @@ extern "C" int rbm_linear_bwd_weight(const float* dpre, int64_t lddpre, const fl
   RBM_REQUIRE(lddpre % 4 == 0 && ldx % 4 == 0 && lddpre >= N && ldx >= K, "rbm_linear_bwd_weight: bad leading dimensions");
   RBM_REQUIRE(ws_bytes >= rbm_linear_bwd_weight_ws_bytes(M, N, K), "rbm_linear_bwd_weight: workspace too small");
   RBM_REQUIRE(rbm_aligned16(dpre) && rbm_aligned16(x) && rbm_aligned16(dw) && rbm_aligned16(ws), "rbm_linear_bwd_weight: pointers must be 16B aligned");
-  if (use_tc() && rbm_dw16_supported(M, N, K, lddpre, ldx, dpre, x)) {  // wide layers: split-fp16 tcgen05 kernel (tc_dw16.cu)
+  if (rbm_dw16_supported(M, N, K, lddpre, ldx, dpre, x)) {  // wide layers: split-fp16 tcgen05 kernel (tc_dw16.cu)
     const int S = rbm_dw16_splits(M, N, K);
     float* part = (float*)ws;
     float* part_b = part + (size_t)S * N * K;
@@ -480,7 +468,7 @@ extern "C" int rbm_linear_bwd_weight(const float* dpre, int64_t lddpre, const fl
     RBM_LAUNCH_CHECK("rbm_linear_bwd_weight(reduce)");
     return 0;
   }
-  if (use_tc() && rbm_tc_dw_supported(M, N, K, lddpre, ldx, dpre, x)) {
+  if (rbm_tc_dw_supported(M, N, K, lddpre, ldx, dpre, x)) {
     const int S = rbm_tc_dw_splits(M);
     float* part = (float*)ws;
     float* part_b = part + (size_t)S * N * K;

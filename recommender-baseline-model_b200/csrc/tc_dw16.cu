@@ -11,8 +11,6 @@
 //   * a CTA owns one [128 x KT] tile of dW and one slab of tokens; partial tiles are summed in fixed order by the caller
 //     (linear.cu, launch_reduce_splits): bit-deterministic, no atomics.
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
 #include "tc_dw16.cuh"
@@ -257,16 +255,12 @@ __global__ void dw16_scales_kernel(const unsigned* __restrict__ bits, float* __r
   scales[i] = ldexpf(1.f, 15 - e);
 }
 
-bool dw16_enabled() {
-  const char* e = getenv("RBM_LINEAR_DW16");
-  return !(e && atoi(e) == 0);
-}
 int tile_k(int K) { return K % 256 == 0 ? 256 : 128; }
 
 }  // namespace
 
 bool rbm_dw16_supported(int64_t M, int N, int K, int64_t lda, int64_t ldb, const void* a, const void* b) {
-  if (!dw16_enabled() || M < 1 || N % 128 != 0 || K % 128 != 0) return false;
+  if (M < 1 || N % 128 != 0 || K % 128 != 0) return false;
   if (!(N > 256 || K > 256 || (N == 256 && K == 256))) return false;  // smaller layers: tc_dw_kernel (one pass over the operands)
   if (lda % 4 != 0 || ldb % 4 != 0 || ((uintptr_t)a & 15) || ((uintptr_t)b & 15)) return false;
   return true;

@@ -1,15 +1,8 @@
-// tc_gemm.cu -- Blackwell-native GEMM for the Linear layers:  D[M,N] = A[M,K] . B[N,K]^T  (+ fused epilogue)
-//   * operands stay fp32 in HBM and are consumed as TF32 by tcgen05.mma (kind::tf32, fp32 accumulation in TMEM);
-//   * A and B tiles are staged by TMA (cp.async.bulk.tensor.2d, 128-byte swizzle, K-major) into a ring of
-//     shared-memory stages guarded by full/empty mbarriers;
-//   * warp-specialised CTA: warp 0 = TMA producer, warp 1 = TMEM allocator + single-thread MMA issuer,
-//     warps 2..5 = epilogue (tcgen05.ld 32x32b: one accumulator row per thread) applying
-//     bias / GELU-ReLU / dropout / residual / dropout / pad-row zeroing and writing y (and the pre-activation).
-// One CTA per (128-row M tile, N tile <= 256).  Used by rbm_linear_fwd and rbm_linear_bwd_data (with the weight
-// transposed by the caller); shapes that do not meet the TMA/UMMA constraints take the SIMT kernels of linear.cu.
-#include <stdlib.h>
-#include <string.h>
-#include <cuda.h>  // CUtensorMap types only; the encode function is fetched at run time (no libcuda link dependency)
+// tc_gemm.cu -- Blackwell-native GEMM for the Linear layers:  D[M,N] = A[M,K] . B[N,K]^T  (+ fused epilogue), and the weight
+// gradient dW = dpre^T . x.  Operands stay fp32 in HBM; TMA (cp.async.bulk.tensor.2d, 128-byte swizzle) stages them into shared
+// memory and tcgen05.mma consumes them as TF32 (kind::tf32, fp32 accumulation in TMEM), with the TF32 residuals of the operands
+// as extra products (3xTF32) for fp32-level accuracy.  The forward kernel serves rbm_linear_fwd and rbm_linear_bwd_data (with the weight transposed by the
+// caller); shapes that do not meet the TMA/UMMA constraints take the SIMT kernels of linear.cu.
 #include "common.cuh"
 #include "tc_gemm.cuh"
 #include "tc_ptx.cuh"
@@ -21,12 +14,6 @@ using namespace rbm_tc;
 constexpr int BM = 128;      // UMMA_M (cta_group::1)
 constexpr int BKE = 32;      // K elements per stage = one 128-byte swizzle row of fp32/tf32
 constexpr int UMMA_K = 8;    // tf32
-
-__device__ __forceinline__ float act_apply(float v, int act) {
-  if (act == RBM_ACT_RELU) return fmaxf(v, 0.f);
-  if (act == RBM_ACT_GELU_TANH) return gelu_tanh_f(v);
-  return v;
-}
 
 struct TcParams {
   float* y;
@@ -46,116 +33,8 @@ struct TcParams {
   uint32_t tmem_cols;
 };
 
-__global__ void __launch_bounds__(192, 1) tc_linear_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                                                           const TcParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t full_bar[16], empty_bar[16], tmem_full_bar;
-  __shared__ uint32_t tmem_base_slot;
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t m0 = (int64_t)blockIdx.x * BM;
-  const int n0 = blockIdx.y * p.BN;
-  const int KB = p.K / BKE;
-  const uint32_t a_bytes = BM * BKE * 4, b_bytes = (uint32_t)p.BN * BKE * 4, stage_bytes = a_bytes + b_bytes;
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;  // 128B-swizzle atoms need 1024-byte alignment
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.nstage; ++s) {
-      mbar_init(smem_u32(&full_bar[s]), 1);
-      mbar_init(smem_u32(&empty_bar[s]), 1);
-    }
-    mbar_init(smem_u32(&tmem_full_bar), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) tmem_alloc(smem_u32(&tmem_base_slot), p.tmem_cols);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_d = tmem_base_slot;
-
-  if (warp == 0) {
-    if (elect_one()) {
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&mapA) : "memory");
-      asm volatile("prefetch.tensormap [%0];" ::"l"(&mapB) : "memory");
-      for (int kb = 0; kb < KB; ++kb) {
-        const int s = kb % p.nstage;
-        if (kb >= p.nstage) mbar_wait(smem_u32(&empty_bar[s]), ((kb / p.nstage) - 1) & 1);
-        const uint32_t bar = smem_u32(&full_bar[s]);
-        const uint32_t sa = smem_base + s * stage_bytes;
-        mbar_expect_tx(bar, stage_bytes);
-        tma_load_2d(sa, &mapA, bar, kb * BKE, (int)m0);
-        tma_load_2d(sa + a_bytes, &mapB, bar, kb * BKE, n0);
-      }
-    }
-  } else if (warp == 1) {
-    if (elect_one()) {
-      const uint32_t idesc = make_idesc_tf32(BM, p.BN);
-      for (int kb = 0; kb < KB; ++kb) {
-        const int s = kb % p.nstage;
-        mbar_wait(smem_u32(&full_bar[s]), (kb / p.nstage) & 1);
-        tc_fence_after();
-        const uint32_t sa = smem_base + s * stage_bytes;
-        const uint64_t adesc = make_sw128_desc(sa), bdesc = make_sw128_desc(sa + a_bytes);
-#pragma unroll
-        for (int k = 0; k < BKE / UMMA_K; ++k)  // +32 bytes (>>4 = 2) per UMMA_K step inside the 128-byte swizzle row
-          umma_tf32(tmem_d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0);
-        umma_commit(smem_u32(&empty_bar[s]));  // stage is free once these MMAs have read it
-      }
-      umma_commit(smem_u32(&tmem_full_bar));   // accumulator complete
-    }
-    __syncwarp();
-  } else {
-    // ---- epilogue: warp w may touch TMEM lanes [32*(w%4), +32); thread <-> accumulator row
-    const int q = warp & 3;
-    const int64_t row = m0 + q * 32 + lane;
-    mbar_wait(smem_u32(&tmem_full_bar), 0);
-    tc_fence_after();
-    const bool live = row < p.M;
-    const bool keep_row = !(p.row_tok && live && p.row_tok[row] == 0);
-    for (int c0 = 0; c0 < p.BN; c0 += 32) {
-      float v[32];
-      tmem_ld32(tmem_d + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, v);  // warp-collective: all lanes take part
-      if (!live) continue;
-      const int col0 = n0 + c0;
-#pragma unroll
-      for (int j = 0; j < 32; j += 4) {
-        const int col = col0 + j;
-        if (col >= p.N) break;
-        float4 x = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-        if (p.bias) {
-          float4 b = ld4(p.bias + col);
-          x.x += b.x; x.y += b.y; x.z += b.z; x.w += b.w;
-        }
-        if (p.pre) st4(p.pre + row * p.N + col, x);
-        x.x = act_apply(x.x, p.act); x.y = act_apply(x.y, p.act); x.z = act_apply(x.z, p.act); x.w = act_apply(x.w, p.act);
-        const uint64_t e4 = (uint64_t)(row * p.N + col) >> 2;
-        if (p.thrA) {
-          float4 m = rbm_drop4(p.seed, rbm_site(p.siteA), e4, p.thrA, p.invA);
-          x.x *= m.x; x.y *= m.y; x.z *= m.z; x.w *= m.w;
-        }
-        if (p.residual) {
-          float4 r = ld4(p.residual + row * p.ldres + col);
-          x.x += r.x; x.y += r.y; x.z += r.z; x.w += r.w;
-        }
-        if (p.thrB) {
-          float4 m = rbm_drop4(p.seed, rbm_site(p.siteB), e4, p.thrB, p.invB);
-          x.x *= m.x; x.y *= m.y; x.z *= m.z; x.w *= m.w;
-        }
-        if (!keep_row) x = make_float4(0.f, 0.f, 0.f, 0.f);
-        st4(p.y + row * p.ldy + col, x);
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_d, p.tmem_cols);
-  }
-}
-
 // =====================================================================================================
-// v2: persistent, weight-resident, 3xTF32.
+// Forward: persistent, weight-resident, 3xTF32.
 //   * one persistent CTA per SM walks M tiles (tile = blockIdx.x + i*gridDim.x);
 //   * the whole weight B[N<=256, K] is TMA-loaded ONCE per CTA and stays in shared memory (raw + lo copy);
 //   * A streams through a ring of 32-wide K-block stages; two "split" warps derive A_lo = A - trunc_tf32(A) next to
@@ -168,7 +47,6 @@ __global__ void __launch_bounds__(192, 1) tc_linear_kernel(const __grid_constant
 // alternating 32-column chunks).
 // =====================================================================================================
 constexpr int STG_LD = 32;  // staging tile: 32x32 floats per warp, 16-byte chunks XOR-swizzled by (row & 7): conflict-free both ways
-
 
 // dst = src - trunc_tf32(src), elementwise over n4 float4 (layout-agnostic: the swizzle is preserved)
 __device__ __forceinline__ void split_lo(const float* src, float* dst, int n4, int tid, int nthr) {
@@ -579,28 +457,9 @@ __global__ void __launch_bounds__(192, 1) tc_dw_kernel(const __grid_constant__ C
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
-
 // 2-D fp32 tensor [rows, cols] with row stride ld (elements); box = [box_rows, 32 cols], 128-byte swizzle
 bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(float)};
@@ -611,26 +470,9 @@ bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int64_t cols,
   return r == CUDA_SUCCESS;
 }
 
-int pick_bn(int N) {
-  if (N <= 256) return N;
-  for (int bn = 256; bn >= 16; bn -= 16)
-    if (N % bn == 0) return bn;
-  return 0;
-}
-
 }  // namespace
 
-// mode: 0 = auto (v2 persistent 3xTF32 when it fits, else refuse), 1 = v1 single-pass TF32 (RBM_LINEAR_IMPL=tf32x1)
-static int tc_mode() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("RBM_LINEAR_IMPL");
-    v = (e && strcmp(e, "tf32x1") == 0) ? 1 : 0;
-  }
-  return v;
-}
-
-static bool v2_fits(int N, int K, int* nstage_out) {
+static bool weight_fits(int N, int K, int* nstage_out) {
   if (N > 256) return false;
   const size_t b_bytes = (size_t)N * K * 4, a_stage = (size_t)2 * BM * BKE * 4, stg = (size_t)EPI_WARPS * 32 * STG_LD * 4;
   const size_t budget = (size_t)231424 - 1024;  // 227 KB per block minus static barriers and alignment slack
@@ -648,7 +490,7 @@ static int pick_groups(int N, int K, int* nstage_out) {
   //  runs as two groups with four stages instead of one group with two -- changed nothing: 138 vs 134 us, tools/time_linear_cfg2.py)
   for (int ng = 1; ng <= 32; ++ng) {
     if (N % ng != 0 || (N / ng) % 16 != 0) continue;
-    if (v2_fits(N / ng, K, nstage_out)) return ng;
+    if (weight_fits(N / ng, K, nstage_out)) return ng;
   }
   return 0;
 }
@@ -658,8 +500,7 @@ bool rbm_tc_linear_supported(int64_t M, int N, int K, int64_t lda, const void* a
   if (lda % 4 != 0 || ((uintptr_t)a & 15) || ((uintptr_t)b & 15)) return false;
   if (get_encode() == nullptr) return false;
   int ns;
-  if (tc_mode() == 0) return pick_groups(N, K, &ns) != 0;
-  return pick_bn(N) != 0;
+  return pick_groups(N, K, &ns) != 0;
 }
 
 static int launch_single(const float* a, int64_t lda, const float* b, int64_t ldb, int64_t M, int N, int K, const RbmTcEpilogue& ep,
@@ -672,8 +513,7 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
 int rbm_tc_linear_launch(const float* a, int64_t lda, const float* b, int64_t M, int N, int K, const RbmTcEpilogue& ep,
                          cudaStream_t st) {
   constexpr int KC = 256;
-  const char* e = getenv("RBM_LINEAR_SPLITK");
-  if (tc_mode() == 0 && !(e && atoi(e) == 0) && K > KC && K % KC == 0) {
+  if (K > KC && K % KC == 0) {
     int ns, ns2;
     const int ng = pick_groups(N, K, &ns), ng2 = pick_groups(N, KC, &ns2);
     if (ng > 0 && ng2 > 0 && N / ng < 64 && N / ng2 >= 64) {
@@ -693,14 +533,13 @@ int rbm_tc_linear_launch(const float* a, int64_t lda, const float* b, int64_t M,
 
 static int launch_single(const float* a, int64_t lda, const float* b, int64_t ldb, int64_t M, int N, int K, const RbmTcEpilogue& ep,
                          const float* acc_in, cudaStream_t st) {
-  const bool v2 = tc_mode() == 0;
-  int ns_v2 = 2;
-  const int NG = v2 ? pick_groups(N, K, &ns_v2) : 1;
-  const int BN = v2 ? N / (NG > 0 ? NG : 1) : pick_bn(N);
-  if (BN <= 0 || NG <= 0) {
+  int ns;
+  const int NG = pick_groups(N, K, &ns);
+  if (NG <= 0) {
     rbm_set_error("rbm_linear(tcgen05): no resident-weight split for N=%d K=%d", N, K);
     return -1;
   }
+  const int BN = N / NG;
   CUtensorMap mapA, mapB;
   if (!encode_map(&mapA, a, M, K, lda, BM) || !encode_map(&mapB, b, N, K, ldb, BN)) {
     rbm_set_error("rbm_linear(tcgen05): cuTensorMapEncodeTiled failed (M=%lld N=%d K=%d lda=%lld)", (long long)M, N, K, (long long)lda);
@@ -712,7 +551,7 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
   p.thrA = ep.thrA; p.thrB = ep.thrB; p.invA = ep.invA; p.invB = ep.invB; p.siteA = ep.siteA; p.siteB = ep.siteB; p.seed = ep.seed;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tc_linear_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024);
+    cudaError_t e = cudaSuccess;
     // every (activation, dropout A, dropout B) variant of the persistent kernel
 #define RBM_TC_ATTR(A, DA, DB) \
     if (e == cudaSuccess) e = cudaFuncSetAttribute(tc_linear_persistent_kernel<A, DA, DB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
@@ -726,49 +565,33 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
     }
     attr_set = true;
   }
-  if (v2) {
-    const int ns = ns_v2;
-    p.nstage = ns;
-    uint32_t cols = 32;
-    while (cols < (uint32_t)(2 * BN) || cols < (uint32_t)(BN + ((BN + 31) & ~31))) cols <<= 1;  // the epilogue reads whole 32-column chunks
-    p.tmem_cols = cols;
-    size_t smem = (size_t)2 * BN * K * 4 + (size_t)ns * 2 * BM * BKE * 4 + (size_t)EPI_WARPS * 32 * STG_LD * 4 + 1024;
-    int tiles = (int)rbm_cdiv(M, BM);
-    int per_group = RBM_NUM_SMS / NG;  // CTAs per column group (one CTA per SM in total)
-    if (per_group > tiles) per_group = tiles;
-    int grid = per_group * NG;
-    const int act = p.act != 0 ? p.act : (p.pre != nullptr ? 3 : 0);  // 3: no activation, pre-activation still stored
-    const bool da = p.thrA != 0, db = p.thrB != 0;
-    const int nthr = 128 + 32 * EPI_WARPS;
+  p.nstage = ns;
+  uint32_t cols = 32;
+  while (cols < (uint32_t)(2 * BN) || cols < (uint32_t)(BN + ((BN + 31) & ~31))) cols <<= 1;  // the epilogue reads whole 32-column chunks
+  p.tmem_cols = cols;
+  size_t smem = (size_t)2 * BN * K * 4 + (size_t)ns * 2 * BM * BKE * 4 + (size_t)EPI_WARPS * 32 * STG_LD * 4 + 1024;
+  int tiles = (int)rbm_cdiv(M, BM);
+  int per_group = RBM_NUM_SMS / NG;  // CTAs per column group (one CTA per SM in total)
+  if (per_group > tiles) per_group = tiles;
+  int grid = per_group * NG;
+  const int act = p.act != 0 ? p.act : (p.pre != nullptr ? 3 : 0);  // 3: no activation, pre-activation still stored
+  const bool da = p.thrA != 0, db = p.thrB != 0;
+  const int nthr = 128 + 32 * EPI_WARPS;
 #define RBM_TC_GO(A, DA, DB) tc_linear_persistent_kernel<A, DA, DB><<<grid, nthr, smem, st>>>(mapA, mapB, p)
-#define RBM_TC_GO4(A)                     \
-    do {                                  \
-      if (da && db) RBM_TC_GO(A, true, true);       \
-      else if (da) RBM_TC_GO(A, true, false);       \
-      else if (db) RBM_TC_GO(A, false, true);       \
-      else RBM_TC_GO(A, false, false);              \
-    } while (0)
-    if (act == 0) RBM_TC_GO4(0);
-    else if (act == RBM_ACT_RELU) RBM_TC_GO4(1);
-    else if (act == RBM_ACT_GELU_TANH) RBM_TC_GO4(2);
-    else RBM_TC_GO4(3);
+#define RBM_TC_GO4(A)                       \
+  do {                                      \
+    if (da && db) RBM_TC_GO(A, true, true); \
+    else if (da) RBM_TC_GO(A, true, false); \
+    else if (db) RBM_TC_GO(A, false, true); \
+    else RBM_TC_GO(A, false, false);        \
+  } while (0)
+  if (act == 0) RBM_TC_GO4(0);
+  else if (act == RBM_ACT_RELU) RBM_TC_GO4(1);
+  else if (act == RBM_ACT_GELU_TANH) RBM_TC_GO4(2);
+  else RBM_TC_GO4(3);
 #undef RBM_TC_GO4
 #undef RBM_TC_GO
-    RBM_LAUNCH_CHECK("rbm_linear(tcgen05 persistent)");
-    return 0;
-  }
-  const uint32_t stage_bytes = (uint32_t)(BM + BN) * BKE * 4;
-  int nstage = (int)((200u * 1024u) / stage_bytes);
-  if (nstage > K / BKE) nstage = K / BKE;
-  if (nstage > 16) nstage = 16;
-  p.nstage = nstage;
-  uint32_t cols = 32;
-  while (cols < (uint32_t)BN) cols <<= 1;
-  p.tmem_cols = cols;
-  size_t smem = (size_t)nstage * stage_bytes + 1024;
-  dim3 grid((unsigned)rbm_cdiv(M, BM), (unsigned)(N / BN));
-  tc_linear_kernel<<<grid, 192, smem, st>>>(mapA, mapB, p);
-  RBM_LAUNCH_CHECK("rbm_linear(tcgen05)");
+  RBM_LAUNCH_CHECK("rbm_linear(tcgen05 persistent)");
   return 0;
 }
 
@@ -776,7 +599,6 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
 namespace {
 bool encode_map_mn(CUtensorMap* map, const float* base, int64_t rows, int64_t cols, int64_t ld) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(float)};
@@ -809,7 +631,7 @@ int rbm_tc_dw_splits(int64_t M) {
 bool rbm_tc_dw_bias_fused(int N, int K) { return dw_wide(N, K, true) || ((N + BM - 1) / BM) * (K + DW_BIAS_N) <= 512; }
 
 bool rbm_tc_dw_supported(int64_t M, int N, int K, int64_t lda, int64_t ldb, const void* a, const void* b) {
-  if (tc_mode() != 0 || M < 1 || N % 32 != 0 || K % 32 != 0 || N > 256 || K > 256 || K < 32 || N < 32) return false;
+  if (M < 1 || N % 32 != 0 || K % 32 != 0 || N > 256 || K > 256 || K < 32 || N < 32) return false;
   if (lda % 4 != 0 || ldb % 4 != 0 || ((uintptr_t)a & 15) || ((uintptr_t)b & 15)) return false;
   int mt;
   if (dw_stages(N, K, &mt) < 2 || mt * K > 512) return false;

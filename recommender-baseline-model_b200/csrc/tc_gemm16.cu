@@ -14,9 +14,6 @@
 //     the MMAs of unit n + 1 run.  The epilogue is the arithmetic of tc_gemm.cu's (same Philox element indexing: the
 //     backward regenerates the masks).
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
-#include <cuda.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
 #include "tc_gemm.cuh"
@@ -306,25 +303,8 @@ __global__ void __launch_bounds__(256) g16_split_kernel(const float* __restrict_
   lo[i] = make_uint2((uint32_t)l[0] | ((uint32_t)l[1] << 16), (uint32_t)l[2] | ((uint32_t)l[3] << 16));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode16() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
 bool encode_half(CUtensorMap* map, const void* base, int64_t rows, int cols) {
-  EncodeTiledFn enc = get_encode16();
-  rbm_bind_context();
+  EncodeTiledFn enc = get_encode();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)cols * 2};
@@ -334,7 +314,7 @@ bool encode_half(CUtensorMap* map, const void* base, int64_t rows, int cols) {
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 bool encode_a32(CUtensorMap* map, const void* base, int64_t rows, int cols, int64_t ld) {
-  EncodeTiledFn enc = get_encode16();
+  EncodeTiledFn enc = get_encode();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * 4};
@@ -343,17 +323,13 @@ bool encode_a32(CUtensorMap* map, const void* base, int64_t rows, int cols, int6
   return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-bool g16_enabled() {
-  const char* e = getenv("RBM_LINEAR_GEMM16");
-  return !(e && atoi(e) == 0);
-}
 
 }  // namespace
 
 bool rbm_gemm16_supported(int64_t M, int N, int K, int64_t lda, const void* a, const void* b) {
-  if (!g16_enabled() || M < 1 || N < 128 || K < 128 || N % 128 != 0 || K % 64 != 0) return false;
+  if (M < 1 || N < 128 || K < 128 || N % 128 != 0 || K % 64 != 0) return false;
   if (lda % 4 != 0 || ((uintptr_t)a & 15) || ((uintptr_t)b & 15)) return false;
-  return get_encode16() != nullptr;
+  return get_encode() != nullptr;
 }
 
 size_t rbm_gemm16_ws_bytes(int N, int K) { return (size_t)N * K * 4 + 256; }  // weight hi + lo (2 B each) + max-abs bits + scales

@@ -1,12 +1,20 @@
 // tc_ptx.cuh -- inline-PTX wrappers for the Blackwell (sm_100a) async/tensor path: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (alloc/mma/commit/ld/st/fences) and UMMA shared-memory / instruction descriptors.
+// tcgen05 (alloc/mma/commit/ld/st/fences) and UMMA shared-memory / instruction descriptors; plus the host-side lookup of the
+// tensor-map encoder.
 #pragma once
-#include <cuda.h>
+#include <cuda.h>  // CUtensorMap types only; the encode function is fetched at run time (no libcuda link dependency)
 #include "common.cuh"
 
 namespace rbm_tc {
 
 constexpr int UMMA_K_TF32 = 8;
+
+// cuTensorMapEncodeTiled from the driver, looked up once per process (tc_encode.cu); nullptr when the driver lacks it.  Every call
+// also binds the calling thread to the primary context (rbm_bind_context), which the encode needs.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn get_encode();
 
 // ------------------------------------------------------------------------------------------------ PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }

@@ -26,7 +26,6 @@
 //     score is the sequential FMA over the hidden dimension (the arithmetic of stage 2 and of the scan kernel).
 #include <cuda_fp16.h>
 #include <stdlib.h>
-#include <string.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
 #include "tc_topk.cuh"
@@ -402,25 +401,8 @@ __global__ void __launch_bounds__(256) maxabs_rows_kernel(const float* __restric
   if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* sym = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = (EncodeTiledFn)sym;
-  }
-  return fn;
-}
 bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16) {
   EncodeTiledFn enc = get_encode();
-  rbm_bind_context();
   if (!enc) return false;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * (f16 ? 2 : 4)};
@@ -428,14 +410,6 @@ bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, 
   cuuint32_t estr[2] = {1, 1};
   return enc(map, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-bool tc_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("RBM_TOPK_IMPL");
-    v = (e && strcmp(e, "simt") == 0) ? 0 : 1;
-  }
-  return v == 1;
 }
 // d <= 64: two 128-user sub-tiles per unit against 128-item tiles (every streamed tile is used by 256 users: the kernel is
 // L2-bandwidth bound, and this halves the item-table traffic); larger d: one sub-tile
@@ -450,7 +424,6 @@ int pick_bn(int d) { return d <= 128 ? 128 : 64; }
 // 4 splits 6.2 ms, 7 splits 8.4 ms).
 int rbm_tc_topk_splits(int64_t U, int64_t n_items, int d) {
   int64_t ut = rbm_cdiv(U, BM * pick_nst(d)), tiles = rbm_cdiv(n_items, pick_bn(d));
-  if (const char* e = getenv("RBM_TOPK_SPLITS")) return atoi(e) < 1 ? 1 : atoi(e);  // bring-up override
   // Units = user tiles x splits run in waves of one CTA per SM: pick the split count with the best (wave fill) x (1 - list
   // warm-up cost), the warm-up cost of a split being ~10^5 items' worth of slow-path insertions (fitted to the measurements
   // above: 16384 users x 10^7 items -> 9 splits, 576 units = 3.9 waves; x 10^6 items -> 2 splits)
@@ -482,10 +455,7 @@ static size_t cand_bytes(int64_t U, int64_t n_items, int d) {
   size_t S = (size_t)rbm_tc_topk_splits(U, n_items, d);
   return S * 2 * (size_t)U * KC * (sizeof(float) + sizeof(int64_t));
 }
-static bool use_f16(int d) {
-  if (const char* e = getenv("RBM_TOPK_F16")) return atoi(e) != 0 && d % 64 == 0;
-  return d % 64 == 0;
-}
+static bool use_f16(int d) { return d % 64 == 0; }
 static size_t half_bytes(int64_t U, int64_t n_items, int d) {  // fp16 copies: item rows [n_items, d], user rows [U padded to 128, d]
   if (!use_f16(d)) return 0;
   return (((size_t)n_items * d * 2 + 255) & ~(size_t)255) + (size_t)rbm_cdiv(U, 128) * 128 * d * 2 + 256;
@@ -498,7 +468,7 @@ size_t rbm_tc_topk_ws_bytes(int64_t U, int64_t n_items, int d, int k) {
 }
 
 bool rbm_tc_topk_supported(int64_t U, int64_t n_items, int d, int k, int64_t ldf, const void* f, const void* table) {
-  if (!tc_enabled() || d % 32 != 0 || d < 32 || d > 256 || k > KC - 6 || U < 1) return false;  // k <= 10: six spare list slots (larger k: exact fp32 scan kernel)
+  if (d % 32 != 0 || d < 32 || d > 256 || k > KC - 6 || U < 1) return false;  // k <= 10: six spare list slots (larger k: exact fp32 scan kernel)
   if (n_items < 8192) return false;  // small catalogues: the fp32 tile kernel is already latency-bound
   if (ldf % 4 != 0 || ((uintptr_t)f & 15) || ((uintptr_t)table & 15)) return false;
   return get_encode() != nullptr;
@@ -585,7 +555,9 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
   RBM_LAUNCH_CHECK("rbm_score_topk(tcgen05)");
   // 2^-10 (two rounded fp16 operands) resp. 2^-9 (two truncated TF32 operands) per product, plus the fp32 accumulation slack
   float eps_mul = f16 ? 1.05e-3f : 2.1e-3f;
-  if (const char* e = getenv("RBM_TOPK_EPS")) eps_mul = (float)atof(e);  // tests: a huge value sends every user through stage 3
+  // RBM_TOPK_EPS overrides the bound: test_score_topk_fused sets a huge value to send every user through the exact re-scan.  Read on
+  // every call, never cached, because the test sets and unsets it inside one process.
+  if (const char* e = getenv("RBM_TOPK_EPS")) eps_mul = (float)atof(e);
   topk_rescore_kernel<<<(unsigned)rbm_cdiv(U, 8), 256, 8 * d * sizeof(float), st>>>(f, ldf, table, bias, p.cand_i, p.cand_s, p.nst == 2 ? p.S : p.S * 2,
                                                                                    id_offset, top_scores, top_ids, U, d, k, bits, eps_mul,
                                                                                    f16 ? scales : nullptr, flag_list, flag_count);

@@ -8,5 +8,3 @@ timeout 300 python tools/dbg_ce_wide.py check > gpurun_out/r2c_ce_check.log 2>&1
 tail -20 gpurun_out/r2c_ce_check.log
 timeout 300 python tools/dbg_ce_wide.py time > gpurun_out/r2c_ce_time.log 2>&1
 tail -20 gpurun_out/r2c_ce_time.log
-RBM_CE_WIDE_NV=32 timeout 300 python tools/dbg_ce_wide.py time > gpurun_out/r2c_ce_time_nv32.log 2>&1
-tail -20 gpurun_out/r2c_ce_time_nv32.log

@@ -1,5 +1,5 @@
 """Per-entry-point device times of the four Linear layers of a BERT4Rec configs[1] block (M = 1024 x 200 rows, d = 64), forward and
-backward, with the epilogues the model uses.  Used to compare kernel choices (RBM_LINEAR_DEEP, RBM_LINEAR_GEMM16, ...)."""
+backward, with the epilogues the model uses.  Used to compare kernel choices: run it on each build and compare."""
 import sys
 import torch
 sys.path.insert(0, ".")
