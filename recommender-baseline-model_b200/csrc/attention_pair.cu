@@ -21,16 +21,18 @@
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E
 #include "tc_ptx.cuh"
+#include "split16.cuh"
+#include "attention_f16.cuh"
 #include "attention_pair.cuh"
 #include "attention_tc.cuh"  // rbm_attn_tc_enabled
 
 namespace {
 
 using namespace rbm_tc;
+using namespace rbm_attn16;
 using rbm_mma::ex2;
 
 constexpr int DK = 64;
-constexpr int THREADS = 256;
 constexpr uint32_t TILE = 128 * 128;  // [128 rows x 64 fp16] = 16 KB
 enum { T_QH = 0, T_QL, T_KH, T_KL, T_VH, T_VL, T_GH, T_GL };
 
@@ -43,58 +45,6 @@ struct PairArgs {
   uint32_t thr16;
   uint64_t seed, site;
 };
-
-// ------------------------------------------------------------------------------------------------ PTX (kind::f16)
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N, int b_mn) {
-  return (1u << 4) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// MN-major view of a [rows = K][128 B = 64 MN elements] 128-byte-swizzled tile of 16-bit elements (see ce_wide.cu)
-__device__ __forceinline__ uint64_t make_sw128_desc_mn16(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)(1024 >> 4) << 16;  // one 64-element MN block: the leading offset is never applied
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]),
-               "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-               : "memory");
-}
-__device__ __forceinline__ void split_pack16(const float (&g)[16], uint32_t (&hi)[8], uint32_t (&lo)[8]) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const __half h0 = __float2half_rn(g[2 * j]), h1 = __float2half_rn(g[2 * j + 1]);
-    const __half l0 = __float2half_rn(g[2 * j] - __half2float(h0)), l1 = __float2half_rn(g[2 * j + 1] - __half2float(h1));
-    hi[j] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-    lo[j] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-  }
-}
-// power of two that brings a maximum magnitude m into [2^13, 2^14)
-__device__ __forceinline__ float pow2_scale(float m) {
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  return ldexpf(1.f, 14 - e);
-}
 
 // ------------------------------------------------------------------------------------------------ tile staging
 // One [128 x 64] tile = the rows of both items of the pair (item s in rows [64 s, 64 s + L); the rest zero).  Thread task
@@ -119,46 +69,10 @@ __device__ __forceinline__ float tile_fetch(float (&v)[4][8], const float* __res
   }
   return mx;
 }
-// scale, split and store into the hi / lo tiles (128-byte swizzle: 16-byte chunk c of row r lands at chunk c ^ (r & 7))
-__device__ __forceinline__ void tile_store(const float (&v)[4][8], float sc, uint8_t* hi, uint8_t* lo) {
-#pragma unroll
-  for (int it = 0; it < 4; ++it) {
-    const int task = it * THREADS + (int)threadIdx.x, r = task >> 3, c = task & 7;
-    uint32_t h[4], l[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float x0 = v[it][2 * e] * sc, x1 = v[it][2 * e + 1] * sc;
-      const __half h0 = __float2half_rn(x0), h1 = __float2half_rn(x1);
-      const __half l0 = __float2half_rn(x0 - __half2float(h0)), l1 = __float2half_rn(x1 - __half2float(h1));
-      h[e] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-      l[e] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-    }
-    const uint32_t off = (uint32_t)r * 128u + (uint32_t)((c ^ (r & 7)) << 4);
-    *reinterpret_cast<uint4*>(hi + off) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo + off) = make_uint4(l[0], l[1], l[2], l[3]);
-  }
-}
-// this thread's share of the tile maximum -> block maximum (shared-memory atomicMax on the bit pattern: order-independent)
-__device__ __forceinline__ void tile_max(float mx, unsigned* maxbits) {
-  mx = warp_max(mx);
-  if ((threadIdx.x & 31) == 0 && mx > 0.f) atomicMax(maxbits, __float_as_uint(mx));
-}
-__device__ __forceinline__ float tile_scale_of(const unsigned* maxbits) { return pow2_scale(__uint_as_float(*maxbits)); }
+__device__ __forceinline__ float tile_scale_of(const unsigned* maxbits) { return pow2_scale(__uint_as_float(*maxbits), 14); }
 
-// 3-pass products.  SS: D = A_tile . B_tile^T (both K-major, contraction over d_k = 64: four k-steps of 16)
-__device__ __forceinline__ void mma_ss3(uint32_t d_t, uint32_t a_hi, uint32_t a_lo, uint32_t b_hi, uint32_t b_lo, uint32_t idesc) {
-  uint32_t acc = 0;
-#pragma unroll
-  for (int pass = 0; pass < 3; ++pass) {
-    const uint64_t ad = make_sw128_desc(pass == 2 ? a_lo : a_hi), bd = make_sw128_desc(pass == 1 ? b_lo : b_hi);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      umma_f16(d_t, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), idesc, acc);
-      acc = 1;
-    }
-  }
-}
-// TS: D[128 x 64] = A (tensor memory, K = 128 tokens: hi words at a_t, lo words at a_t + 64) . B_tile (MN-major view)
+// D[128 x 64] = A (tensor memory, K = 128 tokens: hi words at a_t, lo words at a_t + 64) . B_tile (MN-major view: one 64-element
+// MN block, so its leading offset is never applied); three passes
 __device__ __forceinline__ void mma_ts3(uint32_t d_t, uint32_t a_t, uint32_t b_hi, uint32_t b_lo, uint32_t idesc) {
   uint32_t acc = 0;
 #pragma unroll
@@ -166,51 +80,10 @@ __device__ __forceinline__ void mma_ts3(uint32_t d_t, uint32_t a_t, uint32_t b_h
     const uint32_t at = pass == 2 ? a_t + 64 : a_t, bt = pass == 1 ? b_lo : b_hi;
 #pragma unroll
     for (int ks = 0; ks < 8; ++ks) {
-      umma_f16_ts(d_t, at + (uint32_t)(ks * 8), make_sw128_desc_mn16(bt + ks * 2048), idesc, acc);
+      umma_f16_ts(d_t, at + (uint32_t)(ks * 8), make_sw128_desc_mn16(bt + ks * 2048, 1024), idesc, acc);
       acc = 1;
     }
   }
-}
-
-// keep decisions of query row i for the 16 keys [16 np, 16 np + 16): bit (8 n1 + 2 t + e) of the result.  Rows i and i ^ 8
-// (lanes l and l ^ 8) share their four Philox calls: the rh = 0 lane computes t = 0, 1, the rh = 1 lane t = 2, 3, and they
-// trade the two words the other row's fields live in.  Must be called by both lanes together.
-__device__ __forceinline__ uint32_t keep_bits_row(uint64_t seed, uint64_t site, uint64_t bh, int i, int np, uint32_t thr16) {
-  const int rh = (i >> 3) & 1, g = i & 7, tile = i >> 4;
-  uint32_t own[2][2], got[2][2];  // [tt][e]: words holding MY fields (low half n1 = 0, high half n1 = 1) of call t = 2 rh + tt (own)
-                                  // and of my partner's call t = 2 (1 - rh) + tt (got)
-#pragma unroll
-  for (int tt = 0; tt < 2; ++tt) {
-    const uint4 r = rbm_philox_drop(seed, site, rbm_attn_call(bh, tile, g, 2 * rh + tt, np));
-    own[tt][0] = rh ? r.z : r.x;
-    own[tt][1] = rh ? r.w : r.y;
-    got[tt][0] = __shfl_xor_sync(0xffffffffu, rh ? r.x : r.z, 8);  // my partner's words of my call <-> mine of theirs
-    got[tt][1] = __shfl_xor_sync(0xffffffffu, rh ? r.y : r.w, 8);
-  }
-  uint32_t bits = 0;
-#pragma unroll
-  for (int t = 0; t < 4; ++t)
-#pragma unroll
-    for (int e = 0; e < 2; ++e) {
-      const uint32_t w = ((t >> 1) == rh) ? own[t & 1][e] : got[t & 1][e];
-#pragma unroll
-      for (int n1 = 0; n1 < 2; ++n1)
-        if (((w >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << (8 * n1 + 2 * t + e);
-    }
-  return bits;
-}
-// keep decisions of key j for the 16 queries [16 T, 16 T + 16): bit (g + 8 rh) of the result
-__device__ __forceinline__ uint32_t keep_bits_col(uint64_t seed, uint64_t site, uint64_t bh, int j, int T, uint32_t thr16) {
-  const int t = (j & 7) >> 1, e = j & 1, n1 = (j >> 3) & 1, np = j >> 4;
-  uint32_t bits = 0;
-#pragma unroll
-  for (int g = 0; g < 8; ++g) {
-    const uint4 r = rbm_philox_drop(seed, site, rbm_attn_call(bh, T, g, t, np));
-    const uint32_t w0 = e ? r.y : r.x, w1 = e ? r.w : r.z;  // rh = 0 / rh = 1
-    if (((w0 >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << g;
-    if (((w1 >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << (g + 8);
-  }
-  return bits;
 }
 
 // Packed A operands (K = 128 tokens): hi words [0, 64), lo words [64, 128); word w = tokens (2 w, 2 w + 1); slot s owns words
@@ -253,7 +126,7 @@ __global__ void __launch_bounds__(THREADS, 2) attn_pair_fwd_kernel(const PairArg
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = tmem_base_slot, tS = tmem, tO = tmem + 128;
-  const uint32_t idS = make_idesc_f16(128, 128, 0), idO = make_idesc_f16(128, DK, 1);
+  const uint32_t idS = make_idesc_f16(128, 128, 0, 0), idO = make_idesc_f16(128, DK, 0, 1);
   const int q4 = warp & 3, hf = warp >> 2;
   const int r = q4 * 32 + lane, slot = r >> 6, i = r & 63;
   const uint32_t lane_sel = (uint32_t)(q4 * 32) << 16;
@@ -392,7 +265,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_pair_bwd_kernel(const PairArg
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = tmem_base_slot, tS = tmem, tP = tmem + 128, tDQ = tmem + 256, tDV = tmem + 320, tDK = tmem + 384;
-  const uint32_t idS = make_idesc_f16(128, 128, 0), idO = make_idesc_f16(128, DK, 1);
+  const uint32_t idS = make_idesc_f16(128, 128, 0, 0), idO = make_idesc_f16(128, DK, 0, 1);
   const int q4 = warp & 3, hf = warp >> 2;
   const int r = q4 * 32 + lane, slot = r >> 6, i = r & 63;
   const uint32_t lane_sel = (uint32_t)(q4 * 32) << 16;
@@ -481,7 +354,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_pair_bwd_kernel(const PairArg
       if (lane == 0 && mx > 0.f) atomicMax(&maxbits[4], __float_as_uint(mx));
     }
     __syncthreads();  // max |dS| is known; every score / dP~ column has been read and may be overwritten
-    const float sd = pow2_scale(__uint_as_float(maxbits[4]));
+    const float sd = pow2_scale(__uint_as_float(maxbits[4]), 14);
 #pragma unroll
     for (int pp = 0; pp < 2; ++pp) {
       float(&v)[16] = *reinterpret_cast<float(*)[16]>(&ds[pp * 16]);
@@ -609,11 +482,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_pair_bwd_kernel(const PairArg
   }
 }
 
-float pscale_for(float inv_keep) {
-  int e = 0;
-  frexpf(inv_keep, &e);           // inv_keep <= 2^e
-  return ldexpf(1.f, 14 - e);     // P~ * pscale <= 2^14
-}
+float pscale_for(float inv_keep) { return pow2_scale(inv_keep, 14); }  // P~ <= inv_keep, so P~ * pscale < 2^14
 
 }  // namespace
 

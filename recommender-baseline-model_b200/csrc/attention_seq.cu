@@ -19,16 +19,18 @@
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E, RBM_PADFILL
 #include "tc_ptx.cuh"
+#include "split16.cuh"
+#include "attention_f16.cuh"
 #include "attention_seq.cuh"
 #include "attention_tc.cuh"  // rbm_attn_tc_enabled
 
 namespace {
 
 using namespace rbm_tc;
+using namespace rbm_attn16;
 using rbm_mma::ex2;
 
 constexpr int DK = 64;
-constexpr int THREADS = 256;
 constexpr uint32_t T128 = 128 * 128;  // [128 rows x 64 fp16] = 16 KB
 
 struct SeqArgs {
@@ -41,56 +43,6 @@ struct SeqArgs {
   uint32_t thr16;
   uint64_t seed, site;
 };
-
-// ------------------------------------------------------------------------------------------------ PTX (kind::f16)
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N, int b_mn) {
-  return (1u << 4) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ uint64_t desc_mn16(uint32_t saddr) {  // MN-major view, one 64-element MN block (see ce_wide.cu)
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)(1024 >> 4) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]),
-               "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-               : "memory");
-}
-__device__ __forceinline__ void split_pack16(const float (&g)[16], uint32_t (&hi)[8], uint32_t (&lo)[8]) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const __half h0 = __float2half_rn(g[2 * j]), h1 = __float2half_rn(g[2 * j + 1]);
-    const __half l0 = __float2half_rn(g[2 * j] - __half2float(h0)), l1 = __float2half_rn(g[2 * j + 1] - __half2float(h1));
-    hi[j] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-    lo[j] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-  }
-}
-__device__ __forceinline__ float pow2_scale(float m) {  // power of two that brings a maximum magnitude m into [2^13, 2^14)
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  return ldexpf(1.f, 14 - e);
-}
 
 // ------------------------------------------------------------------------------------------------ tile staging
 // 128 tokens [t0, t0 + 128) of item (b, hh), 64 columns: thread task (row r, 16-byte output chunk c) = 8 consecutive columns.
@@ -112,28 +64,6 @@ __device__ __forceinline__ float tile_fetch(float (&v)[4][8], const float* __res
   }
   return mx;
 }
-__device__ __forceinline__ void tile_store(const float (&v)[4][8], float sc, uint8_t* hi, uint8_t* lo) {
-#pragma unroll
-  for (int it = 0; it < 4; ++it) {
-    const int task = it * THREADS + (int)threadIdx.x, r = task >> 3, c = task & 7;
-    uint32_t h[4], l[4];
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      const float x0 = v[it][2 * e] * sc, x1 = v[it][2 * e + 1] * sc;
-      const __half h0 = __float2half_rn(x0), h1 = __float2half_rn(x1);
-      const __half l0 = __float2half_rn(x0 - __half2float(h0)), l1 = __float2half_rn(x1 - __half2float(h1));
-      h[e] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-      l[e] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-    }
-    const uint32_t off = (uint32_t)r * 128u + (uint32_t)((c ^ (r & 7)) << 4);
-    *reinterpret_cast<uint4*>(hi + off) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo + off) = make_uint4(l[0], l[1], l[2], l[3]);
-  }
-}
-__device__ __forceinline__ void tile_max(float mx, unsigned* maxbits) {
-  mx = warp_max(mx);
-  if ((threadIdx.x & 31) == 0 && mx > 0.f) atomicMax(maxbits, __float_as_uint(mx));
-}
 // all rows of one tensor of the item (up to 256 tokens, two 128-row halves sharing ONE scale) -> hi / lo tiles of 256 rows.
 // Must be called by all THREADS threads; *maxbits must be zero on entry (and is consumed).  Returns the scale.
 __device__ __forceinline__ float stage_rows256(const float* __restrict__ src, int64_t ld, float mul, int b, int hh, int L, uint8_t* hi, uint8_t* lo,
@@ -142,7 +72,7 @@ __device__ __forceinline__ float stage_rows256(const float* __restrict__ src, in
   tile_max(tile_fetch(va, src, ld, mul, b, hh, 0, L), maxbits);
   tile_max(tile_fetch(vb, src, ld, mul, b, hh, 128, L), maxbits);
   __syncthreads();
-  const float sc = pow2_scale(__uint_as_float(*maxbits));
+  const float sc = pow2_scale(__uint_as_float(*maxbits), 14);
   tile_store(va, sc, hi, lo);
   tile_store(vb, sc, hi + T128, lo + T128);
   return sc;
@@ -152,26 +82,14 @@ __device__ __forceinline__ float stage_rows128(const float* __restrict__ src, in
   float va[4][8];
   tile_max(tile_fetch(va, src, ld, mul, b, hh, t0, L), maxbits);
   __syncthreads();
-  const float sc = pow2_scale(__uint_as_float(*maxbits));
+  const float sc = pow2_scale(__uint_as_float(*maxbits), 14);
   tile_store(va, sc, hi, lo);
   return sc;
 }
 
-// D[128 x N] = A_tile (K-major, 128 rows) . B_tile^T (K-major, N rows), contraction over d_k = 64; three passes
-__device__ __forceinline__ void mma_ss3(uint32_t d_t, uint32_t a_hi, uint32_t a_lo, uint32_t b_hi, uint32_t b_lo, uint32_t idesc) {
-  uint32_t acc = 0;
-#pragma unroll
-  for (int pass = 0; pass < 3; ++pass) {
-    const uint64_t ad = make_sw128_desc(pass == 2 ? a_lo : a_hi), bd = make_sw128_desc(pass == 1 ? b_lo : b_hi);
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      umma_f16(d_t, ad + (uint64_t)(k * 2), bd + (uint64_t)(k * 2), idesc, acc);
-      acc = 1;
-    }
-  }
-}
 // D[128 x 64] (+)= A (tensor memory, 128 tokens as two thread-halves: tokens [64 hf, 64 hf + 64) have their hi words at
-// a_t + 64 hf, lo words at a_t + 64 hf + 32) . B_tile rows [0, 128) (MN-major view); three passes
+// a_t + 64 hf, lo words at a_t + 64 hf + 32) . B_tile rows [0, 128) (MN-major view: one 64-element MN block, so its leading
+// offset is never applied); three passes
 __device__ __forceinline__ void mma_ts3_128(uint32_t d_t, uint32_t a_t, uint32_t b_hi, uint32_t b_lo, uint32_t idesc, uint32_t& acc) {
 #pragma unroll
   for (int pass = 0; pass < 3; ++pass) {
@@ -179,49 +97,10 @@ __device__ __forceinline__ void mma_ts3_128(uint32_t d_t, uint32_t a_t, uint32_t
 #pragma unroll
     for (int ks = 0; ks < 8; ++ks) {
       const uint32_t at = a_t + (uint32_t)((ks >> 2) * 64 + (pass == 2 ? 32 : 0) + (ks & 3) * 8);
-      umma_f16_ts(d_t, at, desc_mn16(bt + ks * 2048), idesc, acc);
+      umma_f16_ts(d_t, at, make_sw128_desc_mn16(bt + ks * 2048, 1024), idesc, acc);
       acc = 1;
     }
   }
-}
-
-// keep decisions of query row i for the 16 keys [16 np, 16 np + 16): bit (8 n1 + 2 t + e).  Lanes l and l ^ 8 (rows i, i ^ 8) share
-// their four Philox calls (see attention_pair.cu); both must call together.
-__device__ __forceinline__ uint32_t keep_bits_row(uint64_t seed, uint64_t site, uint64_t bh, int i, int np, uint32_t thr16) {
-  const int rh = (i >> 3) & 1, g = i & 7, tile = i >> 4;
-  uint32_t own[2][2], got[2][2];
-#pragma unroll
-  for (int tt = 0; tt < 2; ++tt) {
-    const uint4 r = rbm_philox_drop(seed, site, rbm_attn_call(bh, tile, g, 2 * rh + tt, np));
-    own[tt][0] = rh ? r.z : r.x;
-    own[tt][1] = rh ? r.w : r.y;
-    got[tt][0] = __shfl_xor_sync(0xffffffffu, rh ? r.x : r.z, 8);
-    got[tt][1] = __shfl_xor_sync(0xffffffffu, rh ? r.y : r.w, 8);
-  }
-  uint32_t bits = 0;
-#pragma unroll
-  for (int t = 0; t < 4; ++t)
-#pragma unroll
-    for (int e = 0; e < 2; ++e) {
-      const uint32_t w = ((t >> 1) == rh) ? own[t & 1][e] : got[t & 1][e];
-#pragma unroll
-      for (int n1 = 0; n1 < 2; ++n1)
-        if (((w >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << (8 * n1 + 2 * t + e);
-    }
-  return bits;
-}
-// keep decisions of key j for the 16 queries [16 T, 16 T + 16): bit (g + 8 rh)
-__device__ __forceinline__ uint32_t keep_bits_col(uint64_t seed, uint64_t site, uint64_t bh, int j, int T, uint32_t thr16) {
-  const int t = (j & 7) >> 1, e = j & 1, n1 = (j >> 3) & 1, np = j >> 4;
-  uint32_t bits = 0;
-#pragma unroll
-  for (int g = 0; g < 8; ++g) {
-    const uint4 r = rbm_philox_drop(seed, site, rbm_attn_call(bh, T, g, t, np));
-    const uint32_t w0 = e ? r.y : r.x, w1 = e ? r.w : r.z;
-    if (((w0 >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << g;
-    if (((w1 >> (16 * n1)) & 0xffffu) >= thr16) bits |= 1u << (g + 8);
-  }
-  return bits;
 }
 
 // shared prologue of the three kernels
@@ -270,7 +149,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_fwd_kernel(const SeqArgs 
   SEQ_PROLOGUE(512);
   __shared__ float xmax[2][128], xsum[2][128];
   const uint32_t tS = tmem, tO = tmem + 256;
-  const uint32_t idS = make_idesc_f16(128, nt == 2 ? 256 : 128, 0), idO = make_idesc_f16(128, DK, 1);
+  const uint32_t idS = make_idesc_f16(128, nt == 2 ? 256 : 128, 0, 0), idO = make_idesc_f16(128, DK, 0, 1);
   for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
     const int b = item / a.h, hh = item - b * a.h;
     if (threadIdx.x < 4) maxbits[threadIdx.x] = 0u;
@@ -356,7 +235,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_fwd_kernel(const SeqArgs 
           for (int kh = 0; kh < nt; ++kh)
 #pragma unroll
             for (int ks = 0; ks < 8; ++ks) {
-              umma_f16_ts(tO, tS + (uint32_t)(kh * 128 + (pass == 2 ? 64 : 0) + ks * 8), desc_mn16(vt + (kh * 128 + ks * 16) * 128), idO, acc);
+              umma_f16_ts(tO, tS + (uint32_t)(kh * 128 + (pass == 2 ? 64 : 0) + ks * 8), make_sw128_desc_mn16(vt + (kh * 128 + ks * 16) * 128, 1024),
+                          idO, acc);
               acc = 1;
             }
         }
@@ -404,7 +284,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_dq_kernel(const SeqArgs a
   SEQ_PROLOGUE(512);
   __shared__ float row_m[128], row_inv[128], row_delta[128];
   const uint32_t tS = tmem, tP = tmem + 128, tDQ = tmem + 256;
-  const uint32_t idS = make_idesc_f16(128, 128, 0), idO = make_idesc_f16(128, DK, 1);
+  const uint32_t idS = make_idesc_f16(128, 128, 0, 0), idO = make_idesc_f16(128, DK, 0, 1);
   for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
     const int b = item / a.h, hh = item - b * a.h;
     if (threadIdx.x < 4) maxbits[threadIdx.x] = 0u;
@@ -440,8 +320,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_dq_kernel(const SeqArgs a
         tile_max(tile_fetch(va, a.q, a.ldq, a.scale * RBM_LOG2E, b, hh, qt * 128, L), &maxbits[2]);
         tile_max(tile_fetch(vb, a.dout, a.lddo, 1.f, b, hh, qt * 128, L), &maxbits[3]);
         __syncthreads();
-        sQ = pow2_scale(__uint_as_float(maxbits[2]));
-        sG = pow2_scale(__uint_as_float(maxbits[3]));
+        sQ = pow2_scale(__uint_as_float(maxbits[2]), 14);
+        sG = pow2_scale(__uint_as_float(maxbits[3]), 14);
         tile_store(va, sQ, sm + OFF_Q, sm + OFF_Q + T128);
         tile_store(vb, sG, sm + OFF_G, sm + OFF_G + T128);
       }
@@ -531,7 +411,7 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_dkv_kernel(const SeqArgs 
   SEQ_PROLOGUE(512);
   __shared__ float row_m[256], row_inv[256], row_delta[256];
   const uint32_t tS = tmem, tP = tmem + 128, tDV = tmem + 256, tDK = tmem + 320;
-  const uint32_t idS = make_idesc_f16(128, 128, 0), idO = make_idesc_f16(128, DK, 1);
+  const uint32_t idS = make_idesc_f16(128, 128, 0, 0), idO = make_idesc_f16(128, DK, 0, 1);
   for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
     const int b = item / a.h, hh = item - b * a.h;
     if (threadIdx.x < 4) maxbits[threadIdx.x] = 0u;
@@ -566,8 +446,8 @@ __global__ void __launch_bounds__(THREADS, 1) attn_seq_dkv_kernel(const SeqArgs 
         tile_max(tile_fetch(va, a.k, a.ldk, 1.f, b, hh, kt * 128, L), &maxbits[2]);
         tile_max(tile_fetch(vb, a.v, a.ldv, 1.f, b, hh, kt * 128, L), &maxbits[3]);
         __syncthreads();
-        sK = pow2_scale(__uint_as_float(maxbits[2]));
-        sV = pow2_scale(__uint_as_float(maxbits[3]));
+        sK = pow2_scale(__uint_as_float(maxbits[2]), 14);
+        sV = pow2_scale(__uint_as_float(maxbits[3]), 14);
         tile_store(va, sK, sm + OFB_K, sm + OFB_K + T128);
         tile_store(vb, sV, sm + OFB_V, sm + OFB_V + T128);
       }
@@ -669,7 +549,7 @@ void fill_common(SeqArgs& a, int B, int L, int h, int mask_mode, float scale, fl
   int e = 0;
   frexpf(a.inv_keep, &e);  // inv_keep <= 2^e
   a.keep_pow2 = ldexpf(1.f, e);
-  a.pscale = ldexpf(1.f, 14 - e);
+  a.pscale = pow2_scale(a.inv_keep, 14);
   a.seed = seed; a.site = site;
 }
 

@@ -30,6 +30,7 @@
 #include "common.cuh"
 #include "mma_tiles.cuh"  // ex2, RBM_LOG2E, RBM_LN2
 #include "tc_ptx.cuh"
+#include "split16.cuh"
 #include "ce_wide.cuh"
 
 namespace {
@@ -75,56 +76,6 @@ __host__ __device__ inline int pick_vs(int RT) {
     }
   }
   return best;
-}
-
-// ------------------------------------------------------------------------------------------------ PTX (kind::f16)
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// cute::UMMA::InstrDescriptor, kind::f16: D = F32 (bits [4,6) = 1), A = B = F16 (format 0), B major in bit 16
-__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N, int b_mn) {
-  return (1u << 4) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// MN-major, 128-byte-swizzled operand of 16-bit elements (cute Layout_MN_SW128_Atom: ((8,8,m),(8,k)):((1,8,LBO),(64,SBO)) in
-// elements): rows of the tile are K, 128 bytes = 64 MN elements per row; SBO = 1024 B between 8-row K groups, further
-// 64-element MN blocks lie `lbo_bytes` apart.  Physically the same bytes TMA writes for the K-major view of the tile.
-__device__ __forceinline__ uint64_t make_sw128_desc_mn16(uint32_t saddr, uint32_t lbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]),
-               "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-               : "memory");
-}
-// x -> (hi, lo) fp16 pair; 16 values -> 8 packed words each (element 2j in the low half of word j: the order a 16-bit A
-// operand in tensor memory is read in)
-__device__ __forceinline__ void split_pack16(const float (&g)[16], uint32_t (&hi)[8], uint32_t (&lo)[8]) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const __half h0 = __float2half_rn(g[2 * j]), h1 = __float2half_rn(g[2 * j + 1]);
-    const __half l0 = __float2half_rn(g[2 * j] - __half2float(h0)), l1 = __float2half_rn(g[2 * j + 1] - __half2float(h1));
-    hi[j] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-    lo[j] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-  }
 }
 
 // --------------------------------------------------------------------------------------------- the backward kernel
@@ -217,7 +168,7 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
   } else if (warp == 1) {
     // ------------------------------------------------------------------------------------------- MMA issuer
     if (elect_one()) {
-      const uint32_t idS = make_idesc_f16(128, NV, 0), idU = make_idesc_f16(128, d, 1);
+      const uint32_t idS = make_idesc_f16(128, NV, 0, 0), idU = make_idesc_f16(128, d, 0, 1);
       mbar_wait(smem_u32(&rt_bar), 0);
       if (!lo_tmem) mbar_wait(smem_u32(&r_bar), 0);
       tc_fence_after();
@@ -524,7 +475,7 @@ ce_wide_fwd128_kernel(const __grid_constant__ CUtensorMap mapSh, const __grid_co
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idS = make_idesc_f16(128, NV, 0);
+      const uint32_t idS = make_idesc_f16(128, NV, 0, 0);
       mbar_wait(smem_u32(&rt_bar), 0);
       tc_fence_after();
       int q = 0;
@@ -656,48 +607,6 @@ ce_wide_fwd128_kernel(const __grid_constant__ CUtensorMap mapSh, const __grid_co
 }
 
 // ---------------------------------------------------------------------------------------------- helper kernels
-// max |x| as the bit pattern of a non-negative float (atomicMax on unsigned: order-independent)
-__global__ void __launch_bounds__(256) maxabs_kernel(const float* __restrict__ x, int64_t n4, unsigned* __restrict__ out_bits) {
-  float m = 0.f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
-    const float4 v = ld4(x + i * 4);
-    m = fmaxf(fmaxf(m, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
-  }
-  m = warp_max(m);
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
-}
-// power-of-two scales that bring max |x| into [2^14, 2^15)  (scales[i] for bits[i]); inf / nan inputs poison the result
-__global__ void scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ scales) {
-  const int i = threadIdx.x;
-  if (i >= 2) return;
-  const float m = __uint_as_float(bits[i]);
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);  // m = f * 2^e, f in [0.5, 1)
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  scales[i] = ldexpf(1.f, 15 - e);
-}
-__device__ __forceinline__ void split4(float4 v, float s, uint2& hi, uint2& lo) {
-  const float x[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
-  unsigned short h[4], l[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const __half hh = __float2half_rn(x[j]);
-    h[j] = __half_as_ushort(hh);
-    l[j] = __half_as_ushort(__float2half_rn(x[j] - __half2float(hh)));
-  }
-  hi = make_uint2((uint32_t)h[0] | ((uint32_t)h[1] << 16), (uint32_t)h[2] | ((uint32_t)h[3] << 16));
-  lo = make_uint2((uint32_t)l[0] | ((uint32_t)l[1] << 16), (uint32_t)l[2] | ((uint32_t)l[3] << 16));
-}
-// hi/lo fp16 copies of w * scales[1]
-__global__ void __launch_bounds__(256) split_w_kernel(const float* __restrict__ w, const float* __restrict__ scales, uint2* __restrict__ hi,
-                                                      uint2* __restrict__ lo, int64_t n4) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n4) return;
-  uint2 a, b;
-  split4(ld4(w + i * 4), scales[1], a, b);
-  hi[i] = a;
-  lo[i] = b;
-}
 // Hc[r] = h[rows[r]] * scales[0] (r < count) as hi/lo fp16; zeros up to the next multiple of 128 PLUS one more tile: the DW
 // kernel streams these rows in NV-row chunks, and the last chunk may reach past the 128-row boundary into what would
 // otherwise be stale workspace (0 x NaN = NaN inside the tensor core)
@@ -768,17 +677,6 @@ __global__ void __launch_bounds__(256) dh_reduce_kernel(const float* __restrict_
   st4(dh_full + ((int64_t)rows[r] * d4 + c4) * 4, make_float4(s.x * mul, s.y * mul, s.z * mul, s.w * mul));
 }
 
-// [rows, d] fp16, box [box_rows x 64 columns], 128-byte swizzle; rows beyond the tensor read as zeros
-bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int d, int box_rows) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)d, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)d * sizeof(__half)};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 // fp16 passes per product: 3 (hi.hi + hi.lo + lo.hi), or 1 (hi.hi) under RBM_CE_WIDE_PASSES=1, the reduced-precision line.
 // Read on every call, never cached: bench.py's labelled reduced-precision line and test_score_ce_wide_million_items set and
 // unset the variable inside one process, and a cached value would time or test the three-pass kernels under the wrong label.
@@ -839,10 +737,10 @@ int prepare(const float* h, const int32_t* rows, const int32_t* count, const flo
   const int64_t cap128 = (cap + 127) / 128 * 128;
   cudaMemsetAsync(ws.bits, 0, 16, st);
   const int64_t nh4 = cap * d / 4, nw4 = (int64_t)V1 * d / 4;
-  maxabs_kernel<<<(unsigned)(rbm_cdiv(nh4, 256) < 4 * RBM_NUM_SMS ? rbm_cdiv(nh4, 256) : 4 * RBM_NUM_SMS), 256, 0, st>>>(h, nh4, ws.bits);
-  maxabs_kernel<<<(unsigned)(rbm_cdiv(nw4, 256) < 4 * RBM_NUM_SMS ? rbm_cdiv(nw4, 256) : 4 * RBM_NUM_SMS), 256, 0, st>>>(w, nw4, ws.bits + 1);
-  scales_kernel<<<1, 32, 0, st>>>(ws.bits, ws.scales);
-  split_w_kernel<<<(unsigned)rbm_cdiv(nw4, 256), 256, 0, st>>>(w, ws.scales, (uint2*)ws.w_hi, (uint2*)ws.w_lo, nw4);
+  maxabs_launch(h, d, cap, d, ws.bits, (int)(rbm_cdiv(nh4, 256) < 4 * RBM_NUM_SMS ? rbm_cdiv(nh4, 256) : 4 * RBM_NUM_SMS), st);
+  maxabs_launch(w, d, V1, d, ws.bits + 1, (int)(rbm_cdiv(nw4, 256) < 4 * RBM_NUM_SMS ? rbm_cdiv(nw4, 256) : 4 * RBM_NUM_SMS), st);
+  scales_launch(ws.bits, ws.scales, st);
+  split_w_launch(w, ws.scales + 1, (uint2*)ws.w_hi, (uint2*)ws.w_lo, nw4, st);
   gather_split_h_kernel<<<(unsigned)rbm_cdiv(cap128 * (d / 4), 256), 256, 0, st>>>(h, rows, count, ws.scales, (uint2*)ws.h_hi, (uint2*)ws.h_lo,
                                                                                   cap128, d / 4);
   RBM_LAUNCH_CHECK("rbm_ce(wide prepare)");
@@ -880,7 +778,7 @@ int rbm_ce_wide_fwd(const float* h, const int32_t* rows, const int64_t* tgt, con
   if (int rc = prepare(h, rows, count, w, cap, V1, d, ws, st)) return rc;
   // 128-row vocabulary tiles through a ring of K-block pieces (N = 128 instructions)
   CUtensorMap mSh, mSl;
-  if (!encode_map(&mSh, ws.w_hi, V1, d, 128) || !encode_map(&mSl, ws.w_lo, V1, d, 128)) {
+  if (!encode_f16_rows(&mSh, ws.w_hi, V1, d, 128) || !encode_f16_rows(&mSl, ws.w_lo, V1, d, 128)) {
     rbm_set_error("rbm_ce_fwd(wide): cuTensorMapEncodeTiled failed");
     return -1;
   }
@@ -908,8 +806,9 @@ int rbm_ce_wide_bwd(const float* h, const int32_t* rows, const int64_t* tgt, con
   if (int rc = prepare(h, rows, count, w, cap, V1, d, ws, st)) return rc;
   const Shape sh = pick_shape(d);
   CUtensorMap mHlr, mWs, mWls, mWlr, mHs, mHls;
-  if (!encode_map(&mHlr, ws.h_lo, cap128, d, 128) || !encode_map(&mWs, ws.w_hi, V1, d, sh.NV) || !encode_map(&mWls, ws.w_lo, V1, d, sh.NV) ||
-      !encode_map(&mWlr, ws.w_lo, V1, d, 128) || !encode_map(&mHs, ws.h_hi, cap128, d, sh.NV) || !encode_map(&mHls, ws.h_lo, cap128, d, sh.NV)) {
+  if (!encode_f16_rows(&mHlr, ws.h_lo, cap128, d, 128) || !encode_f16_rows(&mWs, ws.w_hi, V1, d, sh.NV) ||
+      !encode_f16_rows(&mWls, ws.w_lo, V1, d, sh.NV) || !encode_f16_rows(&mWlr, ws.w_lo, V1, d, 128) ||
+      !encode_f16_rows(&mHs, ws.h_hi, cap128, d, sh.NV) || !encode_f16_rows(&mHls, ws.h_lo, cap128, d, sh.NV)) {
     rbm_set_error("rbm_ce_bwd(wide): cuTensorMapEncodeTiled failed");
     return -1;
   }

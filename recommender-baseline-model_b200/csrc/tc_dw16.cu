@@ -1,5 +1,5 @@
 // tc_dw16.cu -- weight gradient of the wide Linear layers (d >= 256):  dW[N, K] = dpre[M, N]^T . x[M, K], contraction over the
-// M tokens, on the Blackwell tensor path in SPLIT fp16 (see ce_wide.cu for the arithmetic).  Replaces, for N > 256 or K > 256
+// M tokens, on the Blackwell tensor path in SPLIT fp16 (split16.cuh).  Replaces, for N > 256 or K > 256
 // (shapes the TF32 kernel tc_dw_kernel cannot hold in tensor memory; they ran the fp32 SIMT kernel at 24 TFLOP/s), the
 // autograd of nn.Linear's weight (NN/models/bert_modules/utils/feed_forward.py:10-11, attention/multi_head.py:18-19).
 //   * both operands are token-major in HBM, i.e. MN-major for the tensor core: eight converter warps read fp32 rows
@@ -10,9 +10,9 @@
 //     B[16 tokens x KT], three passes (hi.hi + hi.lo + lo.hi), KT = 256 (N = 256 instructions run at the tensor floor);
 //   * a CTA owns one [128 x KT] tile of dW and one slab of tokens; partial tiles are summed in fixed order by the caller
 //     (linear.cu, launch_reduce_splits): bit-deterministic, no atomics.
-#include <cuda_fp16.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
+#include "split16.cuh"
 #include "tc_dw16.cuh"
 
 namespace {
@@ -32,36 +32,12 @@ struct Dw16Args {
   int N, K, KT, tiles_k;
 };
 
-__device__ __forceinline__ void umma_f16_mn(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// MN-major 16-bit operand, 128-byte swizzle: rows = K (tokens), 64 MN elements per row; SBO = 1024 B between 8-token groups,
-// further 64-element MN blocks lie lbo bytes apart
-__device__ __forceinline__ uint64_t desc_mn16(uint32_t saddr, uint32_t lbo_bytes) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
-  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
 // 8 consecutive fp32 values (two float4) x scale -> 8 fp16 hi + 8 fp16 lo (16 bytes each)
 __device__ __forceinline__ void split8(const float4& a, const float4& b, float s, uint4& hi, uint4& lo) {
   const float v[8] = {a.x * s, a.y * s, a.z * s, a.w * s, b.x * s, b.y * s, b.z * s, b.w * s};
   uint32_t h[4], l[4];
 #pragma unroll
-  for (int e = 0; e < 4; ++e) {
-    const __half h0 = __float2half_rn(v[2 * e]), h1 = __float2half_rn(v[2 * e + 1]);
-    const __half l0 = __float2half_rn(v[2 * e] - __half2float(h0)), l1 = __float2half_rn(v[2 * e + 1] - __half2float(h1));
-    h[e] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-    l[e] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
-  }
+  for (int e = 0; e < 4; ++e) split2(v[2 * e], v[2 * e + 1], h[e], l[e]);
   hi = make_uint4(h[0], h[1], h[2], h[3]);
   lo = make_uint4(l[0], l[1], l[2], l[3]);
 }
@@ -98,7 +74,7 @@ __global__ void __launch_bounds__(32 * (NCONV + 1), 1) dw16_kernel(const Dw16Arg
   if (warp == NCONV) {
     // ------------------------------------------------------------------------------------------ MMA issuer
     if (elect_one()) {
-      const uint32_t idesc = (1u << 4) | (1u << 15) | (1u << 16) | ((uint32_t)(KT >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      const uint32_t idesc = make_idesc_f16(128, KT, 1, 1);
       uint32_t acc = 0;
       for (int j = 0; j < nblk; ++j) {
         const int s = j & 1;
@@ -110,7 +86,7 @@ __global__ void __launch_bounds__(32 * (NCONV + 1), 1) dw16_kernel(const Dw16Arg
           const uint32_t pa = pass == 2 ? sAl : sAh, pb = pass == 1 ? sBl : sBh;
 #pragma unroll
           for (int ks = 0; ks < TOKB / 16; ++ks) {
-            umma_f16_mn(tD, desc_mn16(pa + ks * 2048, BLK), desc_mn16(pb + ks * 2048, BLK), idesc, acc);
+            umma_f16(tD, make_sw128_desc_mn16(pa + ks * 2048, BLK), make_sw128_desc_mn16(pb + ks * 2048, BLK), idesc, acc);
             acc = 1;
           }
         }
@@ -235,26 +211,6 @@ __global__ void __launch_bounds__(32 * (NCONV + 1), 1) dw16_kernel(const Dw16Arg
   }
 }
 
-// max |x| over a strided [rows, cols] matrix -> bit pattern (atomicMax on unsigned: order-independent)
-__global__ void __launch_bounds__(256) maxabs2d_kernel(const float* __restrict__ src, int64_t ld, int64_t rows, int c4, unsigned* __restrict__ out_bits) {
-  float m = 0.f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < rows * c4; i += (int64_t)gridDim.x * blockDim.x) {
-    const float4 v = ld4(src + (i / c4) * ld + (i % c4) * 4);
-    m = fmaxf(fmaxf(m, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
-  }
-  m = warp_max(m);
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
-}
-__global__ void dw16_scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ scales) {
-  const int i = threadIdx.x;
-  if (i >= 2) return;
-  const float m = __uint_as_float(bits[i]);
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  scales[i] = ldexpf(1.f, 15 - e);
-}
-
 int tile_k(int K) { return K % 256 == 0 ? 256 : 128; }
 
 }  // namespace
@@ -283,9 +239,9 @@ int rbm_dw16_launch(const float* dpre, int64_t lda, const float* x, int64_t ldb,
   unsigned* bits = (unsigned*)aux;
   float* scales = (float*)((uint8_t*)aux + 16);
   cudaMemsetAsync(aux, 0, 16, st);
-  maxabs2d_kernel<<<2 * RBM_NUM_SMS, 256, 0, st>>>(dpre, lda, M, N / 4, bits);
-  maxabs2d_kernel<<<2 * RBM_NUM_SMS, 256, 0, st>>>(x, ldb, M, K / 4, bits + 1);
-  dw16_scales_kernel<<<1, 32, 0, st>>>(bits, scales);
+  maxabs_launch(dpre, lda, M, N, bits, 2 * RBM_NUM_SMS, st);
+  maxabs_launch(x, ldb, M, K, bits + 1, 2 * RBM_NUM_SMS, st);
+  scales_launch(bits, scales, st);
   Dw16Args a{};
   a.dpre = dpre; a.x = x; a.scales = scales; a.part = part; a.part_b = part_b; a.lda = lda; a.ldb = ldb; a.M = M; a.N = N; a.K = K;
   a.KT = tile_k(K);

@@ -16,6 +16,7 @@
 #include <cuda_fp16.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
+#include "split16.cuh"
 #include "tc_gemm.cuh"
 #include "tc_gemm16.cuh"
 
@@ -48,15 +49,6 @@ struct G16Params {
   float invA, invB;
   uint64_t siteA, siteB, seed;
 };
-
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 
 // shared memory: operand ring NSTG x 64 KB | fp32 A staging NSTG x 32 KB | epilogue transposition buffers 32 KB
 __global__ void __launch_bounds__(THREADS, 1) gemm16_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapBh,
@@ -113,7 +105,7 @@ __global__ void __launch_bounds__(THREADS, 1) gemm16_kernel(const __grid_constan
   } else if (warp == 1) {
     // ------------------------------------------------------------------------------------------- MMA issuer
     if (elect_one()) {
-      const uint32_t idesc = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+      const uint32_t idesc = make_idesc_f16(128, 128, 0, 0);
       int g = 0, it = 0;
       for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++it) {
         const int buf = it & 1;
@@ -257,62 +249,6 @@ __global__ void __launch_bounds__(THREADS, 1) gemm16_kernel(const __grid_constan
   }
 }
 
-// ------------------------------------------------------------------------------------------------- pre-pass kernels
-// four independent 16-byte loads per thread and iteration: a one-load grid-stride loop is latency bound (measured 1.2 TB/s)
-__global__ void __launch_bounds__(256) g16_maxabs_kernel(const float* __restrict__ src, int64_t ld, int64_t rows, int c4, unsigned* __restrict__ out_bits) {
-  float m = 0.f;
-  const int64_t n = rows * c4, stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i0 < n; i0 += 4 * stride) {
-    float4 v[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int64_t i = i0 + j * stride;
-      v[j] = i < n ? ld4(src + (i / c4) * ld + (i % c4) * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) m = fmaxf(fmaxf(m, fmaxf(fabsf(v[j].x), fabsf(v[j].y))), fmaxf(fabsf(v[j].z), fabsf(v[j].w)));
-  }
-  m = warp_max(m);
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
-}
-__global__ void g16_scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ scales) {
-  const int i = threadIdx.x;
-  if (i >= 2) return;
-  const float m = __uint_as_float(bits[i]);
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  scales[i] = ldexpf(1.f, 15 - e);
-}
-// hi / lo fp16 copies of w * scales[1]
-__global__ void __launch_bounds__(256) g16_split_kernel(const float* __restrict__ w, const float* __restrict__ scales, uint2* __restrict__ hi,
-                                                        uint2* __restrict__ lo, int64_t n4) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n4) return;
-  const float4 v = ld4(w + i * 4);
-  const float s = scales[1];
-  const float x[4] = {v.x * s, v.y * s, v.z * s, v.w * s};
-  unsigned short h[4], l[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const __half hh = __float2half_rn(x[j]);
-    h[j] = __half_as_ushort(hh);
-    l[j] = __half_as_ushort(__float2half_rn(x[j] - __half2float(hh)));
-  }
-  hi[i] = make_uint2((uint32_t)h[0] | ((uint32_t)h[1] << 16), (uint32_t)h[2] | ((uint32_t)h[3] << 16));
-  lo[i] = make_uint2((uint32_t)l[0] | ((uint32_t)l[1] << 16), (uint32_t)l[2] | ((uint32_t)l[3] << 16));
-}
-
-bool encode_half(CUtensorMap* map, const void* base, int64_t rows, int cols) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)cols * 2};
-  cuuint32_t box[2] = {64, 128};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 bool encode_a32(CUtensorMap* map, const void* base, int64_t rows, int cols, int64_t ld) {
   EncodeTiledFn enc = get_encode();
   if (!enc) return false;
@@ -342,13 +278,12 @@ int rbm_gemm16_launch(const float* a, int64_t lda, const float* b, int64_t M, in
   unsigned* bits = (unsigned*)(w8 + (size_t)N * K * 4);
   float* scales = (float*)(w8 + (size_t)N * K * 4 + 16);
   cudaMemsetAsync(bits, 0, 16, st);
-  g16_maxabs_kernel<<<8 * RBM_NUM_SMS, 256, 0, st>>>(a, lda, M, K / 4, bits);
-  g16_maxabs_kernel<<<RBM_NUM_SMS, 256, 0, st>>>(b, K, N, K / 4, bits + 1);
-  g16_scales_kernel<<<1, 32, 0, st>>>(bits, scales);
-  const int64_t n4 = (int64_t)N * K / 4;
-  g16_split_kernel<<<(unsigned)rbm_cdiv(n4, 256), 256, 0, st>>>(b, scales, (uint2*)b_hi, (uint2*)b_lo, n4);
+  maxabs_launch(a, lda, M, K, bits, 8 * RBM_NUM_SMS, st);
+  maxabs_launch(b, K, N, K, bits + 1, RBM_NUM_SMS, st);
+  scales_launch(bits, scales, st);
+  split_w_launch(b, scales + 1, (uint2*)b_hi, (uint2*)b_lo, (int64_t)N * K / 4, st);
   CUtensorMap mA, mBh, mBl;
-  if (!encode_half(&mBh, b_hi, N, K) || !encode_half(&mBl, b_lo, N, K) || !encode_a32(&mA, a, M, K, lda)) {
+  if (!encode_f16_rows(&mBh, b_hi, N, K, 128) || !encode_f16_rows(&mBl, b_lo, N, K, 128) || !encode_a32(&mA, a, M, K, lda)) {
     rbm_set_error("rbm_linear(gemm16): cuTensorMapEncodeTiled failed");
     return -1;
   }

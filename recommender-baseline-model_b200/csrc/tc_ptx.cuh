@@ -1,6 +1,6 @@
 // tc_ptx.cuh -- inline-PTX wrappers for the Blackwell (sm_100a) async/tensor path: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (alloc/mma/commit/ld/st/fences) and UMMA shared-memory / instruction descriptors; plus the host-side lookup of the
-// tensor-map encoder.
+// tcgen05 (alloc/mma/commit/ld/st/fences, kind::tf32 and kind::f16) and UMMA shared-memory / instruction descriptors; plus the
+// host-side lookup of the tensor-map encoder and the fp16 row-tile tensor map.
 #pragma once
 #include <cuda.h>  // CUtensorMap types only; the encode function is fetched at run time (no libcuda link dependency)
 #include "common.cuh"
@@ -214,5 +214,51 @@ __host__ __device__ constexpr uint32_t make_idesc_tf32_ex(int M, int N, int a_mn
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) |
          ((uint32_t)(M >> 4) << 24);
 }
+
+// ------------------------------------------------------------------------------------------------ kind::f16
+// D[tmem] (+)= A[smem desc] . B[smem desc], fp16 operands, fp32 accumulate
+__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// D[tmem] (+)= A[tmem] . B[smem desc]   (16-bit A operand in tensor memory: two K elements per 32-bit column, element 2j in the
+// low half)
+__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
+      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// cute::UMMA::InstrDescriptor, kind::f16: D = F32 (bits [4,6) = 1), A = B = F16 (format 0), bit 15: A MN-major, bit 16: B MN-major
+__host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N, int a_mn, int b_mn) {
+  return (1u << 4) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// MN-major, 128-byte-swizzled operand of 16-bit elements (cute Layout_MN_SW128_Atom: ((8,8,m),(8,k)):((1,8,LBO),(64,SBO)) in
+// elements): rows of the tile are K, 128 bytes = 64 MN elements per row; SBO = 1024 B between 8-row K groups, further
+// 64-element MN blocks lie `lbo_bytes` apart.  Physically the same bytes TMA writes for the K-major view of the tile.
+__device__ __forceinline__ uint64_t make_sw128_desc_mn16(uint32_t saddr, uint32_t lbo_bytes) {
+  uint64_t d = 0;
+  d |= (uint64_t)((saddr >> 4) & 0x3FFF);
+  d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
+  d |= (uint64_t)(1024 >> 4) << 32;
+  d |= (uint64_t)1 << 46;
+  d |= (uint64_t)2 << 61;
+  return d;
+}
+__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]),
+               "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
+               : "memory");
+}
+
+// ------------------------------------------------------------------------------------------------ host side
+// [rows, cols] fp16 row-major, box [box_rows x 64 columns], 128-byte swizzle; rows beyond the tensor read as zeros (tc_encode.cu)
+bool encode_f16_rows(CUtensorMap* map, const void* base, int64_t rows, int cols, int box_rows);
 
 }  // namespace rbm_tc

@@ -28,6 +28,7 @@
 #include <stdlib.h>
 #include "common.cuh"
 #include "tc_ptx.cuh"
+#include "split16.cuh"
 #include "tc_topk.cuh"
 
 namespace {
@@ -49,14 +50,6 @@ struct TopkParams {
   uint32_t tmem_cols;
 };
 
-__device__ __forceinline__ void umma_f16_ss(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // F16: operands are the range-scaled fp16 copies (64 elements per 128-byte row, K = 16 per instruction, kind::f16);
 // otherwise the fp32 data itself (32 elements per row, K = 8, kind::tf32)
 template <bool F16>
@@ -121,7 +114,7 @@ __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idesc = F16 ? ((1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24)) : make_idesc_tf32(BM, BN);
+      const uint32_t idesc = F16 ? make_idesc_f16(BM, BN, 0, 0) : make_idesc_tf32(BM, BN);
       int g = 0, it = 0, un = 0;
       for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++un) {
         const int sp = u % p.S;
@@ -143,7 +136,7 @@ __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_
               const uint64_t bdesc = make_sw128_desc(smem_base + a_bytes + s * stage_bytes + kb * kb_bytes);
 #pragma unroll
               for (int k = 0; k < 4; ++k) {  // four 32-byte K steps per 128-byte row
-                if (F16) umma_f16_ss(d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0);
+                if (F16) umma_f16(d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0);
                 else umma_tf32(d, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0);
               }
             }
@@ -369,16 +362,6 @@ __global__ void __launch_bounds__(256) row_norm_max_kernel(const float* __restri
     if (lane == 0) atomicMax(out_bits + 1, __float_as_uint(amax));
   }
 }
-// scales[0] / [1]: powers of two that bring max |item row element| / max |user row element| (bits[1] / bits[2]) into [2^14, 2^15)
-__global__ void topk_scales_kernel(const unsigned* __restrict__ bits, float* __restrict__ scales) {
-  const int i = threadIdx.x;
-  if (i >= 2) return;
-  const float m = __uint_as_float(bits[1 + i]);
-  int e = 0;
-  if (m > 0.f && m < INFINITY) frexpf(m, &e);
-  e = e < -100 ? -100 : (e > 100 ? 100 : e);
-  scales[i] = ldexpf(1.f, 15 - e);
-}
 // fp16 copy of rows [r_begin, r_end) of src (row stride ld) times *scale -> dst rows [r_begin, r_end) (dense, d columns)
 __global__ void __launch_bounds__(256) to_half_kernel(const float* __restrict__ src, int64_t ld, int64_t r_begin, int64_t r_end, int d4,
                                                       const float* __restrict__ scale, uint2* __restrict__ dst) {
@@ -390,15 +373,6 @@ __global__ void __launch_bounds__(256) to_half_kernel(const float* __restrict__ 
   const float s = *scale;
   const __half2 a = __floats2half2_rn(v.x * s, v.y * s), b = __floats2half2_rn(v.z * s, v.w * s);
   dst[r * d4 + c4] = make_uint2(*reinterpret_cast<const uint32_t*>(&a), *reinterpret_cast<const uint32_t*>(&b));
-}
-__global__ void __launch_bounds__(256) maxabs_rows_kernel(const float* __restrict__ src, int64_t ld, int64_t rows, int d4, unsigned* __restrict__ out_bits) {
-  float m = 0.f;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < rows * d4; i += (int64_t)gridDim.x * blockDim.x) {
-    const float4 v = ld4(src + (i / d4) * ld + (i % d4) * 4);
-    m = fmaxf(fmaxf(m, fmaxf(fabsf(v.x), fabsf(v.y))), fmaxf(fabsf(v.z), fabsf(v.w)));
-  }
-  m = warp_max(m);
-  if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(out_bits, __float_as_uint(m));
 }
 
 bool encode_map(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool f16) {
@@ -495,8 +469,8 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
   row_norm_max_kernel<<<RBM_NUM_SMS * 4, 256, 0, st>>>(table, v_begin, v_end, d, lpr, bits, f16 ? 1 : 0);
   RBM_LAUNCH_CHECK("rbm_score_topk(row norms)");
   if (f16) {
-    maxabs_rows_kernel<<<RBM_NUM_SMS, 256, 0, st>>>(f, ldf, U, d / 4, bits + 2);
-    topk_scales_kernel<<<1, 32, 0, st>>>(bits, scales);
+    maxabs_launch(f, ldf, U, d, bits + 2, RBM_NUM_SMS, st);
+    scales_launch(bits + 1, scales, st);  // scales[0] / [1]: item rows (bits[1]) / user rows (bits[2])
     to_half_kernel<<<(unsigned)rbm_cdiv(n_items * (d / 4), 256), 256, 0, st>>>(table + v_begin * d, d, 0, n_items, d / 4, scales, (uint2*)th);
     to_half_kernel<<<(unsigned)rbm_cdiv(U * (d / 4), 256), 256, 0, st>>>(f, ldf, 0, U, d / 4, scales + 1, (uint2*)uh);
     RBM_LAUNCH_CHECK("rbm_score_topk(fp16 copies)");
