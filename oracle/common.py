@@ -5,7 +5,7 @@
 from __future__ import annotations
 
 import math
-from typing import Dict, Optional
+from typing import Dict, NamedTuple, Optional
 
 import numpy as np
 import torch
@@ -148,6 +148,57 @@ def embedding_grad_scatter_chunked(idx: np.ndarray, rows: np.ndarray, vocab: int
             total = acc if total is None else total + acc
         grad[key] += total
     return grad
+
+
+class MaskedCE64(NamedTuple):
+    lse: torch.Tensor   # [count] float64: log-sum-exp of the labelled rows over this block of columns, in row order
+    loss: float         # mean over the labelled rows of (lse - target logit); NaN when no row is labelled
+    dh: torch.Tensor    # [n, d] float64, zero at unlabelled rows
+    dw: torch.Tensor    # [V1, d] float64
+    db: torch.Tensor    # [V1] float64
+
+
+def masked_ce64(h: torch.Tensor, labels: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], v_begin: int = 0,
+                lse: Optional[torch.Tensor] = None, chunk: int = 65536) -> MaskedCE64:
+    """Masked cross-entropy of the BERT4Rec output layer and its gradients in float64, chunked over the vocabulary, on the
+    device the tensors live on: rows with ``labels != 0`` are scored against the columns ``w [V1, d]`` (+ ``bias``, None = zero),
+    ``loss = mean(lse - target logit)``, gradients for an upstream gradient of 1.
+
+    ``w`` may be a row block of the output layer starting at ``v_begin`` (a vocabulary shard): the target column of a row is
+    ``labels - v_begin``, and a target outside ``[0, V1)`` contributes no column (its target logit counts as 0).  ``lse``, when
+    given, replaces the block's own log-sum-exp in the backward (the global one of a sharded layer), so the rows of
+    softmax - onehot over this block need not sum to zero.  With no labelled row the loss is NaN and every gradient is zero,
+    as ``F.cross_entropy`` with every label ignored gives."""
+    sel = labels.reshape(-1) != 0
+    h2 = h.reshape(-1, h.shape[-1])
+    hc = h2[sel].double()
+    tg = labels.reshape(-1)[sel] - int(v_begin)
+    V1 = w.shape[0]
+    inb = (tg >= 0) & (tg < V1)
+    tgc = torch.where(inb, tg, torch.zeros_like(tg))
+    b64 = torch.zeros(V1, dtype=torch.float64, device=w.device) if bias is None else bias.double()
+    P = hc.shape[0]
+    own = torch.full((P,), -math.inf, dtype=torch.float64, device=h.device)
+    for v0 in range(0, V1, chunk):
+        own = torch.logaddexp(own, torch.logsumexp(hc @ w[v0:v0 + chunk].double().t() + b64[v0:v0 + chunk], 1))
+    tl = torch.where(inb, (hc * w[tgc].double()).sum(1) + b64[tgc], torch.zeros((), dtype=torch.float64, device=h.device))
+    loss = float((own - tl).mean()) if P else math.nan
+    L = own if lse is None else lse.reshape(-1)[:P].double()
+    dh_c = torch.zeros_like(hc)
+    dw = torch.zeros(V1, w.shape[1], dtype=torch.float64, device=w.device)
+    db = torch.zeros(V1, dtype=torch.float64, device=w.device)
+    for v0 in range(0, V1, chunk):
+        wc = w[v0:v0 + chunk].double()
+        G = torch.exp(hc @ wc.t() + b64[v0:v0 + chunk] - L[:, None])
+        hit = inb & (tg >= v0) & (tg < v0 + chunk)
+        G[hit.nonzero(as_tuple=True)[0], tg[hit] - v0] -= 1.0
+        G /= max(P, 1)
+        dh_c += G @ wc
+        dw[v0:v0 + chunk] = G.t() @ hc
+        db[v0:v0 + chunk] = G.sum(0)
+    dh = torch.zeros(h2.shape, dtype=torch.float64, device=h.device)
+    dh[sel] = dh_c
+    return MaskedCE64(own, loss, dh.view(h.shape), dw, db)
 
 
 def synth_state_dict(shapes: Dict[str, tuple], seed: int, scale: float = 0.1) -> Dict[str, torch.Tensor]:

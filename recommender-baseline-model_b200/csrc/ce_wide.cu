@@ -385,7 +385,8 @@ ce_wide_kernel(const __grid_constant__ CUtensorMap mapRl, const __grid_constant_
       named_bar_sync(7, NSW * 32);
       xch[grp * 128 + rl] = bsum;
       named_bar_sync(7, NSW * 32);
-      const float gscale = *a.dloss / (float)count;
+      // no labelled row: zero, not 0 x (dloss / 0) = NaN (test_ce_no_labelled_row)
+      const float gscale = count > 0 ? *a.dloss / (float)count : 0.f;
       const float wmul = gscale / (GSCALE * sh);  // D = sum (2^14 G) . (s_h H)
       float* pw = a.dpart + ((int64_t)blockIdx.y * V1 + vrow) * d;
       const int dc = d / 2;

@@ -259,9 +259,11 @@ __global__ void __launch_bounds__(256) ce_bwd_dh_kernel(CeArgs a) {
   stage_rows(Hs, QLD, a.h, a.rows, r0, count, d, RBM_LOG2E, lane);
   int64_t tg[2];
   float lse2[2];
+  bool live[2];
 #pragma unroll
   for (int hr = 0; hr < 2; ++hr) {
     int r = r0 + g + 8 * hr;
+    live[hr] = r < count;
     tg[hr] = (r < count && a.tgt[r] >= 0 && a.tgt[r] < a.V1) ? a.tgt[r] : -1;  // outside the (shard of the) vocabulary: no column
     lse2[hr] = r < count ? a.lse_in[r] * RBM_LOG2E : 0.f;
   }
@@ -299,7 +301,9 @@ __global__ void __launch_bounds__(256) ce_bwd_dh_kernel(CeArgs a) {
 #pragma unroll
       for (int cc = 0; cc < 4; ++cc) {
         int v = c * CH + nt * 8 + 2 * t + (cc & 1), hr = cc >> 1;
-        float p = (v < V1 && tg[hr] >= 0) ? ex2(s[nt][cc] + ((cc & 1) ? b2.y : b2.x) - lse2[hr]) : 0.f;
+        // a live row whose target lies in another vocabulary shard (tg = -1) still has its softmax here: test_ce_vocab_shards
+        // (simt_d48_S3) caught this guard once testing tg >= 0 instead of the row being live
+        float p = (v < V1 && live[hr]) ? ex2(s[nt][cc] + ((cc & 1) ? b2.y : b2.x) - lse2[hr]) : 0.f;
         if ((int64_t)v == tg[hr]) p -= 1.f;
         gg[cc] = p * gscale;
       }
@@ -356,7 +360,7 @@ __global__ void __launch_bounds__(256) ce_bwd_dw_kernel(CeArgs a) {
     panel_load_async(panel + buf * CH * LD, a.h, a.rows, (int64_t)c * CH, count, d, LD);
     for (int j = threadIdx.x; j < CH; j += blockDim.x) {
       int r = c * CH + j;
-      lse_s[buf * CH + j] = r < count ? a.lse_in[r] * RBM_LOG2E : 0.f;
+      lse_s[buf * CH + j] = r < count ? a.lse_in[r] * RBM_LOG2E : INFINITY;  // columns beyond the count: p = 0
       tgt_s[buf * CH + j] = (r < count && a.tgt[r] >= 0 && a.tgt[r] < a.V1) ? (float)a.tgt[r] : -1.f;
     }
     cp_async_commit();
@@ -386,7 +390,9 @@ __global__ void __launch_bounds__(256) ce_bwd_dw_kernel(CeArgs a) {
       for (int cc = 0; cc < 4; ++cc) {
         int hr = cc >> 1;
         float tcol = (cc & 1) ? ts.y : ts.x, lcol = (cc & 1) ? ls.y : ls.x;
-        float p = (vrow[hr] < V1 && tcol >= 0.f) ? ex2(s[nt][cc] + b2[hr] - lcol) : 0.f;
+        // the column of a live row whose target lies in another vocabulary shard (tcol = -1) is not zero: test_ce_vocab_shards
+        // (simt_d48_S3) caught this guard once testing tcol >= 0 instead of the row being live
+        float p = (vrow[hr] < V1 && lcol != INFINITY) ? ex2(s[nt][cc] + b2[hr] - lcol) : 0.f;
         if (tcol == (float)vrow[hr]) p -= 1.f;
         gg[cc] = p * gscale;
         bsum[hr] += gg[cc];

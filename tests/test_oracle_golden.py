@@ -1,10 +1,12 @@
 """Pin the CPU oracle against vectors minted from the unmodified reference
 (tests/golden/make_golden.py).  CPU only."""
+import math
 import os
 
 import numpy as np
 import pytest
 import torch
+import torch.nn.functional as F
 
 from oracle import bert4rec as ob, sasrec as osr, metrics as om, optim as oo, common as oc
 
@@ -328,3 +330,63 @@ def test_data_partition_vs_reference(tmp_path, L, prop, tag):
     np.testing.assert_array_equal(np.array([i for r in tr for i in r], np.int64), z[tag + ".train"])
     np.testing.assert_array_equal(np.array([r[0] for r in va], np.int64), z[tag + ".valid"])
     np.testing.assert_array_equal(np.array([r[0] for r in te], np.int64), z[tag + ".test"])
+
+
+# --------------------------------------------------------------------------------- masked cross-entropy in float64
+def _ce_inputs(n, V1, d, seed, frac=0.6):
+    g = torch.Generator().manual_seed(seed)
+    h = torch.randn(n, d, generator=g, dtype=torch.float64)
+    w = torch.randn(V1, d, generator=g, dtype=torch.float64) * 0.4
+    b = torch.randn(V1, generator=g, dtype=torch.float64)
+    labels = torch.where(torch.rand(n, generator=g) < frac, torch.randint(1, V1, (n,), generator=g), torch.zeros(n, dtype=torch.long))
+    return h, labels, w, b
+
+
+@pytest.mark.parametrize("n,V1,d,frac,bias", [(23, 17, 8, 0.6, True), (40, 101, 16, 0.3, False), (9, 5, 4, 1.0, True), (12, 30, 8, 0.0, True)])
+def test_masked_ce64_equals_torch(n, V1, d, frac, bias):
+    """oc.masked_ce64 is F.cross_entropy(h.w^T + b, labels, ignore_index=0) in float64: loss, dH, dW, db (chunked over a
+    vocabulary that is not a multiple of the chunk); bias=None is a zero bias; no labelled row gives a NaN loss and zero
+    gradients, as torch does."""
+    h, labels, w, b = _ce_inputs(n, V1, d, n)
+    if not bias:
+        b = torch.zeros_like(b)
+    leaves = [t.clone().requires_grad_(True) for t in (h, w, b)]
+    ref = F.cross_entropy(F.linear(*leaves), labels, ignore_index=0)
+    ref.backward()
+    got = oc.masked_ce64(h, labels, w, b if bias else None, chunk=7)
+    sel = labels != 0
+    assert got.lse.shape == (int(sel.sum()),)
+    if not bool(sel.any()):
+        assert math.isnan(got.loss) and math.isnan(ref.item())
+        assert not got.dh.any() and not got.dw.any() and not got.db.any()
+        assert not leaves[0].grad.any() and not leaves[1].grad.any()
+        return
+    torch.testing.assert_close(got.lse, torch.logsumexp(F.linear(h, w, b)[sel], 1), rtol=1e-13, atol=1e-13)
+    assert abs(got.loss - ref.item()) < 1e-13 * abs(ref.item())
+    torch.testing.assert_close(got.dh, leaves[0].grad, rtol=1e-12, atol=1e-14)
+    torch.testing.assert_close(got.dw, leaves[1].grad, rtol=1e-12, atol=1e-14)
+    torch.testing.assert_close(got.db, leaves[2].grad, rtol=1e-12, atol=1e-14)
+
+@pytest.mark.parametrize("bounds", [[0, 37], [0, 20, 37], [0, 13, 26, 37], [0, 5, 10, 15, 20, 25, 30, 35, 37],
+                                    [0, 30, 35, 36, 37], [0, 1, 36, 37]], ids=lambda b: "S%d_%s" % (len(b) - 1, "_".join(map(str, b))))
+def test_masked_ce64_vocab_shards_combine(bounds):
+    """The vocabulary-parallel loss restated with the oracle: per shard [v_begin, v_end) the forward with labels shifted by
+    -v_begin (a target outside the shard contributes no column), dist.combine_shard_lse of the shard log-sum-exps and losses,
+    per shard the backward with the global log-sum-exp, dH summed over the shards.  It reproduces the unsharded log-sum-exp,
+    loss, dW, db and dH for 1, 2, 3 and 8 shards, uneven last shards and one-row shards."""
+    from rbm_b200 import dist as rd
+    n, V1, d = 60, bounds[-1], 8
+    h, labels, w, b = _ce_inputs(n, V1, d, 7)
+    labels[3], labels[4] = V1 - 1, 1  # the last and first scored ids
+    full = oc.masked_ce64(h, labels, w, b)
+    shards = [oc.masked_ce64(h, labels, w[v0:v1], b[v0:v1], v_begin=v0) for v0, v1 in zip(bounds[:-1], bounds[1:])]
+    count = torch.tensor([full.lse.shape[0]], dtype=torch.int32)
+    LSE, loss = rd.combine_shard_lse(torch.stack([s.lse for s in shards]), torch.tensor([s.loss for s in shards]), count)
+    torch.testing.assert_close(LSE.double(), full.lse, rtol=1e-6, atol=1e-6)
+    assert abs(loss.item() - full.loss) < 1e-6 * abs(full.loss)
+    if len(bounds) > 2:  # a shard's own rows of softmax - onehot do not sum to zero: the global LSE matters
+        assert (shards[0].lse - full.lse).abs().max() > 0.1
+    back = [oc.masked_ce64(h, labels, w[v0:v1], b[v0:v1], v_begin=v0, lse=LSE) for v0, v1 in zip(bounds[:-1], bounds[1:])]
+    torch.testing.assert_close(torch.cat([s.dw for s in back]), full.dw, rtol=1e-5, atol=1e-8)
+    torch.testing.assert_close(torch.cat([s.db for s in back]), full.db, rtol=1e-5, atol=1e-8)
+    torch.testing.assert_close(sum(s.dh for s in back), full.dh, rtol=1e-5, atol=1e-8)
