@@ -447,11 +447,7 @@ int launch(Kern kern, const AttnArgs& a, int B, int warps, size_t (*smem_fn)(int
     rbm_set_error("%s: L=%d dk=%d needs %zu B of shared memory (> 227 KB): unsupported shape", name, a.L, a.dk, smem);
     return -1;
   }
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) {
-    rbm_set_error("%s: cudaFuncSetAttribute: %s", name, cudaGetErrorString(e));
-    return (int)e;
-  }
+  if (!set_smem(kern, smem, name)) return -1;
   kern<<<B * a.h, 32 * warps, smem, st>>>(a);
   RBM_LAUNCH_CHECK(name);
   return 0;

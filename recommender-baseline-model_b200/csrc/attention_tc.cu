@@ -22,17 +22,6 @@ using rbm_mma::ex2;
 constexpr int DK = 32;
 constexpr int ROWB = DK * 4;     // 128 bytes per token row
 
-__device__ __forceinline__ void split_lo_bytes(const uint8_t* src, uint8_t* dst, int n4, int tid, int nthr) {
-  for (int i = tid; i < n4; i += nthr) {
-    float4 v = ld4(reinterpret_cast<const float*>(src) + i * 4), o;
-    o.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xffffe000u);
-    o.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xffffe000u);
-    o.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xffffe000u);
-    o.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xffffe000u);
-    st4(reinterpret_cast<float*>(dst) + i * 4, o);
-  }
-}
-
 // =====================================================================================================
 // Dropout words of one query row for the 16 keys [16*npair, 16*npair + 16).  Rows i and i^8 (lanes l, l^8 of a warp
 // whose lanes hold consecutive rows) share their four Philox calls: each lane computes two and trades the words the
@@ -60,41 +49,6 @@ __device__ __forceinline__ KeepWords attn_keep_words(uint64_t seed, uint64_t sit
 __device__ __forceinline__ bool attn_keep_bit(const KeepWords& k, int jj, uint32_t thr_hi) {
   const uint32_t w = k.w[((jj & 7) >> 1) * 2 + (jj & 1)];
   return (jj & 8) ? (w >= thr_hi) : ((w << 16) >= thr_hi);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Bring-up timeline (RBM_TC_ATTN_TRACE=<file>): CTA 0 appends (clock64, event, argument) records to a device buffer that
-// the launcher dumps after the kernel.  trace == nullptr (the default) compiles down to one predictable branch.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int TRACE_WARPS = 16, TRACE_PER_WARP = 500, TRACE_CAP = TRACE_WARPS * TRACE_PER_WARP;
-// every warp owns a slice of the buffer and a private counter: a record costs one clock read and one plain store
-__device__ __forceinline__ void tc_trace(unsigned long long* trace, int& cnt, int ev, int arg) {
-  if (trace != nullptr && blockIdx.x == 0 && (threadIdx.x & 31) == 0 && cnt < TRACE_PER_WARP) {
-    const int w = (threadIdx.x >> 5) % TRACE_WARPS;
-    trace[1 + w * TRACE_PER_WARP + cnt] = ((unsigned long long)clock64() << 24) | ((unsigned long long)(ev & 0xff) << 16) | (unsigned)(arg & 0xffff);
-    ++cnt;
-  }
-}
-static unsigned long long* trace_begin() {
-  const char* path = getenv("RBM_TC_ATTN_TRACE");
-  if (!path) return nullptr;
-  unsigned long long* buf = nullptr;
-  if (cudaMalloc(&buf, (TRACE_CAP + 1) * sizeof(unsigned long long)) != cudaSuccess) return nullptr;
-  cudaMemset(buf, 0, (TRACE_CAP + 1) * sizeof(unsigned long long));
-  return buf;
-}
-static void trace_end(unsigned long long* buf, const char* tag, cudaStream_t st) {
-  if (!buf) return;
-  cudaStreamSynchronize(st);
-  static unsigned long long host[TRACE_CAP + 1];
-  cudaMemcpy(host, buf, sizeof(host), cudaMemcpyDeviceToHost);
-  cudaFree(buf);
-  char name[512];
-  snprintf(name, sizeof(name), "%s.%s", getenv("RBM_TC_ATTN_TRACE"), tag);
-  if (FILE* f = fopen(name, "wb")) {
-    fwrite(host, sizeof(unsigned long long), TRACE_CAP + 1, f);
-    fclose(f);
-  }
 }
 
 // =====================================================================================================
@@ -235,8 +189,8 @@ __global__ void __launch_bounds__(F_THREADS, 1) attn_fwd_tc_kernel(const __grid_
     if (tmem != 0) __trap();  // the CTA owns all 512 columns: literal addresses keep the issue loop on the uniform datapath
     if (elect_one()) {
       constexpr uint32_t tmem = 0;
-      const uint32_t idO2 = make_idesc_tf32_ex(128, 2 * DK, 0, 1);  // A from TMEM, [V | V_lo] MN-major, N = 64
-      const uint32_t idO1 = make_idesc_tf32_ex(128, DK, 0, 1);
+      const uint32_t idO2 = make_idesc_tf32(128, 2 * DK, 0, 1);  // A from TMEM, [V | V_lo] MN-major, N = 64
+      const uint32_t idO1 = make_idesc_tf32(128, DK, 0, 1);
       auto issue_s = [&](int n, int c) {
         const int g = n * NCH + c, s = g % F_NSTG;
         const int k0 = ((c * NU) / NCH) << 4, nh = ((((c + 1) * NU) / NCH) << 4) - k0;
@@ -244,7 +198,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) attn_fwd_tc_kernel(const __grid_
         mbar_wait(smem_u32(&kfull[s]), (g / F_NSTG) & 1);
         mbar_wait(smem_u32(&ksplit[s]), (g / F_NSTG) & 1);
         tc_fence_after();
-        const uint32_t idS = make_idesc_tf32_ex(128, nh, 0, 0);
+        const uint32_t idS = make_idesc_tf32(128, nh, 0, 0);
         const uint32_t sa = smem_base + s * F_STAGE;
         const uint64_t dK = make_sw128_desc(sa), dKl = make_sw128_desc(sa + F_TILE);
         const uint32_t tS = tmem + F_S + (uint32_t)k0;
@@ -369,7 +323,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) attn_fwd_tc_kernel(const __grid_
               sum += p;
               if (DROP) p = attn_keep_bit(kw, jj, thr_hi) ? p * a.inv_keep : 0.f;
               v[jj] = p;
-              lo[jj] = p - __uint_as_float(__float_as_uint(p) & 0xffffe000u);
+              lo[jj] = tf32_lo(p);
             }
             tmem_st16(tS + (uint32_t)j0, v);
             tmem_st16(tPl + (uint32_t)c0, lo);
@@ -472,7 +426,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) attn_fwd_tc_kernel(const __grid_
           for (int c = 0; c < 16; ++c) t16[c] = qv[part * 16 + c];
           tmem_st16(tmem + lane_sel + F_Q + part * 16, t16);
 #pragma unroll
-          for (int c = 0; c < 16; ++c) t16[c] = t16[c] - __uint_as_float(__float_as_uint(t16[c]) & 0xffffe000u);
+          for (int c = 0; c < 16; ++c) t16[c] = tf32_lo(t16[c]);
           tmem_st16(tmem + lane_sel + F_QL + part * 16, t16);
         }
         tmem_st_wait();
@@ -491,8 +445,8 @@ __global__ void __launch_bounds__(F_THREADS, 1) attn_fwd_tc_kernel(const __grid_
     auto split = [&](uint64_t* full, uint64_t* done, uint32_t off, int g) {
       const int s = g % F_NSTG;
       mbar_wait(smem_u32(&full[s]), (g / F_NSTG) & 1);
-      uint8_t* st = gen + off + (size_t)s * F_STAGE;
-      split_lo_bytes(st, st + F_TILE, (int)(F_TILE / 16), tid, 64);
+      float* st = reinterpret_cast<float*>(gen + off + (size_t)s * F_STAGE);
+      split_lo(st, st + F_TILE / 4, (int)(F_TILE / 16), tid, 64);
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&done[s]));
@@ -548,7 +502,6 @@ struct TcBwdArgs {
   uint32_t thr16;
   float inv_keep;
   uint64_t seed, site;
-  unsigned long long* trace;
 };
 
 template <bool CAUSAL, bool DROP>
@@ -570,7 +523,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
   const int NU = LPK >> 4, NCH = (NU + 3) >> 2;  // 16-key units; chunks of <= 4 units, sizes as even as possible
   const int n_items = a.items > (int)blockIdx.x ? (a.items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
   const int n_chunks = n_items * NCH;
-  int tcnt = 0;  // bring-up timeline cursor of this warp
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (smem_base - smem_u32(smem_raw));
 
@@ -632,7 +584,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
           tma_load_3d(sa, &mapKk, bar, hh * DK, k0, b);
           tma_load_3d(sa + A_TILE, &mapVk, bar, hh * DK, k0, b);
           tma_load_3d(sa + 2 * A_TILE, &mapKm, bar, hh * DK, k0, b);
-          tc_trace(a.trace, tcnt, 10, g);
         }
         if (n + 1 < n_items) issue_rows(n + 1);
       }
@@ -647,18 +598,16 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
     // All 32 lanes run the loop in lockstep; one elected lane issues each tcgen05 instruction.  A tcgen05.mma of this
     // size costs the issuing warp (and the pipe) ~64 cycles whatever its N <= 128, so the count of instructions is what
     // matters: the two products that share the A operand dS_raw run as one N = 64 instruction against [K_raw | K_lo].
-    const uint32_t idQ2 = make_idesc_tf32_ex(128, 2 * DK, 0, 1);  // dQ: A from TMEM, [K | K_lo] MN-major, N = 64
-    const uint32_t idQ1 = make_idesc_tf32_ex(128, DK, 0, 1);
+    const uint32_t idQ2 = make_idesc_tf32(128, 2 * DK, 0, 1);  // dQ: A from TMEM, [K | K_lo] MN-major, N = 64
+    const uint32_t idQ1 = make_idesc_tf32(128, DK, 0, 1);
     auto issue_dq = [&](int g) {
       const int n = g / NCH, c = g - n * NCH, s = g % A_NSTG;
       const int k0 = ((c * NU) / NCH) << 4, nh = ((((c + 1) * NU) / NCH) << 4) - k0;
       const uint32_t tS = tmem + (uint32_t)(g & 1) * A_GRP, tP = tS + A_DP, tD = tmem + A_DQ + (uint32_t)(n & 1) * (2 * DK);
       const uint32_t sa = smem_base + s * A_STAGE;
-      tc_trace(a.trace, tcnt, 1, g);
       mbar_wait(smem_u32(&ds_full[g & 1]), (g >> 1) & 1);
       if (c == 0 && n >= 2) mbar_wait(smem_u32(&dq_free[n & 1]), ((n >> 1) - 1) & 1);
       tc_fence_after();
-      tc_trace(a.trace, tcnt, 2, g);
       for (int kk = 0; kk < nh / 8; ++kk) {
         const uint64_t dKm2 = make_sw128_desc_mn(sa + 2 * A_TILE + kk * 1024, 3 * A_TILE);  // second MN block = the residual tile
         const uint64_t dKm = make_sw128_desc_mn(sa + 2 * A_TILE + kk * 1024, 0);
@@ -667,7 +616,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       }
       umma_commit(smem_u32(&empty_bar[s]));
       if (c == NCH - 1) umma_commit(smem_u32(&dq_full[n & 1]));
-      tc_trace(a.trace, tcnt, 3, g);
     };
     int g = 0;
     for (int n = 0; n < n_items; ++n) {
@@ -675,17 +623,12 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
         if (g >= 2) issue_dq(g - 2);  // frees this group's accumulators (the tensor pipe runs in order)
         const int s = g % A_NSTG;
         const int k0 = ((c * NU) / NCH) << 4, nh = ((((c + 1) * NU) / NCH) << 4) - k0;
-        if (c == 0) {
-          tc_trace(a.trace, tcnt, 12, n);
-          mbar_wait(smem_u32(&ops_full), n & 1);
-          tc_trace(a.trace, tcnt, 13, n);
-        }
+        if (c == 0) mbar_wait(smem_u32(&ops_full), n & 1);
         mbar_wait(smem_u32(&full_bar[s]), (g / A_NSTG) & 1);
         mbar_wait(smem_u32(&split_bar[s]), (g / A_NSTG) & 1);
         tc_fence_after();
-        tc_trace(a.trace, tcnt, 4, g);
         const uint32_t tS = tmem + (uint32_t)(g & 1) * A_GRP, tP = tS + A_DP;
-        const uint32_t idS = make_idesc_tf32_ex(128, nh, 0, 0);
+        const uint32_t idS = make_idesc_tf32(128, nh, 0, 0);
         const uint32_t sa = smem_base + s * A_STAGE;
         const uint64_t dK = make_sw128_desc(sa), dKl = make_sw128_desc(sa + 3 * A_TILE);
         const uint64_t dV = make_sw128_desc(sa + A_TILE), dVl = make_sw128_desc(sa + 4 * A_TILE);
@@ -705,7 +648,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
         }
         umma_commit(smem_u32(&s_full[g & 1]));
         if (c == NCH - 1) umma_commit(smem_u32(&ops_free));  // Q / dO of this item have been consumed
-        tc_trace(a.trace, tcnt, 5, g);
       }
     }
     for (int gg = n_chunks >= 2 ? n_chunks - 2 : 0; gg < n_chunks; ++gg) issue_dq(gg);
@@ -743,7 +685,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       }
       mbar_wait(smem_u32(&s_full[grp]), (g >> 1) & 1);
       tc_fence_after();
-      tc_trace(a.trace, tcnt, 6, g * 4 + q);
       if (new_item) ndelta = -xdelta[n & 1][rl];
       if (warp_live) {
         const float* kvp = kvalid[n & 1];
@@ -774,7 +715,7 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
             if (CAUSAL) live = live && (j0 + jj <= i);
             const float ds = live ? p * t : 0.f;
             sv[jj] = ds;
-            lo[jj] = ds - __uint_as_float(__float_as_uint(ds) & 0xffffe000u);
+            lo[jj] = tf32_lo(ds);
           }
           tmem_st16(tS + (uint32_t)c0, sv);
           tmem_st16(tP + (uint32_t)c0, lo);
@@ -783,7 +724,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       }
       tc_fence_before();
       __syncwarp();
-      tc_trace(a.trace, tcnt, 7, g * 4 + q);
       if (lane == 0) mbar_arrive(smem_u32(&ds_full[grp]));
     }
   } else if (warp < 14) {
@@ -835,7 +775,6 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&dq_free[n & 1]));
-      if (q == 0) tc_trace(a.trace, tcnt, 9, n);
       if (i < a.Lq) {
         float* dst = a.dq + ((int64_t)b * a.Lq + i) * a.lddq + hh * DK;
 #pragma unroll
@@ -853,12 +792,10 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       kvalid[n & 1][t128 + 128] = kval1 ? 1.f : 0.f;
       xdelta[n & 1][rl] = dl;
       if (i < a.Lq) a.delta[(int64_t)bh * a.Lq + i] = dl;
-      if (q == 0) tc_trace(a.trace, tcnt, 14, n);
       if (n >= 1) {
         mbar_wait(smem_u32(&ops_free), (n - 1) & 1);  // every S / dP of the previous item has read its Q / dO
         tc_fence_after();
       }
-      if (q == 0) tc_trace(a.trace, tcnt, 15, n);
       {
         float t16[16];
 #pragma unroll
@@ -867,13 +804,13 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
           for (int c = 0; c < 16; ++c) t16[c] = qv[part * 16 + c];
           tmem_st16(tmem + lane_sel + A_Q + part * 16, t16);
 #pragma unroll
-          for (int c = 0; c < 16; ++c) t16[c] = t16[c] - __uint_as_float(__float_as_uint(t16[c]) & 0xffffe000u);
+          for (int c = 0; c < 16; ++c) t16[c] = tf32_lo(t16[c]);
           tmem_st16(tmem + lane_sel + A_QL + part * 16, t16);
 #pragma unroll
           for (int c = 0; c < 16; ++c) t16[c] = dv[part * 16 + c];
           tmem_st16(tmem + lane_sel + A_DO + part * 16, t16);
 #pragma unroll
-          for (int c = 0; c < 16; ++c) t16[c] = t16[c] - __uint_as_float(__float_as_uint(t16[c]) & 0xffffe000u);
+          for (int c = 0; c < 16; ++c) t16[c] = tf32_lo(t16[c]);
           tmem_st16(tmem + lane_sel + A_DOL + part * 16, t16);
         }
         tmem_st_wait();
@@ -881,9 +818,7 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&ops_full));
-      tc_trace(a.trace, tcnt, 8, n * 4 + q);
       if (n + 1 < n_items) load_rows(n + 1);  // in flight while this item is being worked on
-      if (q == 0) tc_trace(a.trace, tcnt, 16, n);
       if (n >= 1) store_dq(n - 1);
     }
     if (n_items > 0) store_dq(n_items - 1);
@@ -893,12 +828,11 @@ __global__ void __launch_bounds__(A_THREADS, 1) attn_bwd_dq_tc_kernel(const __gr
     for (int g = 0; g < n_chunks; ++g) {
       const int s = g % A_NSTG;
       mbar_wait(smem_u32(&full_bar[s]), (g / A_NSTG) & 1);
-      uint8_t* st = gen + (size_t)s * A_STAGE;
-      split_lo_bytes(st, st + 3 * A_TILE, (int)(3 * A_TILE / 16), tid, 64);
+      float* st = reinterpret_cast<float*>(gen + (size_t)s * A_STAGE);
+      split_lo(st, st + 3 * A_TILE / 4, (int)(3 * A_TILE / 16), tid, 64);
       fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_u32(&split_bar[s]));
-      tc_trace(a.trace, tcnt, 11, g);
     }
   }
   tc_fence_before();
@@ -946,7 +880,6 @@ struct TcBwdKvArgs {
   uint32_t thr16;
   float inv_keep;
   uint64_t seed, site;
-  unsigned long long* trace;
 };
 
 template <bool CAUSAL, bool DROP>
@@ -966,7 +899,6 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
   const int L = a.L, LPK = a.LPK;
   const int NSC = (LPK + SQ - 1) / SQ;  // sub-chunks per sequence
   const int n_items = a.items > (int)blockIdx.x ? (a.items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
-  int tcnt = 0;
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* gen = smem_raw + (smem_base - smem_u32(smem_raw));
   const uint32_t off_rows = B_NSTG * B_STAGE, off_out = off_rows + 2 * B_ROWS;
@@ -1038,8 +970,8 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
     if (tmem != 0) __trap();  // the CTA owns all 512 columns: literal addresses keep the issue loop on the uniform datapath
     if (elect_one()) {
       constexpr uint32_t tmem = 0;
-      const uint32_t idA2 = make_idesc_tf32_ex(128, 2 * DK, 0, 1);  // A from TMEM, [B | B_lo] MN-major, N = 64
-      const uint32_t idA1 = make_idesc_tf32_ex(128, DK, 0, 1);
+      const uint32_t idA2 = make_idesc_tf32(128, 2 * DK, 0, 1);  // A from TMEM, [B | B_lo] MN-major, N = 64
+      const uint32_t idA1 = make_idesc_tf32(128, DK, 0, 1);
       // the two most recent sub-chunks (one per group) whose dK / dV update is still to be issued
       int p_g[2] = {-1, -1}, p_nq[2] = {0, 0}, p_n[2] = {0, 0};
       bool p_first[2] = {false, false}, p_last[2] = {false, false};
@@ -1079,7 +1011,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
           mbar_wait(smem_u32(&split_bar[s]), (g / B_NSTG) & 1);
           tc_fence_after();
           const uint32_t tG = tmem + B_GRP0 + (uint32_t)grp * B_GRP;
-          const uint32_t idS = make_idesc_tf32_ex(128, nq, 0, 0);
+          const uint32_t idS = make_idesc_tf32(128, nq, 0, 0);
           const uint32_t sa = smem_base + s * B_STAGE, sl = sa + 4 * B_TILE;
           const uint64_t dQk = make_sw128_desc(sa + 0 * B_TILE), dQkl = make_sw128_desc(sl + 0 * B_TILE);
           const uint64_t dOk = make_sw128_desc(sa + 2 * B_TILE), dOkl = make_sw128_desc(sl + 2 * B_TILE);
@@ -1185,14 +1117,14 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
               }
               const float ds = jpad ? 0.f : p * (mk * __uint_as_float(rd[ii]) - sd[i]);
               sv[ii] = ds;
-              dlo[ii] = ds - __uint_as_float(__float_as_uint(ds) & 0xffffe000u);
+              dlo[ii] = tf32_lo(ds);
               t16[ii] = p * mk;
             }
             tmem_st16(tG + (uint32_t)c0, sv);
             tmem_st16(tG + B_DPT + (uint32_t)c0, dlo);
             tmem_st16(tG + B_P + (uint32_t)c0, t16);
 #pragma unroll
-            for (int ii = 0; ii < 16; ++ii) t16[ii] = t16[ii] - __uint_as_float(__float_as_uint(t16[ii]) & 0xffffe000u);
+            for (int ii = 0; ii < 16; ++ii) t16[ii] = tf32_lo(t16[ii]);
             tmem_st16(tG + B_PL + (uint32_t)c0, t16);
           }
           tmem_st_wait();
@@ -1293,13 +1225,13 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
           for (int c = 0; c < 16; ++c) t16[c] = kv[part * 16 + c];
           tmem_st16(tmem + lane_sel + B_K + part * 16, t16);
 #pragma unroll
-          for (int c = 0; c < 16; ++c) t16[c] = t16[c] - __uint_as_float(__float_as_uint(t16[c]) & 0xffffe000u);
+          for (int c = 0; c < 16; ++c) t16[c] = tf32_lo(t16[c]);
           tmem_st16(tmem + lane_sel + B_KL + part * 16, t16);
 #pragma unroll
           for (int c = 0; c < 16; ++c) t16[c] = vv[part * 16 + c];
           tmem_st16(tmem + lane_sel + B_V + part * 16, t16);
 #pragma unroll
-          for (int c = 0; c < 16; ++c) t16[c] = t16[c] - __uint_as_float(__float_as_uint(t16[c]) & 0xffffe000u);
+          for (int c = 0; c < 16; ++c) t16[c] = tf32_lo(t16[c]);
           tmem_st16(tmem + lane_sel + B_VL + part * 16, t16);
         }
         tmem_st_wait();
@@ -1322,15 +1254,14 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_dkv_tc_kernel(const __g
       for (int c = first_chunk(item % a.NT); c < NSC; ++c, ++g) {
         const int s = g % B_NSTG;
         mbar_wait(smem_u32(&full_bar[s]), (g / B_NSTG) & 1);
-        uint8_t* st = gen + (size_t)s * B_STAGE;
-        split_lo_bytes(st, st + 4 * B_TILE, (int)(4 * B_TILE / 16), tid, 64);
+        float* st = reinterpret_cast<float*>(gen + (size_t)s * B_STAGE);
+        split_lo(st, st + 4 * B_TILE / 4, (int)(4 * B_TILE / 16), tid, 64);
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_u32(&split_bar[s]));
       }
     }
   }
-  (void)tcnt;
   tc_fence_before();
   __syncthreads();
   if (warp == 1) {
@@ -1396,14 +1327,11 @@ int rbm_attn_fwd_tc_launch(const float* q, int64_t ldq, const float* k, int64_t 
   const size_t smem = (size_t)2 * F_NSTG * F_STAGE + F_ROWS + 4 * F_OUT + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fwd_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_attn_fwd(tcgen05): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(attn_fwd_tc_kernel<false, false>, smem, "rbm_attn_fwd(tcgen05)") ||
+        !set_smem(attn_fwd_tc_kernel<false, true>, smem, "rbm_attn_fwd(tcgen05)") ||
+        !set_smem(attn_fwd_tc_kernel<true, false>, smem, "rbm_attn_fwd(tcgen05)") ||
+        !set_smem(attn_fwd_tc_kernel<true, true>, smem, "rbm_attn_fwd(tcgen05)"))
+      return -1;
     attr_set = true;
   }
   const bool causal = mask_mode == RBM_MASK_CAUSAL, drop = a.thr16 != 0;
@@ -1441,18 +1369,14 @@ int rbm_attn_bwd_dq_tc_launch(const float* q, int64_t ldq, const float* k, int64
   a.tok = tok; a.L = L; a.Lq = Lq; a.LPK = LPK; a.h = h; a.NT = NT; a.mask_mode = mask_mode; a.scale = scale; a.scale_log2 = scale * RBM_LOG2E;
   a.thr16 = rbm_drop_threshold16(p); a.inv_keep = 1.f / (1.f - p); a.seed = seed; a.site = site;
   a.items = B * h * NT;
-  a.trace = trace_begin();
   const size_t smem = (size_t)A_NSTG * A_STAGE + 3 * A_ROWS + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_dq_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dq_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dq_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dq_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_attn_bwd(tcgen05): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(attn_bwd_dq_tc_kernel<false, false>, smem, "rbm_attn_bwd(tcgen05)") ||
+        !set_smem(attn_bwd_dq_tc_kernel<false, true>, smem, "rbm_attn_bwd(tcgen05)") ||
+        !set_smem(attn_bwd_dq_tc_kernel<true, false>, smem, "rbm_attn_bwd(tcgen05)") ||
+        !set_smem(attn_bwd_dq_tc_kernel<true, true>, smem, "rbm_attn_bwd(tcgen05)"))
+      return -1;
     attr_set = true;
   }
   const bool causal = mask_mode == RBM_MASK_CAUSAL, drop = a.thr16 != 0;
@@ -1462,7 +1386,6 @@ int rbm_attn_bwd_dq_tc_launch(const float* q, int64_t ldq, const float* k, int64
   else if (drop) attn_bwd_dq_tc_kernel<false, true><<<grid, A_THREADS, smem, st>>>(mapKk, mapKm, mapVk, mapQ, mapDO, mapO, a);
   else attn_bwd_dq_tc_kernel<false, false><<<grid, A_THREADS, smem, st>>>(mapKk, mapKm, mapVk, mapQ, mapDO, mapO, a);
   RBM_LAUNCH_CHECK("rbm_attn_bwd(tcgen05 dq)");
-  trace_end(a.trace, "dq", st);
   return 0;
 }
 
@@ -1491,18 +1414,14 @@ int rbm_attn_bwd_dkv_tc_launch(const float* q, int64_t ldq, const float* k, int6
   a.tok = tok; a.L = L; a.Lq = Lq; a.LPK = LPK; a.h = h; a.NT = NT; a.mask_mode = mask_mode; a.scale = scale; a.scale_log2 = scale * RBM_LOG2E;
   a.thr16 = rbm_drop_threshold16(p); a.inv_keep = 1.f / (1.f - p); a.seed = seed; a.site = site;
   a.items = B * h * NT;
-  a.trace = nullptr;
   const size_t smem = (size_t)B_NSTG * B_STAGE + 2 * B_ROWS + 8 * B_OUT + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(attn_bwd_dkv_tc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dkv_tc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dkv_tc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_bwd_dkv_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_attn_bwd(tcgen05 dkv): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(attn_bwd_dkv_tc_kernel<false, false>, smem, "rbm_attn_bwd(tcgen05 dkv)") ||
+        !set_smem(attn_bwd_dkv_tc_kernel<false, true>, smem, "rbm_attn_bwd(tcgen05 dkv)") ||
+        !set_smem(attn_bwd_dkv_tc_kernel<true, false>, smem, "rbm_attn_bwd(tcgen05 dkv)") ||
+        !set_smem(attn_bwd_dkv_tc_kernel<true, true>, smem, "rbm_attn_bwd(tcgen05 dkv)"))
+      return -1;
     attr_set = true;
   }
   const bool causal = mask_mode == RBM_MASK_CAUSAL, drop = a.thr16 != 0;

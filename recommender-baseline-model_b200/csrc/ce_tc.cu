@@ -38,8 +38,6 @@ struct CeTcArgs {
   int bias_vec;        // bias pointer is 16-byte aligned: whole-chunk float4 loads
 };
 
-__device__ __forceinline__ float lo_of(float x) { return x - __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
-
 // thread-owned row (d floats, global) -> TMEM raw / lo regions, scaled
 __device__ __forceinline__ void row_to_tmem(const float* __restrict__ src, bool valid, float mul, int d, uint32_t t_raw, uint32_t t_lo) {
   for (int c0 = 0; c0 < d; c0 += 16) {
@@ -50,7 +48,7 @@ __device__ __forceinline__ void row_to_tmem(const float* __restrict__ src, bool 
       v[c] = x.x * mul; v[c + 1] = x.y * mul; v[c + 2] = x.z * mul; v[c + 3] = x.w * mul;
     }
 #pragma unroll
-    for (int c = 0; c < 16; ++c) lo[c] = lo_of(v[c]);
+    for (int c = 0; c < 16; ++c) lo[c] = tf32_lo(v[c]);
     tmem_st16(t_raw + c0, v);
     tmem_st16(t_lo + c0, lo);
   }
@@ -125,7 +123,7 @@ __global__ void __launch_bounds__(64 + 32 * NSW, 1) ce_fwd_tc_kernel(const __gri
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idS = make_idesc_tf32_ex(128, CW, 0, 0);
+      const uint32_t idS = make_idesc_tf32(128, CW, 0, 0);
       mbar_wait(smem_u32(&h_bar), 0);
       tc_fence_after();
       for (int c = 0; c < NC; ++c) {
@@ -298,7 +296,7 @@ __global__ void __launch_bounds__(64 + 32 * NSW, 1) ce_bwd_dh_tc_kernel(const __
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idS = make_idesc_tf32_ex(128, CW, 0, 0), id2 = make_idesc_tf32_ex(128, 2 * d, 0, 1), id1 = make_idesc_tf32_ex(128, d, 0, 1);
+      const uint32_t idS = make_idesc_tf32(128, CW, 0, 0), id2 = make_idesc_tf32(128, 2 * d, 0, 1), id1 = make_idesc_tf32(128, d, 0, 1);
       mbar_wait(smem_u32(&h_bar), 0);
       tc_fence_after();
       int pend[2] = {-1, -1};
@@ -377,7 +375,7 @@ __global__ void __launch_bounds__(64 + 32 * NSW, 1) ce_bwd_dh_tc_kernel(const __
           if (hit && ts == (uint32_t)j) p -= 1.f;
           const float gg = p * gscale;
           v[j] = gg;
-          lo[j] = lo_of(gg);
+          lo[j] = tf32_lo(gg);
         }
         tmem_st16(tS + (uint32_t)(part * 16), v);
         tmem_st16(tGl + (uint32_t)(part * 16), lo);
@@ -466,7 +464,7 @@ __global__ void __launch_bounds__(64 + 32 * NSW, 1) ce_bwd_dw_tc_kernel(const __
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idS = make_idesc_tf32_ex(128, CW, 0, 0), id2 = make_idesc_tf32_ex(128, 2 * d, 0, 1), id1 = make_idesc_tf32_ex(128, d, 0, 1);
+      const uint32_t idS = make_idesc_tf32(128, CW, 0, 0), id2 = make_idesc_tf32(128, 2 * d, 0, 1), id1 = make_idesc_tf32(128, d, 0, 1);
       mbar_wait(smem_u32(&w_bar), 0);
       tc_fence_after();
       int pend[2] = {-1, -1};
@@ -548,7 +546,7 @@ __global__ void __launch_bounds__(64 + 32 * NSW, 1) ce_bwd_dw_tc_kernel(const __
           const float gg = p * gscale;
           bsum += gg;
           v[j] = gg;
-          lo[j] = lo_of(gg);
+          lo[j] = tf32_lo(gg);
         }
         tmem_st16(tS + (uint32_t)(part * 16), v);
         tmem_st16(tGl + (uint32_t)(part * 16), lo);
@@ -594,7 +592,7 @@ __global__ void __launch_bounds__(256) lo_copy_kernel(const float* __restrict__ 
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n4) return;
   float4 v = ld4(src + i * 4);
-  st4(lo + i * 4, make_float4(lo_of(v.x), lo_of(v.y), lo_of(v.z), lo_of(v.w)));
+  st4(lo + i * 4, make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)));
 }
 // Hc[r] = h[rows[r]] (r < count), zeros up to the next multiple of 128; plus its TF32 residual
 __global__ void __launch_bounds__(256) gather_split_kernel(const float* __restrict__ h, const int32_t* __restrict__ rows,
@@ -610,21 +608,9 @@ __global__ void __launch_bounds__(256) gather_split_kernel(const float* __restri
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
   if (r < count) v = ld4(h + ((int64_t)rows[r] * d4 + c4) * 4);
   st4(hc + i * 4, v);
-  st4(hcl + i * 4, make_float4(lo_of(v.x), lo_of(v.y), lo_of(v.z), lo_of(v.w)));
+  st4(hcl + i * 4, make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)));
 }
 
-// [rows, d] fp32, box [64 rows x 32 cols]; K-major consumers: 128B swizzle, MN-major consumers: 32-byte-atom variant
-bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int d, bool mn) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)d, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)d * sizeof(float)};
-  cuuint32_t box[2] = {32, (cuuint32_t)CW};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             mn ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 }  // namespace
 
 bool rbm_ce_tc_supported(int V1, int d, const void* h, const void* w) {
@@ -653,7 +639,7 @@ int rbm_ce_tc_fwd(const float* h, const int32_t* rows, const int64_t* tgt, const
   const int64_t nw4 = (int64_t)V1 * d / 4;
   lo_copy_kernel<<<(unsigned)rbm_cdiv(nw4, 256), 256, 0, st>>>(w, w_lo, nw4);
   CUtensorMap mW, mWl;
-  if (!encode_map(&mW, w, V1, d, false) || !encode_map(&mWl, w_lo, V1, d, false)) {
+  if (!encode_f32_rows(&mW, w, V1, d, d, CW, false) || !encode_f32_rows(&mWl, w_lo, V1, d, d, CW, false)) {
     rbm_set_error("rbm_ce_fwd(tcgen05): cuTensorMapEncodeTiled failed");
     return -1;
   }
@@ -687,9 +673,11 @@ int rbm_ce_tc_bwd(const float* h, const int32_t* rows, const int64_t* tgt, const
   lo_copy_kernel<<<(unsigned)rbm_cdiv(nw4, 256), 256, 0, st>>>(w, w_lo, nw4);
   gather_split_kernel<<<(unsigned)rbm_cdiv(cap128 * (d / 4), 256), 256, 0, st>>>(h, rows, count, hc, hcl, cap128, d / 4);
   CUtensorMap mW, mWl, mWm, mWml, mH, mHl, mHm, mHml;
-  if (!encode_map(&mW, w, V1, d, false) || !encode_map(&mWl, w_lo, V1, d, false) || !encode_map(&mWm, w, V1, d, true) ||
-      !encode_map(&mWml, w_lo, V1, d, true) || !encode_map(&mH, hc, cap128, d, false) || !encode_map(&mHl, hcl, cap128, d, false) ||
-      !encode_map(&mHm, hc, cap128, d, true) || !encode_map(&mHml, hcl, cap128, d, true)) {
+  // 64-row chunks of [rows, d]: K-major maps for the score products, MN-major ones for the accumulations
+  if (!encode_f32_rows(&mW, w, V1, d, d, CW, false) || !encode_f32_rows(&mWl, w_lo, V1, d, d, CW, false) ||
+      !encode_f32_rows(&mWm, w, V1, d, d, CW, true) || !encode_f32_rows(&mWml, w_lo, V1, d, d, CW, true) ||
+      !encode_f32_rows(&mH, hc, cap128, d, d, CW, false) || !encode_f32_rows(&mHl, hcl, cap128, d, d, CW, false) ||
+      !encode_f32_rows(&mHm, hc, cap128, d, d, CW, true) || !encode_f32_rows(&mHml, hcl, cap128, d, d, CW, true)) {
     rbm_set_error("rbm_ce_bwd(tcgen05): cuTensorMapEncodeTiled failed");
     return -1;
   }

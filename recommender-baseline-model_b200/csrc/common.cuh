@@ -164,6 +164,16 @@ __device__ __forceinline__ float warp_max(float v) {
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 
+// TF32 residual of the 3xTF32 products: x minus x with its low 13 mantissa bits cleared (the part the tensor core drops)
+__device__ __forceinline__ float tf32_lo(float x) { return x - __uint_as_float(__float_as_uint(x) & 0xffffe000u); }
+// dst = tf32_lo(src), elementwise over n4 float4 (layout-agnostic: a swizzled tile stays swizzled)
+__device__ __forceinline__ void split_lo(const float* src, float* dst, int n4, int tid, int nthr) {
+  for (int i = tid; i < n4; i += nthr) {
+    const float4 v = ld4(src + i * 4);
+    st4(dst + i * 4, make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)));
+  }
+}
+
 // 0.5*x*(1+tanh(u)), u = sqrt(2/pi)*(x+0.044715*x^3)   NN/models/bert_modules/utils/gelu.py:12
 // evaluated through the identity 0.5*(1+tanh(u)) = sigmoid(2u) = 1/(1+2^(-2u*log2e)): no 1+tanh cancellation for negative x
 // (a few ulp relative error everywhere) and ~8 instructions (ex2 + rcp) instead of libdevice tanhf's ~25 with branches

@@ -216,8 +216,7 @@ extern "C" int rbm_embed_bwd_rows(const int64_t* tok, const int32_t* rows, const
   const size_t smem = (size_t)L * d * sizeof(float);
   static size_t smem_set = 0;
   if (smem > 48 * 1024 && smem > smem_set) {
-    cudaError_t e = cudaFuncSetAttribute(embed_dpos_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    RBM_REQUIRE(e == cudaSuccess, "rbm_embed_bwd_rows: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    if (!set_smem(embed_dpos_partial_kernel, smem, "rbm_embed_bwd_rows")) return -1;
     smem_set = smem;
   }
   const int threads = d4 <= 32 ? 32 : (d4 <= 64 ? 64 : 128);

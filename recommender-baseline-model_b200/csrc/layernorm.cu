@@ -256,8 +256,7 @@ extern "C" int rbm_layernorm_bwd_fanout(const float* x, const float* gamma, cons
 #define LN_BWD(NV, GW)                                                                                              \
   do {                                                                                                              \
     size_t smem = (size_t)(32 * LN_BWD_WARPS / GW) * 2 * d * sizeof(float);                                         \
-    if (smem > 48 * 1024)                                                                                           \
-      cudaFuncSetAttribute(layernorm_bwd_kernel<NV, GW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);   \
+    if (smem > 48 * 1024 && !set_smem(layernorm_bwd_kernel<NV, GW>, smem, "rbm_layernorm_bwd")) return -1;         \
     layernorm_bwd_kernel<NV, GW><<<nblk, 32 * LN_BWD_WARPS, smem, st>>>(x, gamma, dy, dy2, dres, stats, dx, (float*)ws,  \
                                                                         rows, d, rpb, eps, flavour);                \
   } while (0)

@@ -20,7 +20,7 @@ __device__ __forceinline__ int swz(int r) { return (((r & 3) << 1) | ((r >> 2) &
 // O(2^-22 |x|), the same order as the lo*lo term 3xTF32 neglects anyway.
 __device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
   hi = __float_as_uint(x) & 0xffffe000u;
-  lo = __float_as_uint(x - __uint_as_float(hi));
+  lo = __float_as_uint(tf32_lo(x));
 }
 __device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
   asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"

@@ -512,7 +512,7 @@ extern "C" int rbm_ce_fwd(const float* h, const int32_t* rows, const int64_t* tg
   int warps = ce_warps(d, false);
   int nblk = (int)rbm_cdiv(cap, 16 * warps);
   size_t smem = ce_smem(d, warps, false);
-  cudaFuncSetAttribute(ce_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (!set_smem(ce_fwd_kernel, smem, "rbm_ce_fwd")) return -1;
   CeArgs a{};
   a.h = h; a.rows = rows; a.tgt = tgt; a.count = count; a.w = w; a.bias = bias; a.lse_out = lse; a.partial = (float*)ws; a.V1 = V1; a.d = d;
   ce_fwd_kernel<<<nblk, 32 * warps, smem, st>>>(a);
@@ -567,9 +567,9 @@ extern "C" int rbm_ce_bwd(const float* h, const int32_t* rows, const int64_t* tg
   dim3 gdw((unsigned)rbm_cdiv(V1, 16 * warps), S);
 #define CE_BWD(DT)                                                                                          \
   do {                                                                                                      \
-    cudaFuncSetAttribute(ce_bwd_dh_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
+    if (!set_smem(ce_bwd_dh_kernel<DT>, smem, "rbm_ce_bwd(dh)")) return -1;                               \
     ce_bwd_dh_kernel<DT><<<nblk, 32 * warps, smem, st>>>(a);                                                \
-    cudaFuncSetAttribute(ce_bwd_dw_kernel<DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);     \
+    if (!set_smem(ce_bwd_dw_kernel<DT>, smem, "rbm_ce_bwd(dw)")) return -1;                               \
     ce_bwd_dw_kernel<DT><<<gdw, 32 * warps, smem, st>>>(a);                                                 \
   } while (0)
   if (d <= 32) CE_BWD(4);

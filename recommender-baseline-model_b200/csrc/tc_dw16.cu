@@ -249,11 +249,7 @@ int rbm_dw16_launch(const float* dpre, int64_t lda, const float* x, int64_t ldb,
   const size_t smem = 2 * (size_t)(4 * BLK + 2 * (a.KT / 64) * BLK) + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(dw16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * (4 * BLK + 8 * BLK) + 1024);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_linear_bwd_weight(dw16): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(dw16_kernel, 2 * (4 * BLK + 8 * BLK) + 1024, "rbm_linear_bwd_weight(dw16)")) return -1;
     attr_set = true;
   }
   dim3 grid((unsigned)((N / 128) * a.tiles_k), (unsigned)rbm_dw16_splits(M, N, K));

@@ -48,18 +48,6 @@ struct TcParams {
 // =====================================================================================================
 constexpr int STG_LD = 32;  // staging tile: 32x32 floats per warp, 16-byte chunks XOR-swizzled by (row & 7): conflict-free both ways
 
-// dst = src - trunc_tf32(src), elementwise over n4 float4 (layout-agnostic: the swizzle is preserved)
-__device__ __forceinline__ void split_lo(const float* src, float* dst, int n4, int tid, int nthr) {
-  for (int i = tid; i < n4; i += nthr) {
-    float4 v = ld4(src + i * 4), o;
-    o.x = v.x - __uint_as_float(__float_as_uint(v.x) & 0xffffe000u);
-    o.y = v.y - __uint_as_float(__float_as_uint(v.y) & 0xffffe000u);
-    o.z = v.z - __uint_as_float(__float_as_uint(v.z) & 0xffffe000u);
-    o.w = v.w - __uint_as_float(__float_as_uint(v.w) & 0xffffe000u);
-    st4(dst + i * 4, o);
-  }
-}
-
 constexpr int EPI_WARPS = 8;
 // ACT: 0 none, 1 ReLU, 2 tanh-GELU, 3 none but the pre-activation is stored; DROPA / DROPB: the Philox dropout sites.  The
 // variant is a compile-time property so that the unrolled epilogue rows are straight-line code (uniform runtime branches
@@ -123,7 +111,7 @@ __global__ void __launch_bounds__(128 + 32 * EPI_WARPS, 1) tc_linear_persistent_
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idesc = make_idesc_tf32(BM, BN);
+      const uint32_t idesc = make_idesc_tf32(BM, BN, 0, 0);
       mbar_wait(smem_u32(&bsplit_bar), 0);
       tc_fence_after();
       int g = 0, it = 0;
@@ -361,8 +349,8 @@ __global__ void __launch_bounds__(192, 1) tc_dw_kernel(const __grid_constant__ C
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idesc = make_idesc_tf32_ex(BM, p.wide ? NB : p.K, 1, 1);
-      const uint32_t idesc_b = make_idesc_tf32_ex(BM, DW_BIAS_N, 1, 1);
+      const uint32_t idesc = make_idesc_tf32(BM, p.wide ? NB : p.K, 1, 1);
+      const uint32_t idesc_b = make_idesc_tf32(BM, DW_BIAS_N, 1, 1);
       for (int g = 0; g < nst; ++g) {
         const int s = g % p.nstage;
         mbar_wait(smem_u32(&full_bar[s]), (g / p.nstage) & 1);
@@ -456,20 +444,6 @@ __global__ void __launch_bounds__(192, 1) tc_dw_kernel(const __grid_constant__ C
   }
 }
 
-// ------------------------------------------------------------------------------------------------ host side
-// 2-D fp32 tensor [rows, cols] with row stride ld (elements); box = [box_rows, 32 cols], 128-byte swizzle
-bool encode_map(CUtensorMap* map, const float* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(float)};
-  cuuint32_t box[2] = {(cuuint32_t)BKE, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS;
-}
-
 }  // namespace
 
 static bool weight_fits(int N, int K, int* nstage_out) {
@@ -541,7 +515,7 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
   }
   const int BN = N / NG;
   CUtensorMap mapA, mapB;
-  if (!encode_map(&mapA, a, M, K, lda, BM) || !encode_map(&mapB, b, N, K, ldb, BN)) {
+  if (!encode_f32_rows(&mapA, a, M, K, lda, BM, false) || !encode_f32_rows(&mapB, b, N, K, ldb, BN, false)) {
     rbm_set_error("rbm_linear(tcgen05): cuTensorMapEncodeTiled failed (M=%lld N=%d K=%d lda=%lld)", (long long)M, N, K, (long long)lda);
     return -1;
   }
@@ -551,18 +525,13 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
   p.thrA = ep.thrA; p.thrB = ep.thrB; p.invA = ep.invA; p.invB = ep.invB; p.siteA = ep.siteA; p.siteB = ep.siteB; p.seed = ep.seed;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaSuccess;
     // every (activation, dropout A, dropout B) variant of the persistent kernel
-#define RBM_TC_ATTR(A, DA, DB) \
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc_linear_persistent_kernel<A, DA, DB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
-#define RBM_TC_ATTR4(A) RBM_TC_ATTR(A, false, false) RBM_TC_ATTR(A, true, false) RBM_TC_ATTR(A, false, true) RBM_TC_ATTR(A, true, true)
-    RBM_TC_ATTR4(0) RBM_TC_ATTR4(1) RBM_TC_ATTR4(2) RBM_TC_ATTR4(3)
+#define RBM_TC_ATTR(A, DA, DB) set_smem(tc_linear_persistent_kernel<A, DA, DB>, 231424, "rbm_linear(tcgen05)")
+#define RBM_TC_ATTR4(A) RBM_TC_ATTR(A, false, false) && RBM_TC_ATTR(A, true, false) && RBM_TC_ATTR(A, false, true) && RBM_TC_ATTR(A, true, true)
+    const bool ok = RBM_TC_ATTR4(0) && RBM_TC_ATTR4(1) && RBM_TC_ATTR4(2) && RBM_TC_ATTR4(3);
 #undef RBM_TC_ATTR4
 #undef RBM_TC_ATTR
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_linear(tcgen05): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!ok) return -1;
     attr_set = true;
   }
   p.nstage = ns;
@@ -597,16 +566,6 @@ static int launch_single(const float* a, int64_t lda, const float* b, int64_t ld
 
 // ------------------------------------------------------------------------------------------ weight gradient launch
 namespace {
-bool encode_map_mn(CUtensorMap* map, const float* base, int64_t rows, int64_t cols, int64_t ld) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)ld * sizeof(float)};
-  cuuint32_t box[2] = {32, (cuuint32_t)DW_TOK};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 int dw_stages(int N, int K, int* mtiles_out) {
   int mtiles = (N + BM - 1) / BM;
   size_t stage = (size_t)2 * ((size_t)N / 32 + K / 32) * DW_BLK + DW_BLK;  // + the all-ones block
@@ -643,7 +602,7 @@ bool rbm_tc_dw_supported(int64_t M, int N, int K, int64_t lda, int64_t ldb, cons
 int rbm_tc_dw_launch(const float* dpre, int64_t lda, const float* x, int64_t ldb, float* part, float* part_b, int64_t M, int N, int K,
                      cudaStream_t st) {
   CUtensorMap mapA, mapB;
-  if (!encode_map_mn(&mapA, dpre, M, N, lda) || !encode_map_mn(&mapB, x, M, K, ldb)) {
+  if (!encode_f32_rows(&mapA, dpre, M, N, lda, DW_TOK, true) || !encode_f32_rows(&mapB, x, M, K, ldb, DW_TOK, true)) {
     rbm_set_error("rbm_linear_bwd_weight(tcgen05): cuTensorMapEncodeTiled failed");
     return -1;
   }
@@ -660,11 +619,7 @@ int rbm_tc_dw_launch(const float* dpre, int64_t lda, const float* x, int64_t ldb
   size_t smem = (size_t)p.nstage * (2 * ((size_t)p.nblkA + p.nblkB) + 1) * DW_BLK + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tc_dw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_linear_bwd_weight(tcgen05): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(tc_dw_kernel, 231424, "rbm_linear_bwd_weight(tcgen05)")) return -1;
     attr_set = true;
   }
   tc_dw_kernel<<<S, 192, smem, st>>>(mapA, mapB, p);

@@ -249,17 +249,6 @@ __global__ void __launch_bounds__(THREADS, 1) gemm16_kernel(const __grid_constan
   }
 }
 
-bool encode_a32(CUtensorMap* map, const void* base, int64_t rows, int cols, int64_t ld) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) return false;
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstride[1] = {(cuuint64_t)ld * 4};
-  cuuint32_t box[2] = {32, 128};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace
 
 bool rbm_gemm16_supported(int64_t M, int N, int K, int64_t lda, const void* a, const void* b) {
@@ -283,7 +272,7 @@ int rbm_gemm16_launch(const float* a, int64_t lda, const float* b, int64_t M, in
   scales_launch(bits, scales, st);
   split_w_launch(b, scales + 1, (uint2*)b_hi, (uint2*)b_lo, (int64_t)N * K / 4, st);
   CUtensorMap mA, mBh, mBl;
-  if (!encode_f16_rows(&mBh, b_hi, N, K, 128) || !encode_f16_rows(&mBl, b_lo, N, K, 128) || !encode_a32(&mA, a, M, K, lda)) {
+  if (!encode_f16_rows(&mBh, b_hi, N, K, 128) || !encode_f16_rows(&mBl, b_lo, N, K, 128) || !encode_f32_rows(&mA, a, M, K, lda, 128, false)) {
     rbm_set_error("rbm_linear(gemm16): cuTensorMapEncodeTiled failed");
     return -1;
   }
@@ -294,11 +283,7 @@ int rbm_gemm16_launch(const float* a, int64_t lda, const float* b, int64_t M, in
   const size_t smem = (size_t)NSTG * (STAGE + A32) + STG_BYTES + 1024;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(gemm16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_linear(gemm16): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(gemm16_kernel, smem, "rbm_linear(gemm16)")) return -1;
     attr_set = true;
   }
   const int64_t units = rbm_cdiv(M, 128) * (N / 128);

@@ -1,13 +1,11 @@
 // tc_ptx.cuh -- inline-PTX wrappers for the Blackwell (sm_100a) async/tensor path: mbarrier, TMA (cp.async.bulk.tensor),
 // tcgen05 (alloc/mma/commit/ld/st/fences, kind::tf32 and kind::f16) and UMMA shared-memory / instruction descriptors; plus the
-// host-side lookup of the tensor-map encoder and the fp16 row-tile tensor map.
+// host-side lookup of the tensor-map encoder and the fp32 and fp16 row-tile tensor maps.
 #pragma once
 #include <cuda.h>  // CUtensorMap types only; the encode function is fetched at run time (no libcuda link dependency)
 #include "common.cuh"
 
 namespace rbm_tc {
-
-constexpr int UMMA_K_TF32 = 8;
 
 // cuTensorMapEncodeTiled from the driver, looked up once per process (tc_encode.cu); nullptr when the driver lacks it.  Every call
 // also binds the calling thread to the primary context (rbm_bind_context), which the encode needs.
@@ -94,11 +92,11 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t saddr) {
   d |= (uint64_t)2 << 61;
   return d;
 }
-// cute::UMMA::InstrDescriptor for kind::tf32, fp32 accumulate, both operands K-major
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// cute::UMMA::InstrDescriptor, kind::tf32: D = F32 (bits [4,6) = 1), A = B = TF32 (format 2), bit 15: A MN-major, bit 16: B MN-major
+__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N, int a_mn, int b_mn) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) |
+         ((uint32_t)(M >> 4) << 24);
 }
-
 
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -126,34 +124,6 @@ __device__ __forceinline__ bool elect_one() {
       "@p mov.s32 %0, 1;\n\t}"
       : "+r"(pred));
   return pred != 0;
-}
-// Warp-converged issue: every lane of the (fully active) warp executes the call with identical operands and one
-// elected lane issues the instruction.  Unlike a call under `if (lane == 0)`, the compiler does not have to wrap the
-// single-thread instruction in a per-active-lane loop (ELECT / PLOP3 / BRA.U.ANY around every UTCHMMA).
-__device__ __forceinline__ void umma_tf32_ts_w(uint32_t d_tmem, uint32_t a_tmem, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p, e;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "elect.sync _|e, 0xffffffff;\n\t"
-      "@e tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_tf32_w(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p, e;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "elect.sync _|e, 0xffffffff;\n\t"
-      "@e tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_w(uint32_t bar) {
-  asm volatile(
-      "{\n\t.reg .pred e;\n\t"
-      "elect.sync _|e, 0xffffffff;\n\t"
-      "@e tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar)
-      : "memory");
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   uint32_t r[16];
@@ -209,11 +179,6 @@ __device__ __forceinline__ uint64_t make_sw128_desc_mn(uint32_t saddr, uint32_t 
   d |= (uint64_t)1 << 61;
   return d;
 }
-// instruction descriptor with explicit majors (bit 15: A MN-major, bit 16: B MN-major)
-__host__ __device__ constexpr uint32_t make_idesc_tf32_ex(int M, int N, int a_mn, int b_mn) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) |
-         ((uint32_t)(M >> 4) << 24);
-}
 
 // ------------------------------------------------------------------------------------------------ kind::f16
 // D[tmem] (+)= A[smem desc] . B[smem desc], fp16 operands, fp32 accumulate
@@ -258,6 +223,9 @@ __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&v)[8])
 }
 
 // ------------------------------------------------------------------------------------------------ host side
+// [rows, cols] fp32 with row stride ld (elements), box [box_rows x 32 columns]: 128-byte swizzle for K-major consumers, its
+// 32-byte-atom variant for MN-major ones (mn_major); rows beyond the tensor read as zeros (tc_encode.cu)
+bool encode_f32_rows(CUtensorMap* map, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows, bool mn_major);
 // [rows, cols] fp16 row-major, box [box_rows x 64 columns], 128-byte swizzle; rows beyond the tensor read as zeros (tc_encode.cu)
 bool encode_f16_rows(CUtensorMap* map, const void* base, int64_t rows, int cols, int box_rows);
 

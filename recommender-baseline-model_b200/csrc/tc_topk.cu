@@ -114,7 +114,7 @@ __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      const uint32_t idesc = F16 ? make_idesc_f16(BM, BN, 0, 0) : make_idesc_tf32(BM, BN);
+      const uint32_t idesc = F16 ? make_idesc_f16(BM, BN, 0, 0) : make_idesc_tf32(BM, BN, 0, 0);
       int g = 0, it = 0, un = 0;
       for (int u = blockIdx.x; u < n_units; u += gridDim.x, ++un) {
         const int sp = u % p.S;
@@ -504,12 +504,8 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
   p.tmem_cols = cols;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(tc_topk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc_topk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 231424);
-    if (e != cudaSuccess) {
-      rbm_set_error("rbm_score_topk(tcgen05): cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      return (int)e;
-    }
+    if (!set_smem(tc_topk_kernel<false>, 231424, "rbm_score_topk(tcgen05)") || !set_smem(tc_topk_kernel<true>, 231424, "rbm_score_topk(tcgen05)"))
+      return -1;
     attr_set = true;
   }
   size_t smem = a_bytes + (size_t)ns * stage + 1024;

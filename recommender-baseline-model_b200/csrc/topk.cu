@@ -300,7 +300,7 @@ extern "C" int rbm_score_topk(const float* f, int64_t ldf, const float* table, c
   int S = topk_splits(U, n_items);
   int64_t tps = rbm_cdiv(rbm_cdiv(n_items, T), S);
   size_t smem = sizeof(float) * ((size_t)d * LDT + KC * LDT + T * LDT);
-  cudaFuncSetAttribute(score_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (!set_smem(score_topk_kernel, smem, "rbm_score_topk")) return -1;
   int64_t* part_i = (int64_t*)ws;
   float* part_s = (float*)(part_i + (size_t)S * U * k);
   dim3 grid((unsigned)rbm_cdiv(U, T), S);
@@ -322,7 +322,7 @@ int rbm_simt_topk_listed(const float* f, int64_t ldf, const float* table, const 
                          const int32_t* ucount, void* part_ws, int S, cudaStream_t st) {
   int64_t tps = rbm_cdiv(rbm_cdiv(v_end - v_begin, T), S);
   size_t smem = sizeof(float) * ((size_t)d * LDT + KC * LDT + T * LDT);
-  cudaFuncSetAttribute(score_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (!set_smem(score_topk_kernel, smem, "rbm_score_topk(exact re-scan)")) return -1;
   int64_t* part_i = (int64_t*)part_ws;
   float* part_s = (float*)(part_i + (size_t)S * U * k);
   dim3 grid((unsigned)rbm_cdiv(U, T), S);
