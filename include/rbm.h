@@ -276,6 +276,16 @@ size_t rbm_score_topk_ws_bytes_d(int64_t U, int64_t n_items, int d, int k);
 int rbm_score_topk(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin,
                    int64_t v_end, int64_t id_offset, float* top_scores, int64_t* top_ids, int64_t U, int d,
                    int k, void* ws, size_t ws_bytes, rbm_stream_t stream);
+/* rbm_score_topk over the catalogue minus each user's already-seen items (the "full sort" protocol of full-ranking
+ * evaluation: the reference's argsort over all items, NN/trainers/utils.py:36-38, after the history is removed).  Row u of
+ * excl [U, n_excl] (row stride ld_excl, int64) holds the ids user u must not be ranked, in output-id space (v + id_offset,
+ * the ids this call returns), sorted ascending; duplicates are allowed and ids outside [v_begin, v_end) + id_offset never
+ * match (0 / -1 padding and other shards' ids are harmless).  Result: the canonical top-k of the remaining items (same
+ * order and scores as rbm_score_topk; fewer than k remaining -> trailing (-inf, -1)).  excl == NULL or n_excl == 0 gives
+ * results bit-identical to rbm_score_topk.  Same workspace query. */
+int rbm_score_topk_excl(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin, int64_t v_end,
+                        int64_t id_offset, const int64_t* excl, int64_t ld_excl, int n_excl, float* top_scores,
+                        int64_t* top_ids, int64_t U, int d, int k, void* ws, size_t ws_bytes, rbm_stream_t stream);
 /* top-k of materialised scores [U,C] (ld = row stride), same order rule; id = column + id_offset.
  * replaces (-scores).argsort(dim=1)[:, :k]  NN/trainers/utils.py:36-38 */
 int rbm_topk_rows(const float* scores, int64_t ld, float* top_scores, int64_t* top_ids, int64_t U, int64_t C,

@@ -26,6 +26,7 @@
 //     score is the sequential FMA over the hidden dimension (the arithmetic of stage 2 and of the scan kernel).
 #include <cuda_fp16.h>
 #include <stdlib.h>
+#include <type_traits>
 #include "common.cuh"
 #include "tc_ptx.cuh"
 #include "split16.cuh"
@@ -49,12 +50,32 @@ struct TopkParams {
   int nst;  // 128-row user sub-tiles per unit: 2 (d <= 64: 256 users share every streamed item tile) or 1
   uint32_t tmem_cols;
 };
+// the exclusion path's parameters extend the struct instead of growing it: the kernels without exclusion keep their code
+struct TopkExclParams : TopkParams {
+  const int64_t* excl;  // row u = user u's excluded output ids, ascending (row stride ld_excl, n_excl entries)
+  int64_t ld_excl;
+  int n_excl;
+};
+
+// first index of the ascending row ex[0 .. n) whose id is >= key (n when none)
+__device__ __forceinline__ int excl_lower_bound(const int64_t* __restrict__ ex, int n, int64_t key) {
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (ex[mid] < key) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
 
 // F16: operands are the range-scaled fp16 copies (64 elements per 128-byte row, K = 16 per instruction, kind::f16);
-// otherwise the fp32 data itself (32 elements per row, K = 8, kind::tf32)
-template <bool F16>
+// otherwise the fp32 data itself (32 elements per row, K = 8, kind::tf32).
+// EX: items of the user's exclusion row never enter a candidate list.  The filter sits on the rare insertion path only: a
+// thread meets its item ids in ascending order within a unit, so a cursor into the sorted row (next excluded id in a
+// register) advances monotonically and reads each entry at most once per unit.
+template <bool F16, bool EX>
 __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                                                                   const TopkParams p) {
+                                                                   const std::conditional_t<EX, TopkExclParams, TopkParams> p) {
   constexpr int BKE = F16 ? 64 : 32;      // elements per 128-byte K block
   constexpr int ESZ = F16 ? 2 : 4;
   extern __shared__ uint8_t smem_raw[];
@@ -168,6 +189,19 @@ __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_
       }
       const int64_t tb = (int64_t)sp * p.tiles_per_split;
       const int64_t te = tb + p.tiles_per_split < n_tiles ? tb + p.tiles_per_split : n_tiles;
+      // EX cursor: ex_row[ex_pos] = ex_next is the first excluded id >= every id this thread has offered so far in the unit
+      // (rows past U read nothing: n = 0, next = +inf)
+      const int64_t* ex_row = nullptr;
+      int ex_n = 0, ex_pos = 0;
+      int64_t ex_next = INT64_MAX;
+      if constexpr (EX) {
+        if (user < p.U) {
+          ex_row = p.excl + user * p.ld_excl;
+          ex_n = p.n_excl;
+          ex_pos = excl_lower_bound(ex_row, ex_n, p.v_begin + tb * BN + p.row_base + p.id_offset);
+          ex_next = ex_pos < ex_n ? ex_row[ex_pos] : INT64_MAX;
+        }
+      }
       for (int64_t t = tb; t < te; ++t, ++it) {
         const int buf = it & 1;
         mbar_wait(smem_u32(&tfull[buf]), (it >> 1) & 1);
@@ -216,6 +250,11 @@ __global__ void __launch_bounds__(64 + 32 * EPI, 1) tc_topk_kernel(const __grid_
               const float x = loc[j];
               if (x > ls[KC - 1]) {
                 const int id = (int)(r0 + j + p.row_base);
+                if constexpr (EX) {
+                  const int64_t key = (int64_t)id + p.id_offset;
+                  while (ex_next < key) ex_next = ++ex_pos < ex_n ? ex_row[ex_pos] : INT64_MAX;
+                  if (ex_next == key) continue;
+                }
                 bool placed = false;
 #pragma unroll
                 for (int tt = KC - 1; tt > 0; --tt) {
@@ -449,7 +488,8 @@ bool rbm_tc_topk_supported(int64_t U, int64_t n_items, int d, int k, int64_t ldf
 }
 
 int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin, int64_t v_end,
-                       int64_t id_offset, float* top_scores, int64_t* top_ids, int64_t U, int d, int k, void* ws, cudaStream_t st) {
+                       int64_t id_offset, const int64_t* excl, int64_t ld_excl, int n_excl, float* top_scores, int64_t* top_ids, int64_t U,
+                       int d, int k, void* ws, cudaStream_t st) {
   const int BN = pick_bn(d);
   const int64_t n_items = v_end - v_begin;
   const bool f16 = use_f16(d);
@@ -484,6 +524,7 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
   }
   TopkParams p{};
   p.bias = bias; p.scales = scales; p.U = U; p.v_begin = v_begin; p.v_end = v_end; p.id_offset = id_offset; p.d = d; p.BN = BN;
+  const bool ex = excl != nullptr && n_excl > 0;
   p.S = rbm_tc_topk_splits(U, n_items, d);
   p.nst = pick_nst(d);
   p.n_utiles = (int)rbm_cdiv(U, (int64_t)BM * p.nst);
@@ -504,7 +545,8 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
   p.tmem_cols = cols;
   static bool attr_set = false;
   if (!attr_set) {
-    if (!set_smem(tc_topk_kernel<false>, 231424, "rbm_score_topk(tcgen05)") || !set_smem(tc_topk_kernel<true>, 231424, "rbm_score_topk(tcgen05)"))
+    if (!set_smem(tc_topk_kernel<false, false>, 231424, "rbm_score_topk(tcgen05)") || !set_smem(tc_topk_kernel<true, false>, 231424, "rbm_score_topk(tcgen05)") ||
+        !set_smem(tc_topk_kernel<false, true>, 231424, "rbm_score_topk(tcgen05)") || !set_smem(tc_topk_kernel<true, true>, 231424, "rbm_score_topk(tcgen05)"))
       return -1;
     attr_set = true;
   }
@@ -518,9 +560,11 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
     ph.v_begin = 0;
     ph.v_end = n_items;
     ph.row_base = v_begin;
-    tc_topk_kernel<true><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, ph);
+    if (ex) tc_topk_kernel<true, true><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, TopkExclParams{ph, excl, ld_excl, n_excl});
+    else tc_topk_kernel<true, false><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, ph);
   } else {
-    tc_topk_kernel<false><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, p);
+    if (ex) tc_topk_kernel<false, true><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, TopkExclParams{p, excl, ld_excl, n_excl});
+    else tc_topk_kernel<false, false><<<grid, 64 + 32 * EPI, smem, st>>>(mapA, mapB, p);
   }
   RBM_LAUNCH_CHECK("rbm_score_topk(tcgen05)");
   // 2^-10 (two rounded fp16 operands) resp. 2^-9 (two truncated TF32 operands) per product, plus the fp32 accumulation slack
@@ -532,7 +576,9 @@ int rbm_tc_topk_launch(const float* f, int64_t ldf, const float* table, const fl
                                                                                    id_offset, top_scores, top_ids, U, d, k, bits, eps_mul,
                                                                                    f16 ? scales : nullptr, flag_list, flag_count);
   RBM_LAUNCH_CHECK("rbm_score_topk(rescore)");
-  // stage 3: users whose answer the certificate does not cover are re-ranked by the exact fp32 scan (grid exits when none)
-  return rbm_simt_topk_listed(f, ldf, table, bias, v_begin, v_end, id_offset, top_scores, top_ids, U, d, k, flag_list, flag_count, fb_ws,
-                              rbm_tc_topk_fb_splits(U, n_items, k), st);
+  // stage 3: users whose answer the certificate does not cover are re-ranked by the exact fp32 scan (grid exits when none).
+  // Stage 2 needs no exclusion filter: the lists hold non-excluded items only, and an excluded item is no candidate of the
+  // certificate either (every non-excluded item a list dropped still has approximate score <= tau)
+  return rbm_simt_topk_listed(f, ldf, table, bias, v_begin, v_end, id_offset, ex ? excl : nullptr, ld_excl, ex ? n_excl : 0, top_scores, top_ids,
+                              U, d, k, flag_list, flag_count, fb_ws, rbm_tc_topk_fb_splits(U, n_items, k), st);
 }

@@ -53,6 +53,33 @@ __device__ __forceinline__ void list_offer(Entry& mine, float s, int64_t id, boo
   }
 }
 
+// lane's candidate id is in the ascending row ex[0 .. n) (binary search; only asked of lanes that would enter the list)
+__device__ __forceinline__ bool excluded(const int64_t* __restrict__ ex, int n, int64_t id) {
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (ex[mid] < id) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo < n && ex[lo] == id;
+}
+
+// list_offer for a user with an exclusion row (ex, n): the filter runs after the cheap compare, on the rare survivors only
+__device__ __forceinline__ void list_offer_excl(Entry& mine, float s, int64_t id, bool valid, int k, int lane, const int64_t* ex, int n) {
+  float ts = __shfl_sync(0xffffffffu, mine.s, k - 1);
+  int64_t tid = __shfl_sync(0xffffffffu, mine.id, k - 1);
+  bool pass = valid && better(s, id, ts, tid);
+  if (pass) pass = !excluded(ex, n, id);
+  unsigned m = __ballot_sync(0xffffffffu, pass);
+  while (m) {
+    int src = __ffs(m) - 1;
+    m &= m - 1;
+    float cs = __shfl_sync(0xffffffffu, s, src);
+    int64_t cid = __shfl_sync(0xffffffffu, id, src);
+    list_insert(mine, cs, cid, k, lane);
+  }
+}
+
 __device__ __forceinline__ void list_store(const Entry& mine, float* out_s, int64_t* out_i, int64_t u, int k, int lane) {
   if (lane < k) {
     out_s[u * k + lane] = mine.id == ID_NONE ? -INFINITY : mine.s;
@@ -61,11 +88,14 @@ __device__ __forceinline__ void list_store(const Entry& mine, float* out_s, int6
 }
 
 // -------------------------------------------------------------------------------- fused scoring + top-k
+// EX: row u of excl (stride ld_excl, n_excl ascending output ids) lists what user u must not be offered
+template <bool EX>
 __global__ void __launch_bounds__(256) score_topk_kernel(const float* __restrict__ f, int64_t ldf, const float* __restrict__ table,
                                                          const float* __restrict__ bias, int64_t v_begin, int64_t v_end, int64_t id_offset,
                                                          float* __restrict__ out_s, int64_t* __restrict__ out_i, int64_t U, int d, int k,
                                                          int64_t tiles_per_split, const int32_t* __restrict__ ulist,
-                                                         const int32_t* __restrict__ ucount) {
+                                                         const int32_t* __restrict__ ucount, const int64_t* __restrict__ excl, int64_t ld_excl,
+                                                         int n_excl) {
   // listed mode (ulist != null): row slot j of the launch is user ulist[j], j < *ucount (device-side count); results go
   // to slot j of the partial lists (stride U)
   const int64_t U_eff = ulist ? (int64_t)*ucount : U;
@@ -94,6 +124,14 @@ __global__ void __launch_bounds__(256) score_topk_kernel(const float* __restrict
   for (int q = 0; q < 8; ++q) {
     lists[q].s = -INFINITY;
     lists[q].id = ID_NONE;
+  }
+  int ex_user[8];  // EX: the user (not the slot) of list q; -1 past the last user
+  if (EX) {
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      const int64_t slot = u0 + warp * 8 + q;
+      ex_user[q] = slot < U_eff ? (ulist ? ulist[slot] : (int)slot) : -1;
+    }
   }
   const int64_t t_begin = (int64_t)blockIdx.y * tiles_per_split;
   const int64_t n_tiles = (v_end - v_begin + T - 1) / T;
@@ -149,7 +187,8 @@ __global__ void __launch_bounds__(256) score_topk_kernel(const float* __restrict
       for (int hlf = 0; hlf < 2; ++hlf) {
         int c = lane + 32 * hlf;
         int64_t v = v0 + c;
-        list_offer(lists[q], row[c], v + id_offset, v < v_end, k, lane);
+        if (EX) list_offer_excl(lists[q], row[c], v + id_offset, v < v_end, k, lane, excl + (int64_t)ex_user[q] * ld_excl, ex_user[q] < 0 ? 0 : n_excl);
+        else list_offer(lists[q], row[c], v + id_offset, v < v_end, k, lane);
       }
     }
   }
@@ -283,10 +322,36 @@ extern "C" size_t rbm_score_topk_ws_bytes(int64_t U, int64_t n_items, int k) {
   return best;
 }
 
+static size_t simt_smem(int d) { return sizeof(float) * ((size_t)d * LDT + KC * LDT + T * LDT); }
+
+// one launch of the fp32 scan kernel: EX instantiation exactly when there is something to exclude
+static void launch_score_topk(dim3 grid, size_t smem, cudaStream_t st, const float* f, int64_t ldf, const float* table, const float* bias,
+                              int64_t v_begin, int64_t v_end, int64_t id_offset, float* out_s, int64_t* out_i, int64_t U, int d, int k,
+                              int64_t tps, const int32_t* ulist, const int32_t* ucount, const int64_t* excl, int64_t ld_excl, int n_excl) {
+  if (excl && n_excl > 0)
+    score_topk_kernel<true><<<grid, 256, smem, st>>>(f, ldf, table, bias, v_begin, v_end, id_offset, out_s, out_i, U, d, k, tps, ulist, ucount,
+                                                     excl, ld_excl, n_excl);
+  else
+    score_topk_kernel<false><<<grid, 256, smem, st>>>(f, ldf, table, bias, v_begin, v_end, id_offset, out_s, out_i, U, d, k, tps, ulist, ucount,
+                                                      nullptr, 0, 0);
+}
+
+static bool set_simt_smem(size_t smem, const char* name) {
+  return set_smem(score_topk_kernel<false>, smem, name) && set_smem(score_topk_kernel<true>, smem, name);
+}
+
 extern "C" int rbm_score_topk(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin, int64_t v_end,
                               int64_t id_offset, float* top_scores, int64_t* top_ids, int64_t U, int d, int k, void* ws,
                               size_t ws_bytes, rbm_stream_t stream) {
+  return rbm_score_topk_excl(f, ldf, table, bias, v_begin, v_end, id_offset, nullptr, 0, 0, top_scores, top_ids, U, d, k, ws, ws_bytes, stream);
+}
+
+extern "C" int rbm_score_topk_excl(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin, int64_t v_end,
+                                   int64_t id_offset, const int64_t* excl, int64_t ld_excl, int n_excl, float* top_scores,
+                                   int64_t* top_ids, int64_t U, int d, int k, void* ws, size_t ws_bytes, rbm_stream_t stream) {
   RBM_REQUIRE(f && table && top_scores && top_ids && ws, "rbm_score_topk: null pointer");
+  RBM_REQUIRE(n_excl >= 0 && (n_excl == 0 || (excl && ld_excl >= n_excl)), "rbm_score_topk_excl: bad exclusion matrix (n_excl=%d, ld_excl=%lld)",
+              n_excl, (long long)ld_excl);
   RBM_REQUIRE(U > 0 && v_begin >= 0 && v_end > v_begin, "rbm_score_topk: empty user or item range");
   RBM_REQUIRE(k >= 1 && k <= 32, "rbm_score_topk: k=%d out of [1,32]", k);
   RBM_REQUIRE(d >= 4 && d % 4 == 0 && d <= 256 && ldf % 4 == 0 && ldf >= d, "rbm_score_topk: unsupported d=%d (need d%%4==0, d<=256)", d);
@@ -296,19 +361,21 @@ extern "C" int rbm_score_topk(const float* f, int64_t ldf, const float* table, c
   int64_t n_items = v_end - v_begin;
   // catalogue-scale path: tcgen05 candidate selection + exact fp32 re-score (tc_topk.cu)
   if (rbm_tc_topk_supported(U, n_items, d, k, ldf, f, table))
-    return rbm_tc_topk_launch(f, ldf, table, bias, v_begin, v_end, id_offset, top_scores, top_ids, U, d, k, ws, st);
+    return rbm_tc_topk_launch(f, ldf, table, bias, v_begin, v_end, id_offset, excl, ld_excl, n_excl, top_scores, top_ids, U, d, k, ws, st);
   int S = topk_splits(U, n_items);
   int64_t tps = rbm_cdiv(rbm_cdiv(n_items, T), S);
-  size_t smem = sizeof(float) * ((size_t)d * LDT + KC * LDT + T * LDT);
-  if (!set_smem(score_topk_kernel, smem, "rbm_score_topk")) return -1;
+  size_t smem = simt_smem(d);
+  if (!set_simt_smem(smem, "rbm_score_topk")) return -1;
   int64_t* part_i = (int64_t*)ws;
   float* part_s = (float*)(part_i + (size_t)S * U * k);
   dim3 grid((unsigned)rbm_cdiv(U, T), S);
   if (S == 1) {
-    score_topk_kernel<<<grid, 256, smem, st>>>(f, ldf, table, bias, v_begin, v_end, id_offset, top_scores, top_ids, U, d, k, tps, nullptr, nullptr);
+    launch_score_topk(grid, smem, st, f, ldf, table, bias, v_begin, v_end, id_offset, top_scores, top_ids, U, d, k, tps, nullptr, nullptr, excl,
+                      ld_excl, n_excl);
     RBM_LAUNCH_CHECK("rbm_score_topk");
   } else {
-    score_topk_kernel<<<grid, 256, smem, st>>>(f, ldf, table, bias, v_begin, v_end, id_offset, part_s, part_i, U, d, k, tps, nullptr, nullptr);
+    launch_score_topk(grid, smem, st, f, ldf, table, bias, v_begin, v_end, id_offset, part_s, part_i, U, d, k, tps, nullptr, nullptr, excl, ld_excl,
+                      n_excl);
     RBM_LAUNCH_CHECK("rbm_score_topk");
     topk_merge_kernel<<<(unsigned)rbm_cdiv(U, 8), 256, 0, st>>>(part_s, part_i, top_scores, top_ids, S, U, k, nullptr, nullptr);
     RBM_LAUNCH_CHECK("rbm_score_topk(merge)");
@@ -318,15 +385,16 @@ extern "C" int rbm_score_topk(const float* f, int64_t ldf, const float* table, c
 
 // exact fp32 scan + top-k of the users ulist[0 .. *ucount) (tc_topk.cu stage 3): partial lists per item split, then merge
 int rbm_simt_topk_listed(const float* f, int64_t ldf, const float* table, const float* bias, int64_t v_begin, int64_t v_end,
-                         int64_t id_offset, float* top_scores, int64_t* top_ids, int64_t U, int d, int k, const int32_t* ulist,
-                         const int32_t* ucount, void* part_ws, int S, cudaStream_t st) {
+                         int64_t id_offset, const int64_t* excl, int64_t ld_excl, int n_excl, float* top_scores, int64_t* top_ids, int64_t U,
+                         int d, int k, const int32_t* ulist, const int32_t* ucount, void* part_ws, int S, cudaStream_t st) {
   int64_t tps = rbm_cdiv(rbm_cdiv(v_end - v_begin, T), S);
-  size_t smem = sizeof(float) * ((size_t)d * LDT + KC * LDT + T * LDT);
-  if (!set_smem(score_topk_kernel, smem, "rbm_score_topk(exact re-scan)")) return -1;
+  size_t smem = simt_smem(d);
+  if (!set_simt_smem(smem, "rbm_score_topk(exact re-scan)")) return -1;
   int64_t* part_i = (int64_t*)part_ws;
   float* part_s = (float*)(part_i + (size_t)S * U * k);
   dim3 grid((unsigned)rbm_cdiv(U, T), S);
-  score_topk_kernel<<<grid, 256, smem, st>>>(f, ldf, table, bias, v_begin, v_end, id_offset, part_s, part_i, U, d, k, tps, ulist, ucount);
+  launch_score_topk(grid, smem, st, f, ldf, table, bias, v_begin, v_end, id_offset, part_s, part_i, U, d, k, tps, ulist, ucount, excl, ld_excl,
+                    n_excl);
   RBM_LAUNCH_CHECK("rbm_score_topk(exact re-scan)");
   topk_merge_kernel<<<(unsigned)rbm_cdiv(U, 8), 256, 0, st>>>(part_s, part_i, top_scores, top_ids, S, U, k, ulist, ucount);
   RBM_LAUNCH_CHECK("rbm_score_topk(exact re-scan merge)");

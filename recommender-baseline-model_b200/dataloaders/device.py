@@ -120,21 +120,47 @@ class DeviceEvalLoader:
     """``DataLoader(BertEvalDataset | SASEvalDataset, shuffle=False)`` (NN/dataloaders/bert.py:44-62,116-142, sas.py:49-62,124-153):
     batches of ``(seq, candidates, labels)`` device tensors in user order; ``mask_token`` = V+1 for BERT4Rec (appended to the
     history before the cut to ``max_len``), -1 for SASRec.  ``history`` is what the reference passes as ``u2seq`` (train for
-    validation; train ++ val for the test split of the 'leave one out' protocol), ``answers`` one held-out item per user."""
+    validation; train ++ val for the test split of the 'leave one out' protocol), ``answers`` one held-out item per user.
 
-    def __init__(self, history, answers, negatives: torch.Tensor, max_len: int, batch_size: int, device, mask_token: int = -1):
+    ``full_catalogue=True`` (full-ranking protocol; ``negatives`` unused): batches of ``(seq [B, L], answers [B],
+    exclude [B, n])`` instead, where row u of ``exclude`` is user u's whole history (not only its last ``max_len`` items), zero-
+    padded to the batch's longest, with the user's own answer removed so that an item the user returns to stays rankable."""
+
+    def __init__(self, history, answers, negatives: torch.Tensor, max_len: int, batch_size: int, device, mask_token: int = -1,
+                 full_catalogue: bool = False):
         self.ptr, self.items = histories_to_csr(history, device)
         self.num_users = self.ptr.numel() - 1
         users = sorted(answers) if isinstance(answers, dict) else range(len(answers))
         ans = [answers[u][0] if isinstance(answers[u], (list, tuple, np.ndarray)) else answers[u] for u in users]
         self.answers = torch.tensor(ans, dtype=torch.int64, device=device)
-        self.negatives = None if negatives is None else negatives.to(device).contiguous()
+        self.full_catalogue = bool(full_catalogue)
+        self.negatives = None if (negatives is None or self.full_catalogue) else negatives.to(device).contiguous()
         self.max_len, self.batch_size, self.mask_token = max_len, batch_size, mask_token
+        # row lengths on the host: the width of a batch's exclusion matrix is known without a device round trip
+        self.lengths = self.ptr.diff().cpu().numpy() if self.full_catalogue else None
 
     def __len__(self):
         return (self.num_users + self.batch_size - 1) // self.batch_size
 
+    def _exclude(self, b0: int, b1: int, answers: torch.Tensor) -> torch.Tensor:
+        """The histories of users [b0, b1) as a zero-padded [b1 - b0, n] matrix (their CSR rows are one contiguous slice)."""
+        n = int(self.lengths[b0:b1].max()) if b1 > b0 else 0
+        dev = self.ptr.device
+        if n == 0:
+            return torch.zeros(b1 - b0, 0, device=dev, dtype=torch.int64)
+        start = self.ptr[b0:b1].unsqueeze(1)
+        col = torch.arange(n, device=dev, dtype=torch.int64).unsqueeze(0)
+        valid = col < (self.ptr[b0 + 1:b1 + 1].unsqueeze(1) - start)
+        ex = torch.where(valid, self.items[(start + col).clamp_max(self.items.numel() - 1)], 0)
+        return ex.masked_fill_(ex == answers.unsqueeze(1), 0)
+
     def __iter__(self):
         for b in range(len(self)):
-            users = torch.arange(b * self.batch_size, min((b + 1) * self.batch_size, self.num_users), device=self.ptr.device)
-            yield ops.eval_batch(self.ptr, self.items, self.answers, self.negatives, users, self.max_len, self.mask_token)
+            b0, b1 = b * self.batch_size, min((b + 1) * self.batch_size, self.num_users)
+            users = torch.arange(b0, b1, device=self.ptr.device)
+            seq, cand, labels = ops.eval_batch(self.ptr, self.items, self.answers, self.negatives, users, self.max_len, self.mask_token)
+            if self.full_catalogue:
+                answers = self.answers[b0:b1]
+                yield seq, answers, self._exclude(b0, b1, answers)
+            else:
+                yield seq, cand, labels

@@ -26,7 +26,9 @@ class AbstractDataloader(metaclass=ABCMeta):
         self.max_len = args.max_len
         self.device = args.device
         self.seed = int(getattr(args, "dataloader_random_seed", 0) or 0)
-        self.test_negative_samples = DeviceNegativeSampler(
+        # full-catalogue evaluation ranks every item the user has not seen: no sampled negatives
+        self.full_catalogue = bool(getattr(args, "full_catalogue_eval", False))
+        self.test_negative_samples = None if self.full_catalogue else DeviceNegativeSampler(
             self.train, self.val, self.test, self.user_count, self.item_count, args.test_negative_sample_size,
             args.test_negative_sampling_seed, self.device, code=args.test_negative_sampler_code).get_negative_samples()
 
@@ -43,13 +45,15 @@ class AbstractDataloader(metaclass=ABCMeta):
 
     def _eval_loader(self, mode):
         """NN/dataloaders/bert.py:44-62, sas.py:49-62: validation scores train histories against the validation item, the test
-        split appends the validation item to the history first."""
+        split appends the validation item to the history first.  ``args.full_catalogue_eval``: batches of (seq, answers,
+        exclude) for ranking the whole catalogue minus that history (see ``DeviceEvalLoader``)."""
         if mode == "val":
             history, answers, bs = self.train, self.val, self.args.val_batch_size
         else:
             history = [list(seq) + [self.val[u][0]] for u, seq in enumerate(self.train)]
             answers, bs = self.test, self.args.test_batch_size
-        return DeviceEvalLoader(history, answers, self.test_negative_samples, self.max_len, bs, self.device, mask_token=self.mask_token)
+        return DeviceEvalLoader(history, answers, self.test_negative_samples, self.max_len, bs, self.device, mask_token=self.mask_token,
+                                full_catalogue=self.full_catalogue)
 
     def get_pytorch_dataloaders(self):
         return self._train_loader(), self._eval_loader("val"), self._eval_loader("test")

@@ -116,16 +116,18 @@ def gather_topk(vals: torch.Tensor, ids: torch.Tensor, group=None) -> Tuple[torc
     return torch.stack(vs), torch.stack(is_)
 
 
-def sharded_full_catalogue_topk(last_hidden: torch.Tensor, table: torch.Tensor, bias, num_items: int, k: int, group=None):
+def sharded_full_catalogue_topk(last_hidden: torch.Tensor, table: torch.Tensor, bias, num_items: int, k: int, group=None,
+                                exclude=None):
     """Vocab-parallel top-k: every rank scores ALL users against ITS row block of the (replicated or locally held)
     table with global item ids, the per-shard lists are exchanged and merged with the same (score desc, id asc) rule,
-    so the result does not depend on the number of shards."""
+    so the result does not depend on the number of shards.  ``exclude`` ([U, n] global item ids, see ``ops.score_topk``):
+    the users are the same on every rank, so every shard filters with the same rows."""
     from . import ops
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     b, e = shard_range(num_items, rank, world)  # items are rows 1..V
     if e > b:
-        vals, ids = ops.score_topk(last_hidden, table, bias, 1 + b, 1 + e, k)
+        vals, ids = ops.score_topk(last_hidden, table, bias, 1 + b, 1 + e, k, exclude=exclude)
     else:
         U = last_hidden.shape[0]
         vals = torch.full((U, k), float("-inf"), device=last_hidden.device)
@@ -458,27 +460,39 @@ def _score_layer(model):
     return model.sas.item_emb.weight, None, sh.tok_begin
 
 
-def sharded_model_topk(model, x, k: int = 10):
+def sharded_model_topk(model, x, k: int = 10, exclude=None):
     """Full-catalogue top-k of the last position for a model cut by :func:`shard_bert_model` / :func:`shard_sas_model`
     (SURVEY.md 8e, top-k eval): the last hidden rows of all ranks' users are all-gathered ([B, d] per rank), every rank runs
     the fused scoring + top-k on ITS rows of the scored layer with GLOBAL item ids, the per-shard lists are exchanged with an
     all-to-all by user range (each rank receives the lists of its own users only: k * 12 B per user and shard) and merged
     under the single-GPU order rule (score desc, id asc), so the result equals the unsharded model's.  Every rank must pass
-    the same number of users."""
+    the same number of users.  ``exclude`` ([B, n] global item ids of this rank's users, see ``ops.score_topk``; every rank
+    passes one or every rank passes None) travels with the hidden rows: padded to the largest n of all ranks and all-gathered,
+    so every shard filters every user with global ids."""
     from . import ops
     sh = model._shard
     group, world, rank = sh.group, sh.world, sh.rank
     h = model.last_hidden(x).contiguous()
     B, d = h.shape
+    if exclude is not None:
+        exclude = model._device_long(exclude).reshape(B, -1)
     if world > 1:
         h_all = torch.empty(world * B, d, device=h.device, dtype=h.dtype)
         dist.all_gather_into_tensor(h_all, h, group=group)
+        if exclude is not None:
+            n = torch.tensor([exclude.shape[1]], device=h.device, dtype=torch.int64)
+            dist.all_reduce(n, op=dist.ReduceOp.MAX, group=group)
+            n = int(n.item())
+            padded = torch.zeros(B, n, device=h.device, dtype=torch.int64)
+            padded[:, :exclude.shape[1]] = exclude
+            exclude = torch.empty(world * B, n, device=h.device, dtype=torch.int64)
+            dist.all_gather_into_tensor(exclude, padded, group=group)
     else:
         h_all = h
     w, b, begin = _score_layer(model)
     lo = 1 if begin == 0 else 0  # row 0 is the padding id, not an item
     if w.shape[0] > lo:
-        vals, ids = ops.score_topk(h_all, w, b, lo, w.shape[0], k, id_offset=begin)
+        vals, ids = ops.score_topk(h_all, w, b, lo, w.shape[0], k, id_offset=begin, exclude=exclude)
     else:
         vals = torch.full((world * B, k), float("-inf"), device=h.device)
         ids = torch.full((world * B, k), -1, device=h.device, dtype=torch.int64)

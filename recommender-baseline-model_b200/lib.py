@@ -82,6 +82,7 @@ SIGNATURES = {
     "rbm_score_topk_ws_bytes": (_SZ, [_L, _L, _I]),
     "rbm_score_topk_ws_bytes_d": (_SZ, [_L, _L, _I, _I]),
     "rbm_score_topk": (_I, [_P, _L, _P, _P, _L, _L, _L, _P, _P, _L, _I, _I, _P, _SZ, _P]),
+    "rbm_score_topk_excl": (_I, [_P, _L, _P, _P, _L, _L, _L, _P, _L, _I, _P, _P, _L, _I, _I, _P, _SZ, _P]),
     "rbm_topk_rows": (_I, [_P, _L, _P, _P, _L, _L, _I, _L, _P]),
     "rbm_topk_merge": (_I, [_P, _P, _P, _P, _I, _L, _I, _P]),
     "rbm_rank_metrics": (_I, [_P, _P, _P, _P, _P, _P, _I, _P, _L, _I, _L, _L, _P]),

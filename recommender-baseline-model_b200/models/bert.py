@@ -310,9 +310,11 @@ class BERTModel(BaseModel):
             return sharded_candidate_scores(self, x, candidates)
         return ops.candidate_scores(self.last_hidden(x), self.out.weight, self.out.bias, self._device_long(candidates))
 
-    def full_catalogue_topk(self, x, k=10):
-        """Top-k items (ids 1..V) of the last position, (score desc, id asc); scores never materialised (K19-K21)."""
+    def full_catalogue_topk(self, x, k=10, exclude=None):
+        """Top-k items (ids 1..V) of the last position, (score desc, id asc); scores never materialised (K19-K21).
+        ``exclude`` ([B, n] int64 item ids, ids <= 0 = padding): items each user must not be ranked, e.g. their history."""
         if getattr(self, "_shard", None) is not None:
             from ..dist import sharded_model_topk
-            return sharded_model_topk(self, x, k)
-        return ops.score_topk(self.last_hidden(x), self.out.weight, self.out.bias, 1, self.num_items + 1, k)
+            return sharded_model_topk(self, x, k, exclude=exclude)
+        return ops.score_topk(self.last_hidden(x), self.out.weight, self.out.bias, 1, self.num_items + 1, k,
+                              exclude=self._device_long(exclude) if exclude is not None else None)

@@ -236,9 +236,12 @@ class SASModel(BaseModel):
             return sharded_candidate_scores(self, log_seqs, item_indices)
         return ops.candidate_scores(self.last_hidden(log_seqs), self.sas.item_emb.weight, None, self._device_long(item_indices))
 
-    def full_catalogue_topk(self, log_seqs, k=10):
-        """Top-k items (ids 1..V), (score desc, id asc); the [B, V, d] gather of ``predict`` is never built (K19-K21)."""
+    def full_catalogue_topk(self, log_seqs, k=10, exclude=None):
+        """Top-k items (ids 1..V), (score desc, id asc); the [B, V, d] gather of ``predict`` is never built (K19-K21).
+        ``exclude`` ([B, n] int64 item ids, ids <= 0 = padding): items each user must not be ranked; ``exclude=log_seqs``
+        ranks everything that is not in the input."""
         if getattr(self, "_shard", None) is not None:
             from ..dist import sharded_model_topk
-            return sharded_model_topk(self, log_seqs, k)
-        return ops.score_topk(self.last_hidden(log_seqs), self.sas.item_emb.weight, None, 1, self.sas.item_num + 1, k)
+            return sharded_model_topk(self, log_seqs, k, exclude=exclude)
+        return ops.score_topk(self.last_hidden(log_seqs), self.sas.item_emb.weight, None, 1, self.sas.item_num + 1, k,
+                              exclude=self._device_long(exclude) if exclude is not None else None)

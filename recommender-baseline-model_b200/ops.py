@@ -813,18 +813,38 @@ def candidate_scores(f, table, bias, cand):
     return out
 
 
-def score_topk(f, table, bias, v_begin, v_end, k, id_offset=0):
-    """Fused full-catalogue scoring + top-k over table rows [v_begin, v_end)  (K19-K21)."""
+def score_topk(f, table, bias, v_begin, v_end, k, id_offset=0, exclude=None):
+    """Fused full-catalogue scoring + top-k over table rows [v_begin, v_end)  (K19-K21); ids = row + id_offset.
+
+    ``exclude`` (optional ``[U, n]`` int64 CUDA tensor): row u lists ids (same id space as the result) that user u must not be
+    ranked, in any order, with duplicates allowed; ids <= 0 are padding.  The result is then the top-k of the remaining items
+    (trailing ``(-inf, -1)`` when fewer than k remain)."""
     lib = L.load()
     L.require_cuda(f, table)
     f2 = _rows2d(f)
     U, d = f2.shape
+    ex, n_ex = None, 0
+    if exclude is not None:
+        if not torch.is_tensor(exclude) or not exclude.is_cuda or exclude.device != f.device:
+            raise RuntimeError("score_topk: exclude must be a CUDA tensor on the device of f")
+        if exclude.dtype != torch.int64 or exclude.dim() != 2 or exclude.shape[0] != U:
+            raise RuntimeError("score_topk: exclude must be int64 [U=%d, n], got %s %s" % (U, exclude.dtype, tuple(exclude.shape)))
+        n_ex = int(exclude.shape[1])
+        if n_ex > 0:
+            ex = exclude
+            if v_begin + id_offset <= 0:  # ids <= 0 are real items of this call: keep the padding from matching them
+                ex = ex.masked_fill(ex <= 0, torch.iinfo(torch.int64).min)
+            ex = torch.sort(ex, dim=1).values.contiguous()  # the kernels walk each row in ascending order
     vals = torch.empty(U, k, device=f.device, dtype=torch.float32)
     ids = torch.empty(U, k, device=f.device, dtype=torch.int64)
     nb = lib.rbm_score_topk_ws_bytes_d(U, v_end - v_begin, d, k)
     ws = _ws("topk", nb, f.device)
-    check(lib.rbm_score_topk(ptr(f2), f2.stride(0), ptr(table), ptr(bias), v_begin, v_end, id_offset, ptr(vals), ptr(ids), U, d, k,
-                             ptr(ws), nb, stream()), "score_topk")
+    if ex is None:
+        check(lib.rbm_score_topk(ptr(f2), f2.stride(0), ptr(table), ptr(bias), v_begin, v_end, id_offset, ptr(vals), ptr(ids), U, d, k,
+                                 ptr(ws), nb, stream()), "score_topk")
+    else:
+        check(lib.rbm_score_topk_excl(ptr(f2), f2.stride(0), ptr(table), ptr(bias), v_begin, v_end, id_offset, ptr(ex), ex.stride(0), n_ex,
+                                      ptr(vals), ptr(ids), U, d, k, ptr(ws), nb, stream()), "score_topk")
     count_launches(2)
     return vals, ids
 

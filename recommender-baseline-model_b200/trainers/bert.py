@@ -2,7 +2,7 @@
 import torch
 
 from .base import AbstractTrainer
-from .utils import recalls_ndcgs_and_mrr_for_ks
+from .utils import full_catalogue_batch_metrics, recalls_ndcgs_and_mrr_for_ks
 
 
 class BERTTrainer(AbstractTrainer):
@@ -17,7 +17,10 @@ class BERTTrainer(AbstractTrainer):
         return self.model.loss(seqs, labels)
 
     def calculate_metrics(self, batch):
-        """NN/trainers/bert.py:43-52: last-position scores at the candidates -> Recall/NDCG/MRR@k."""
+        """NN/trainers/bert.py:43-52: last-position scores at the candidates -> Recall/NDCG/MRR@k.  With
+        ``args.full_catalogue_eval`` the batch is (seq, answers, exclude) and every unseen item is ranked instead."""
+        if getattr(self.args, 'full_catalogue_eval', False):
+            return full_catalogue_batch_metrics(self.model, batch, self.metric_ks, self.device)
         seqs, candidates, labels = [x.to(self.device, non_blocking=True) for x in batch]
         scores = self.model.candidate_scores(seqs, candidates)
         return recalls_ndcgs_and_mrr_for_ks(scores, labels, self.metric_ks)

@@ -3,7 +3,7 @@ import numpy as np
 import torch
 
 from .base import AbstractTrainer
-from .utils import recalls_ndcgs_and_mrr_for_ks
+from .utils import full_catalogue_batch_metrics, recalls_ndcgs_and_mrr_for_ks
 
 
 class SASTrainer(AbstractTrainer):
@@ -31,7 +31,10 @@ class SASTrainer(AbstractTrainer):
         return loss
 
     def calculate_metrics(self, batch):
-        """NN/trainers/sas.py:56-62."""
+        """NN/trainers/sas.py:56-62.  With ``args.full_catalogue_eval`` the batch is (seq, answers, exclude) and every unseen item
+        is ranked instead."""
+        if getattr(self.args, 'full_catalogue_eval', False):
+            return full_catalogue_batch_metrics(self.model, batch, self.metric_ks, self.device)
         seqs, candidates, labels = batch
         logits = self.model.predict(seqs, candidates)
         return recalls_ndcgs_and_mrr_for_ks(logits, labels, self.metric_ks)

@@ -40,3 +40,15 @@ def full_catalogue_metrics(top_ids, positives, ks):
     per_user = ops.rank_metrics(top_ids, ks, positives=positives.to(device=top_ids.device, dtype=torch.long))
     means = ops.column_mean(per_user).tolist()
     return _as_dict(ks, means)
+
+
+def full_catalogue_batch_metrics(model, batch, ks, device):
+    """Metrics of one ``(seq, answers, exclude)`` batch of the full-catalogue protocol (``args.full_catalogue_eval``): each user's
+    answer ranked among ALL items minus ``exclude`` (their history), same keys as the sampled protocol.  max(ks) <= 10 runs the
+    tcgen05 selection path; 11..32 the exact fp32 scan, which is exact but slow at 10^7 items."""
+    K = max(int(k) for k in ks)
+    if K > 32:
+        raise RuntimeError("metric cut-offs above 32 are not supported by the top-k kernel (got %d)" % K)
+    seqs, answers, exclude = [x.to(device, non_blocking=True) for x in batch]
+    _, top_ids = model.full_catalogue_topk(seqs, K, exclude=exclude)
+    return full_catalogue_metrics(top_ids, answers, ks)
