@@ -65,7 +65,8 @@ int rbm_embed_bwd(const int64_t* tok, const float* dout, float* g, float* dpos, 
 /* Row-sharded item table (SURVEY 8e "input lookup"): `table_shard` holds rows [v_begin, v_end) of the [vocab, d] table.  Same as
  * rbm_embed_fwd for tokens inside the shard; tokens of other shards produce exact zeros (their owner produces the value, so a
  * sum over the shards -- reduce-scatter -- is the unsharded result bit for bit).  `tok` is the rank-ordered concatenation of the
- * ranks' batches, so the dropout element index is the index in the global batch. */
+ * ranks' batches, so the dropout element index is the index in the global batch.  An empty shard (v_begin == v_end) may pass
+ * table_shard = NULL. */
 int rbm_embed_fwd_shard(const int64_t* tok, const float* table_shard, const float* pos, float* out, int64_t rows, int L,
                         int d, int64_t vocab, int64_t v_begin, int64_t v_end, float scale, int zero_pad, float p,
                         uint64_t seed, uint64_t site, rbm_stream_t stream);

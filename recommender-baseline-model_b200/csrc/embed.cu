@@ -158,7 +158,8 @@ extern "C" int rbm_embed_fwd(const int64_t* tok, const float* table, const float
 extern "C" int rbm_embed_fwd_shard(const int64_t* tok, const float* table, const float* pos, float* out, int64_t rows, int L,
                                    int d, int64_t vocab, int64_t v_begin, int64_t v_end, float scale, int zero_pad, float p,
                                    uint64_t seed, uint64_t site, rbm_stream_t stream) {
-  RBM_REQUIRE(tok && table && pos && out, "rbm_embed_fwd: null pointer");
+  // an empty shard (v_begin == v_end) is never read: its table may be NULL, which is what a zero-row tensor hands over
+  RBM_REQUIRE(tok && (table || v_begin == v_end) && pos && out, "rbm_embed_fwd: null pointer");
   RBM_REQUIRE(v_begin >= 0 && v_begin <= v_end && v_end <= vocab, "rbm_embed_fwd: bad shard range [%lld, %lld) of %lld rows",
               (long long)v_begin, (long long)v_end, (long long)vocab);
   RBM_REQUIRE(d > 0 && d % 4 == 0, "rbm_embed_fwd: d=%d must be a positive multiple of 4", d);

@@ -24,34 +24,6 @@ def close(a, b, rtol=1e-4, atol=1e-5, msg=""):
 
 
 # ------------------------------------------------------------------------------------------- embedding
-@pytest.mark.parametrize("zero_pad,scale", [(1, 8.0), (0, 1.0)])
-@pytest.mark.parametrize("p", [0.0, 0.25])
-def test_embed_fwd_bwd(zero_pad, scale, p):
-    torch.manual_seed(0)
-    B, Ln, d, V = 5, 12, 32, 41
-    tok = torch.randint(0, V, (B, Ln))
-    tok[0, :4] = 0
-    table = torch.randn(V, d)
-    pos = torch.randn(Ln, d)
-    dout = torch.randn(B, Ln, d)
-    seed, site = 1234, 7
-    tg, pg = g(table).requires_grad_(True), g(pos).requires_grad_(True)
-    out = ops.EmbedFn.apply(g(tok), tg, pg, scale, zero_pad, p, seed, site)
-    out.backward(g(dout))
-    mask = ops.dropout_mask(B * Ln * d, p, seed, site, DEV).cpu().view(B, Ln, d) if p > 0 else None
-    tr, pr = table.clone().requires_grad_(True), pos.clone().requires_grad_(True)
-    ref = F.embedding(tok, tr, padding_idx=0) * scale + pr.unsqueeze(0)
-    if p > 0:
-        assert abs(mask.float().mean().item() - (1 - p)) < 0.03
-        ref = ref * mask * (1.0 / (1.0 - p))
-    if zero_pad:
-        ref = ref * (tok != 0).unsqueeze(-1)
-    ref.backward(dout)
-    close(out, ref, 1e-6, 1e-6)
-    close(pg.grad, pr.grad, 1e-5, 1e-5)
-    close(tg.grad, tr.grad, 1e-5, 1e-5)
-
-
 def test_embed_bad_shapes_raise():
     with pytest.raises(RuntimeError):
         ops.EmbedFn.apply(g(torch.zeros(2, 4, dtype=torch.long)), g(torch.randn(5, 6)), g(torch.randn(4, 6)), 1.0, 0, 0.0, 0, 0)
@@ -91,27 +63,6 @@ def test_scatter_golden():
     np.testing.assert_array_equal(got[short], z["scatter.grad"][short])  # torch's own embedding_dense_backward, bit for bit
     np.testing.assert_allclose(got[~short], z["scatter.grad"][~short], rtol=1e-5, atol=1e-5)  # >64 contributions: fixed piece tree
     np.testing.assert_array_equal(got, oc.embedding_grad_scatter_chunked(z["scatter.idx"], z["scatter.rows"], 53))
-
-
-# -------------------------------------------------------------------------------------------- layernorm
-@pytest.mark.parametrize("flavour", [L.LN_TORCH, L.LN_BERT])
-@pytest.mark.parametrize("rows,d", [(7, 16), (33, 32), (1000, 64), (129, 128), (65, 256), (9, 512)])
-def test_layernorm(flavour, rows, d):
-    torch.manual_seed(rows + d)
-    x = torch.randn(rows, d) * 2 + 0.5
-    w, b = torch.randn(d), torch.randn(d)
-    dy = torch.randn(rows, d)
-    eps = 1e-8 if flavour == L.LN_TORCH else 1e-6
-    xg, wg, bg = (g(t).requires_grad_(True) for t in (x, w, b))
-    y = ops.layernorm(xg, wg, bg, eps, flavour)
-    y.backward(g(dy))
-    xr, wr, br = (t.clone().requires_grad_(True) for t in (x, w, b))
-    ref = oc.torch_layernorm(xr, wr, br, eps) if flavour == L.LN_TORCH else oc.bert_layernorm(xr, wr, br, eps)
-    ref.backward(dy)
-    close(y, ref, 1e-5, 1e-5)
-    close(xg.grad, xr.grad, 1e-4, 1e-5)
-    close(wg.grad, wr.grad, 1e-4, 1e-4)
-    close(bg.grad, br.grad, 1e-4, 1e-4)
 
 
 # ----------------------------------------------------------------------------------------------- linear
@@ -387,44 +338,6 @@ def test_score_ce(n, V1, d, frac):
     for got, rv, name in ((hg.grad, ref.dh, "dH"), (wg.grad, ref.dw, "dW"), (bg.grad, ref.db, "db")):
         e = float((got.double() - 1.7 * rv).abs().max() / (1.7 * rv).abs().max())
         assert e < 1e-4, (name, e)
-
-
-# -------------------------------------------------------------------------------------- SAS scoring + BCE
-@pytest.mark.parametrize("rows,d,V", [(30, 16, 20), (1000, 64, 3417), (640, 128, 12102)])
-def test_sas_score_bce(rows, d, V):
-    torch.manual_seed(rows)
-    f, table = torch.randn(rows, d), torch.randn(V, d) * 0.3
-    table[0] = 0
-    pos = torch.randint(0, V, (rows,))
-    pos[::3] = 0
-    neg = torch.randint(0, V, (rows,))
-    fg, tg = g(f).requires_grad_(True), g(table).requires_grad_(True)
-    pl, nl = ops.sas_scores(fg, tg, g(pos), g(neg))
-    loss = ops.bce_pair_loss(pl, nl, g(pos))
-    loss.backward()
-    fr, tr = f.clone().requires_grad_(True), table.clone().requires_grad_(True)
-    plr = (fr * F.embedding(pos, tr, padding_idx=0)).sum(-1)
-    nlr = (fr * F.embedding(neg, tr, padding_idx=0)).sum(-1)
-    idx = pos != 0
-    ref = F.binary_cross_entropy_with_logits(plr[idx], torch.ones(int(idx.sum()))) + \
-        F.binary_cross_entropy_with_logits(nlr[idx], torch.zeros(int(idx.sum())))
-    ref.backward()
-    close(pl, plr, 1e-4, 1e-5)
-    close(nl, nlr, 1e-4, 1e-5)
-    assert abs(loss.item() - ref.item()) < 1e-5 * max(1.0, abs(ref.item()))
-    close(fg.grad, fr.grad, 1e-4, 1e-7)
-    close(tg.grad, tr.grad, 1e-4, 1e-7)
-
-
-def test_candidate_scores():
-    torch.manual_seed(0)
-    U, Cn, d, V = 9, 101, 64, 500
-    f3 = torch.randn(U, 7, d)
-    table, bias = torch.randn(V, d), torch.randn(V)
-    cand = torch.randint(0, V, (U, Cn))
-    out = ops.candidate_scores(g(f3)[:, -1, :], g(table), g(bias), g(cand))
-    ref = torch.einsum("ucd,ud->uc", table[cand], f3[:, -1, :]) + bias[cand]
-    close(out, ref, 1e-4, 1e-5)
 
 
 # ------------------------------------------------------------------------------------------------ top-k
